@@ -2,6 +2,7 @@
 """bench.py — train tokens/s of Llama-3.1-8B (frozen INT8 base + LoRA r=8) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload text|speech|both]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -19,6 +20,10 @@ parameters.
     its heaviest shape against a cuBLASLt `torch._int_mm` 8192^3 peak measured in this process (outside every timed
     region), because MEASURED_PEAKS.json has no INT8 figure and the metric asks for "GEMM % INT8 peak".
 `--impl reference` times the UNMODIFIED reference (baseline/_ref) on the host cores.
+`--dump-outputs DIR` keeps the loss and gradients of the last timed step for comparing two builds output for output.
+Batch and initial parameters are seeded and the optimizer runs at learning rate 0, so every step computes from the same
+inputs. Float atomics (attention dQ, LoRA weight gradients, the loss sum) still make two runs agree to rounding, not bit
+for bit: compare with a tolerance.
 """
 import argparse
 import gc
@@ -37,6 +42,8 @@ UNIT = "tokens/s"
 
 LLAMA8B = dict(embed_dim=4096, num_layers=32, head_dim=128, num_heads=32, num_kv_heads=8, intermediate_dim=14336,
                vocab_size=128256, rope_base=500000, is_llama3_1=True)
+# --dump-outputs: gradients kept per workload (float32, 16 MiB each; the speech step alone trains ~72 M parameters)
+DUMP_GRADS = 1 << 22
 
 
 def parse():
@@ -61,7 +68,17 @@ def parse():
     ap.add_argument("--mixed-gemm", action="store_true",
                     help="opt-in: mixed-input bf16 x int8 GEMMs (SURVEY K4/K5) for the weight-only forward and every "
                          "grad_input; identical results, no bf16 weight operands in HBM")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last resident-timed step of each workload computed as "
+                         "DIR/<workload>_loss.npy (the loss) and DIR/<workload>_grads.npy (the trainable gradients after "
+                         "the all-reduce, flattened in parameter order; a fixed seeded sample of %d of them where there "
+                         "are more), float32" % DUMP_GRADS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -221,15 +238,25 @@ def run_workload(args, workload, rank, world, device, steps, warmup):
 
     model, cfg = build_model(args, device, workload)
     params = [p for p in model.parameters() if p.requires_grad]
-    opt = torch.optim.AdamW(params, lr=1e-4, weight_decay=0.0, fused=True)
+    # lr 0: the fused AdamW does the same work, but the parameters stay the seeded ones. With a real step size its
+    # sign-like first updates turn the rounding noise of the float atomics into different parameters from run to run
+    opt = torch.optim.AdamW(params, lr=0.0, weight_decay=0.0, fused=True)
     bucket = GradBucket(params)
     host, positions, n_label = make_batch(args, cfg, rank, workload)
     resident = {k: v.to(device) for k, v in host.items()}
     h2d_bytes = sum(v.numel() * v.element_size() for v in host.values())
     dp_events, compute_events = [], []
     track = {"on": False}
+    dump = None
+    if args.dump_outputs:
+        n_grad = sum(p.numel() for p in params)
+        pick = None
+        if n_grad > DUMP_GRADS:
+            pick = torch.randperm(n_grad, generator=torch.Generator().manual_seed(0))[:DUMP_GRADS].sort().values
+            pick = pick.to(device)
+        dump = {"pick": pick}
 
-    def step(batch):
+    def step(batch, keep=None):
         if track["on"]:
             c0, c1, c2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
             c0.record()
@@ -245,6 +272,10 @@ def run_workload(args, workload, rank, world, device, steps, warmup):
             c2.record()
             compute_events.append((c0, c1))
             dp_events.append((c1, c2))
+        if keep is not None:   # the gradients exist only until zero_grad below
+            flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])
+            keep["loss"] = loss.detach().clone()
+            keep["grads"] = flat if keep["pick"] is None else flat[keep["pick"]]
         opt.step()
         opt.zero_grad(set_to_none=True)
         return loss
@@ -254,17 +285,17 @@ def run_workload(args, workload, rank, world, device, steps, warmup):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(n, e2e):
+    def timed(n, e2e, keep=None):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         last = None
-        for _ in range(n):
+        for i in range(n):
             if e2e:
                 batch = {k: v.to(device, non_blocking=True) for k, v in host.items()}
                 last = step(batch).item()          # D2H read of the loss, every step
             else:
-                last = step(resident)
+                last = step(resident, keep if i == n - 1 else None)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -285,7 +316,7 @@ def run_workload(args, workload, rank, world, device, steps, warmup):
     # costs nothing measurable; the full per-kernel breakdown comes from a separate instrumented pass
     ops.TIMING.enable(only={"bf16_gemm", "int8_gemm"})
     track["on"] = world > 1
-    ms, loss_val = timed(steps, e2e=False)
+    ms, loss_val = timed(steps, e2e=False, keep=dump)
     kern_dom = ops.TIMING.summary()
     ops.TIMING.disable()
     track["on"] = False
@@ -334,6 +365,8 @@ def run_workload(args, workload, rank, world, device, steps, warmup):
     res = dict(ms=ms, ms_e2e=ms_e2e, ms_prof=ms_prof, prof_steps=prof_steps, loss=loss_val, kern=kern,
                kern_dom=kern_dom, clocks=clocks, positions=positions, n_label=n_label, h2d_bytes=h2d_bytes,
                dp_payload=bucket.nbytes(), dp=dp, seq=(args.seq if workload == "text" else positions // args.batch))
+    if dump is not None:
+        res["dump"] = {k: dump[k].float().cpu().numpy() for k in ("loss", "grads")}
     del model, opt, bucket, params, resident, host
     gc.collect()
     torch.cuda.empty_cache()
@@ -386,6 +419,13 @@ def run_ours(args):
             dist.destroy_process_group()
     if rank != 0:
         return
+    if args.dump_outputs:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for wl, r in ((head_wl, main), ("speech", pl)):
+            for k, v in (r["dump"].items() if r is not None else ()):
+                np.save(os.path.join(args.dump_outputs, f"{wl}_{k}.npy"), v)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

@@ -16,6 +16,8 @@ Reference entry points executed (file:line in the reference repo):
     modelling/llama.py:143-174    FeedForward, TransformerLayer (SDPA branch with a dense prefix-LM mask)
     modelling/audio.py:38-77      LlamaAudio.forward (tiny config, prefix-LM via the causal_mask/input_pos hook)
 """
+import io
+import lzma
 import os
 import sys
 
@@ -141,8 +143,11 @@ def main():
                             state={k: (v if not isinstance(v, ref_int8.Int8LinearWeight) else dict(int_data=v.int_data, scale=v.scale))
                                    for k, v in model.state_dict().items()})
 
-    path = os.path.join(OUT, "reference_vectors.pt")
-    torch.save(g, path)
+    path = os.path.join(OUT, "reference_vectors.pt.xz")
+    buf = io.BytesIO()
+    torch.save(g, buf)
+    with open(path, "wb") as f:   # xz halves the 1.8 MB: many inputs repeat across records (tests/helpers.load_golden)
+        f.write(lzma.compress(buf.getvalue(), preset=9 | lzma.PRESET_EXTREME))
     print("wrote", path, os.path.getsize(path) // 1024, "KiB;", "torch", torch.__version__)
 
 

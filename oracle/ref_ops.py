@@ -7,7 +7,7 @@ the product (`llamax_b200/`) never does.
 
 Parity pin: the reference ships no tests or golden vectors (SURVEY.md §4), so this restatement is pinned against
 outputs of the reference code itself, executed in the build container with fixed seeds
-(`oracle/make_golden.py` -> `tests/golden/*.pt`; checked by `tests/test_oracle_golden.py`).
+(`oracle/make_golden.py` -> `tests/golden/reference_vectors.pt.xz`; checked by `tests/test_oracle_golden.py`).
 
 Two flavours are provided where rounding matters:
   * `*_ref`  : the reference's own bf16 op sequence (bit-comparable to the reference on CPU)

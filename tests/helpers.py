@@ -1,7 +1,19 @@
 """Shared builders for the parity tests: a tiny model on the product path and the matching oracle weights."""
+import io
+import lzma
+import os
+
 import torch
 
 from oracle import ref_ops as R
+
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_vectors.pt.xz")
+
+
+def load_golden() -> dict:
+    """The vectors the reference code itself produced (oracle/make_golden.py): a torch.save'd dict, xz-compressed."""
+    with open(GOLD, "rb") as f:
+        return torch.load(io.BytesIO(lzma.decompress(f.read())), weights_only=False)
 
 
 def rel_err(a: torch.Tensor, b: torch.Tensor) -> float:

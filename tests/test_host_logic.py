@@ -1,7 +1,5 @@
 """CPU: host-side logic of the drop-in seams (no kernels launched): subclass behaviour, module surgery, state-dict
 compatibility with the reference, mask helpers, and loud failure off-GPU."""
-import os
-
 import pytest
 import torch
 from torch import nn
@@ -10,13 +8,12 @@ from llamax_b200.modelling import (AudioConfig, Llama, LlamaAudio, LlamaConfig, 
                                    apply_linear_adapter_)
 from llamax_b200.modelling import llama as L
 from llamax_b200.subclasses import Int8LinearWeight, int8_mm_dequant, quantize_int8_rowwise, quantize_linear_
-
-GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_vectors.pt")
+from tests.helpers import load_golden
 
 
 @pytest.fixture(scope="module")
 def gold():
-    return torch.load(GOLD, weights_only=False)
+    return load_golden()
 
 
 def test_from_float_matches_reference(gold):
@@ -196,3 +193,15 @@ def test_bench_arms_share_one_config(monkeypatch):
         ref = bench.workload_config(a, max(1, a.gpus), "text", a.batch * a.seq, bench.text_label_count(a))
         assert ours == ref and ours["parallelism"] == f"dp{gpus}" and ours["global_batch"] == batch * gpus
         assert "l2" in ours and ours["label_tokens_per_step"] == n_label * gpus
+
+
+def test_bench_rejects_arguments_it_cannot_honour():
+    """bench.py: fewer than one timed step, or an output dump from the CPU reference arm, is an argument error."""
+    import os
+    import subprocess
+    import sys
+
+    bench = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, bench, *extra], capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "error:" in r.stderr, (extra, r.stderr)

@@ -1,19 +1,16 @@
 """CPU: the oracle restatement (oracle/ref_ops.py) against golden vectors produced by the reference code itself
 (oracle/make_golden.py, run in the build container against /root/reference). Bit-exact wherever the oracle is the
 same op sequence as the reference."""
-import os
-
 import pytest
 import torch
 
 from oracle import ref_ops as R
-
-GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_vectors.pt")
+from tests.helpers import load_golden
 
 
 @pytest.fixture(scope="module")
 def gold():
-    return torch.load(GOLD, weights_only=False)
+    return load_golden()
 
 
 def test_quantize_rowwise_bit_exact(gold):
