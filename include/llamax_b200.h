@@ -193,6 +193,15 @@ int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
                     int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
                     const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
                     const void* rope_inverse, void* stream);
+/* Deterministic form (torch.use_deterministic_algorithms): same arguments without dq_accum, bitwise identical results
+ * from run to run. dq comes from a kernel that owns 128 query rows of one head and sums over the kv tiles in ascending
+ * order in tensor memory (no fp32 atomics, no workspace); dk / dv are bitwise those of llamax_attn_bwd. */
+int llamax_attn_bwd_deterministic(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                                  const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
+                                  int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* delta, int64_t B,
+                                  int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
+                                  const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
+                                  const void* rope_inverse, void* stream);
 
 /* ---- audio stem (modelling/audio.py:26-31,51-60): Conv1d(k3,s1)+GELU, Conv1d(k3,s2)+GELU -------------------------
  * The convolutions run on llamax_bf16_gemm: with channels-last activations padded by one zero row on each side of a
@@ -231,6 +240,12 @@ int llamax_batched_copy(const llamax_copy_job_t* jobs, int32_t n_jobs, void* str
  * of the big tensor); rank <= 32; `out` is zeroed by the call, token-dimension splits are reduced with fp32 red.add. */
 int llamax_lora_wgrad(const void* X, int64_t ldx, const void* Ht, int64_t ldht, void* out, int64_t M, int64_t P,
                       int32_t R, float alpha, void* stream);
+/* Deterministic form: each token split stores its fp32 partial into workspace [LLAMAX_LORA_WGRAD_MAX_SPLITS, P, R]
+ * (caller-provided; only the first `splits` slices are written) and the splits are summed in split order into `out`.
+ * Same arguments as llamax_lora_wgrad plus the workspace. */
+#define LLAMAX_LORA_WGRAD_MAX_SPLITS 32
+int llamax_lora_wgrad_deterministic(const void* X, int64_t ldx, const void* Ht, int64_t ldht, void* out,
+                                    void* workspace, int64_t M, int64_t P, int32_t R, float alpha, void* stream);
 
 /* Fused pair for one LoRA linear's backward (autograd of modelling/lora.py:43), ONE pass over dY [M,N] (pitch lddy):
  *   dh [M,R] bf16 (pitch lddh) = dY . Bt^T            Bt = lora_scale * B^T, bf16 [R,N] pitch ldbt
@@ -249,6 +264,10 @@ int llamax_lora_bwd_pair(const void* dY, int64_t lddy, const void* Bt, int64_t l
  * logits bf16 [M, V] pitch ld; labels int64 [M]; loss_sum, inv_n: fp32 device scalars. */
 int llamax_cross_entropy(void* logits, int64_t ld, const void* labels, void* loss_sum, const void* inv_n, int64_t M,
                          int64_t V, int write_grad, void* stream);
+/* Deterministic form: loss_rows fp32 [M] receives each row's loss (0 for ignored rows) instead of an atomic sum into one
+ * scalar; the caller sums the rows in a fixed order. The gradient written into the logits is that of llamax_cross_entropy. */
+int llamax_cross_entropy_rows(void* logits, int64_t ld, const void* labels, void* loss_rows, const void* inv_n,
+                              int64_t M, int64_t V, int write_grad, void* stream);
 
 #ifdef __cplusplus
 }

@@ -40,6 +40,7 @@ class Epilogue(Structure):
 EP = POINTER(Epilogue)
 
 MAX_COPY_JOBS = 64
+LORA_WGRAD_MAX_SPLITS = 32
 
 
 class CopyJob(Structure):
@@ -81,13 +82,17 @@ SIGNATURES = {
     "llamax_attn_fwd": [P, I64, P, I64, P, I64, P, I64, P, I64, I64, I32, I32, I32, I64, P, P, c_float, P],
     "llamax_attn_bwd": [P, I64, P, I64, P, I64, P, I64, P, P, I64, P, I64, P, I64, P, I64, P, P,
                         I64, I64, I32, I32, I32, I64, P, P, P, c_float, P, P],
+    "llamax_attn_bwd_deterministic": [P, I64, P, I64, P, I64, P, I64, P, P, I64, P, I64, P, I64, P, I64, P,
+                                      I64, I64, I32, I32, I32, I64, P, P, P, c_float, P, P],
     "llamax_lora_wgrad": [P, I64, P, I64, P, I64, I64, I32, c_float, P],
+    "llamax_lora_wgrad_deterministic": [P, I64, P, I64, P, P, I64, I64, I32, c_float, P],
     "llamax_lora_bwd_pair": [P, I64, P, I64, P, I64, P, I64, P, I64, P, P, I64, I64, I32, c_float, P],
     "llamax_gelu_bias_fwd": [P, P, P, I64, I64, I32, I32, I32, P],
     "llamax_gelu_bwd": [P, P, P, I64, I64, I32, I32, I32, P],
     "llamax_conv_s2k3_col2im": [P, P, I64, I64, I64, P],
     "llamax_batched_copy": [POINTER(CopyJob), I32, P],
     "llamax_cross_entropy": [P, I64, P, P, P, I64, I64, c_int, P],
+    "llamax_cross_entropy_rows": [P, I64, P, P, P, I64, I64, c_int, P],
 }
 
 _lib = None

@@ -89,6 +89,21 @@ constexpr int kNB = 2;                             // smem stages of K and V, TM
 constexpr int kThreads = 256;                     // warp0 TMA, warp1 MMA, warp2 TMEM alloc, warps 4-7 softmax
 }  // namespace fwd
 
+// Tile classification of a 128-row query tile starting at q0 (attn_fwd_kernel, attn_bwd_dq_kernel): the kv tiles it
+// visits are [j_begin, j_begin + n_kv) — up to max(P, q0 + 128), and, with packed documents, from the start of the first
+// row's document on; a visited tile needs no element test when every (q, kv) pair of it is visible and in range.
+template <bool kDocs>
+__device__ __forceinline__ void q_tile_kv_range(int S, int Pb, const int32_t* doc_start, int b, int q0, int& j_begin,
+                                                int& n_kv) {
+  const int kv_end = min(S, max(Pb, q0 + 128));
+  j_begin = kDocs ? doc_start[(int64_t)b * S + q0] / 128 : 0;
+  n_kv = (kv_end + 127) / 128 - j_begin;
+}
+// ds_tile: document start of the tile's last row (0 without documents)
+__device__ __forceinline__ bool q_tile_full(int S, int Pb, int ds_tile, int q0, int kv0) {
+  return (kv0 + 128 <= S) && ((kv0 + 128 <= Pb) || (kv0 + 127 <= q0)) && (kv0 >= ds_tile);
+}
+
 // kDocs: packed-document mask compiled in; kD: real head dim (64 runs on zero-padded 128-wide tiles).
 // (A variant with two softmax warpgroups per query tile — column halves, row maxima exchanged through smem — was
 // measured 10 % slower than this single-warpgroup version on B200: the extra 256-thread barrier per tile and the
@@ -130,10 +145,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   const int Pb = p.prefix_b ? min(max(p.prefix_b[b], 0), p.S) : p.P;   // prefix length of this sequence
   const int hk = h / (p.Hq / p.Hkv);
   const int q0 = qt * kTile;
-  const int kv_end = min(p.S, max(Pb, q0 + kTile));
-  // packed documents: keys before the start of the first row's document are never visible to this tile
-  const int j_begin = kDocs ? p.doc_start[(int64_t)b * p.S + q0] / kTile : 0;
-  const int n_kv = (kv_end + kTile - 1) / kTile - j_begin;  // number of visited kv tiles
+  int j_begin, n_kv;   // visited kv tiles
+  q_tile_kv_range<kDocs>(p.S, Pb, p.doc_start, b, q0, j_begin, n_kv);
 
   if (warp == 0 && elect_one()) {
     tma_prefetch_desc(&tmQ);
@@ -248,8 +261,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     for (int j = 0; j < n_kv; ++j) {
       const int st = kNB == 2 ? (j & 1) : 0;
       const int kv0 = (j_begin + j) * kTile;
-      // tile needs the element test unless every (q, kv) pair is visible and in range
-      const bool full_tile = (kv0 + kTile <= p.S) && ((kv0 + kTile <= Pb) || (kv0 + kTile - 1 <= q0)) && (kv0 >= ds_tile);
+      const bool full_tile = q_tile_full(p.S, Pb, ds_tile, q0, kv0);
       LX_TR(tr_cta, j, 4);
       mbar_wait(&s_full[st], (kNB == 2 ? (j >> 1) : j) & 1);
       tc_fence_after();
@@ -1745,6 +1757,7 @@ constexpr int kQ = 128;                           // query rows per step
 // warpgroup 0: control (warp 0 TMA, warp 1 MMA issue, warp 2 TMEM alloc); warpgroups 1-2: softmax-grad workers;
 // warpgroup 3: dQ drain (TMEM -> fp32 smem tile -> bulk reduce-add)
 constexpr int kThreads = 512;
+constexpr int kThreadsNoDQ = 384;                 // attn_bwd_kernel<.., kNoDQ = true>: no drain warpgroup
 constexpr int kWorkers = 256;
 constexpr int kRegsCtrl = 64, kRegsWork = 144, kRegsDrain = 160;   // setmaxnreg: 64 + 2 * 144 + 160 = 4 * 128
 constexpr int kTileBytes = 128 * kHD * 2;         // 32 KB: two 16 KB boxes of [128 rows x 128 B]
@@ -1776,8 +1789,12 @@ constexpr int kColdV = 0, kColdK = 128, kColX = 256, kColY = 384;
 // MMA issue order per step:  dV(s), S^T(s+1) | dQ^T(s), dK(s) | dP^T(s+1)
 //   workers compute dS(s) under dV(s)/S^T(s+1), P(s+1) under dQ^T(s)/dK(s)/dP^T(s+1); the drain pulls dQ^T(s) into
 //   registers under dK(s), so the pipe only waits on semaphores that have normally fired already.
-template <bool kDocs, int kD>
-__global__ void __launch_bounds__(bwd::kThreads, 1)
+// kNoDQ (deterministic mode): dQ^T(s) is neither computed nor drained — attn_bwd_dq_kernel produces dQ without atomics —
+// and dP^T(s+1) waits only for dS^T(s); dV and dK accumulate in the same MMA order, so they are bitwise those of the
+// default instantiation. Without the drain warpgroup the CTA has 384 threads and no setmaxnreg rebalancing (the 168
+// registers a thread gets need no spills).
+template <bool kDocs, int kD, bool kNoDQ = false>
+__global__ void __launch_bounds__(kNoDQ ? bwd::kThreadsNoDQ : bwd::kThreads, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                 const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
                 const AttnBwdParams p) {
@@ -1852,7 +1869,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp < 4) {
-    setmaxnreg_dec<kRegsCtrl>();
+    if constexpr (!kNoDQ) setmaxnreg_dec<kRegsCtrl>();
     if (warp == 0) {
       // ------------------------------------ TMA producer ------------------------------------
       if (elect_one()) {
@@ -1934,11 +1951,13 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
           mbar_wait(ds_full, s & 1);                 // dS^T(s) is in smem, dP^T(s) has been read
           tc_fence_after();
           LX_TR(tr_cta, s, 3);
-          // dQ^T = K^T dS^T   (M = d, N = q, K dim = kv)
+          if constexpr (!kNoDQ) {
+            // dQ^T = K^T dS^T   (M = d, N = q, K dim = kv)
 #pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma_ss<false, 1>(tY, desc_join(loKmn + ks * 128, kHi), desc_join(lodSmn + ks * 128, kHi), idesc_dq, ks != 0);
-          umma_commit(dq_full);
+            for (int ks = 0; ks < 8; ++ks)
+              umma_ss<false, 1>(tY, desc_join(loKmn + ks * 128, kHi), desc_join(lodSmn + ks * 128, kHi), idesc_dq, ks != 0);
+            umma_commit(dq_full);
+          }
           // dK += dS^T Q      (K dim = q: boxes of 64 queries)
 #pragma unroll
           for (int ks = 0; ks < 8; ++ks)
@@ -1947,7 +1966,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
           umma_commit(&q_empty[st]);
           LX_TR(tr_cta, s, 4);
           if (s + 1 < n_steps) {
-            mbar_wait(dq_empty, s & 1);              // the drain warps hold dQ^T(s) in registers
+            if constexpr (!kNoDQ) mbar_wait(dq_empty, s & 1);   // the drain warps hold dQ^T(s) in registers
             mbar_wait(do_full, (s + 1) & 1);
             tc_fence_after();
             mma_kk(tY, loV, lodO);                   // dP^T(s+1)
@@ -1961,7 +1980,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     }
   } else if (warp < 12) {
     // ------------------------------------ workers: thread = kv row, 64 query columns ------------------------------------
-    setmaxnreg_inc<kRegsWork>();
+    if constexpr (!kNoDQ) setmaxnreg_inc<kRegsWork>();
     const int wt = threadIdx.x - 128;           // 0..255
     const int grp = (warp - 4) >> 2;            // query-column half handled by this warp
     const int lq = warp & 3;                    // TMEM lane quarter (hardware: warp % 4)
@@ -2138,7 +2157,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       }
     }
     tc_fence_before();
-  } else {
+  } else if constexpr (!kNoDQ) {
     // ------------------------------------ dQ drain (thread = head-dim element) ------------------------------------
     // TMEM dQ^T [d][128 q] -> registers (Y is released at once) -> red.global.add into dq_accum[b, hq, q0 : q0 + 128, :]
     setmaxnreg_inc<kRegsDrain>();
@@ -2176,6 +2195,285 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       }
       LX_TR(tr_cta, s, 15);
     }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) tmem_dealloc<1>(tmem_base, 512);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Deterministic dQ (torch.use_deterministic_algorithms): CTA = (128 query rows, 1 query head), the forward's structure.
+// The CTA walks the visible kv tiles of its rows in ascending order (attn_fwd_kernel's tile range and full-tile test)
+// and accumulates dQ in TMEM, so the summation order is fixed by construction: no fp32 atomics, no dq_accum.
+// Per kv tile j (every MMA 128 x 128 x 16):
+//   S = Q K^T, dP = dO V^T          (TMEM, thread = query row)
+//   P = exp2(S * scale_log2 - lse2) from the saved LSE (no online max), dS = P o (dP - delta) * scale, written as bf16
+//   pairs over the score columns just read
+//   dQ += dS K                      (A = dS from TMEM, B = K as the MN-major operand, like V in the forward's PV)
+//   TMEM (512 columns): S0 | S1 | dP | dQ.   MMA issue order: S(j+1) | dQ(j), dP(j+1)
+// The epilogue applies the RoPE backward to the fp32 accumulator with attn_dq_convert_kernel's arithmetic and rounds
+// once to bf16. The S and dP products are recomputed here (attn_bwd_kernel<.., kNoDQ> computes them for dK / dV).
+// ------------------------------------------------------------------------------------------------
+namespace bwdq {
+constexpr int kTile = 128;
+constexpr int kTileBytes = kTile * kHD * 2;        // 32 KB
+constexpr int kOffQ = 0;
+constexpr int kOffdO = kOffQ + kTileBytes;
+constexpr int kOffK = kOffdO + kTileBytes;         // 2 stages
+constexpr int kOffV = kOffK + 2 * kTileBytes;      // 2 stages
+constexpr int kOffBar = kOffV + 2 * kTileBytes;
+// qdo_full, k full/empty[2], v full/empty[2], s full/empty[2], dp_full, ds_full, dq_done
+constexpr int kNumBars = 1 + 4 + 4 + 4 + 3;
+constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 16 + 1024;
+static_assert(kSmemBytes <= 232448, "deterministic dQ shared memory budget");
+constexpr int kThreads = 256;                      // warp 0 TMA, warp 1 MMA, warp 2 TMEM alloc, warps 4-7: thread = query row
+constexpr int kColS = 0, kColdP = 256, kColdQ = 384;
+}  // namespace bwdq
+
+template <bool kDocs, int kD>
+__global__ void __launch_bounds__(bwdq::kThreads, 1)
+attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
+                   const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
+                   const AttnBwdParams p, __nv_bfloat16* __restrict__ dq, int64_t lddq) {
+  using namespace bwdq;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
+  uint64_t* qdo_full = bars;
+  uint64_t* k_full = bars + 1;     // [2]
+  uint64_t* k_empty = bars + 3;    // [2]
+  uint64_t* v_full = bars + 5;     // [2]
+  uint64_t* v_empty = bars + 7;    // [2]
+  uint64_t* s_full = bars + 9;     // [2]
+  uint64_t* s_empty = bars + 11;   // [2]: dQ(j) has consumed dS(j), written over S buffer j & 1
+  uint64_t* dp_full = bars + 13;
+  uint64_t* ds_full = bars + 14;   // dS(j) is in TMEM and dP(j) has been read
+  uint64_t* dq_done = bars + 15;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars);
+
+  const int warp = threadIdx.x >> 5;
+  // grid = (query heads, batch, query tiles), longest tiles first (as attn_fwd_kernel)
+  const int qt = gridDim.z - 1 - blockIdx.z;
+  const int h = blockIdx.x, b = blockIdx.y;
+  const int Pb = p.prefix_b ? min(max(p.prefix_b[b], 0), p.S) : p.P;
+  const int hk = h / (p.Hq / p.Hkv);
+  const int q0 = qt * kTile;
+  int j_begin, n_kv;
+  q_tile_kv_range<kDocs>(p.S, Pb, p.doc_start, b, q0, j_begin, n_kv);
+
+  if (warp == 0 && elect_one()) {
+    tma_prefetch_desc(&tmQ);
+    tma_prefetch_desc(&tmK);
+    tma_prefetch_desc(&tmV);
+    tma_prefetch_desc(&tmdO);
+  }
+  if (warp == 1 && elect_one()) {
+    mbar_init(qdo_full, 1);
+    for (int i = 0; i < 2; ++i) {
+      mbar_init(&k_full[i], 1);
+      mbar_init(&k_empty[i], 1);
+      mbar_init(&v_full[i], 1);
+      mbar_init(&v_empty[i], 1);
+      mbar_init(&s_full[i], 1);
+      mbar_init(&s_empty[i], 1);
+    }
+    mbar_init(dp_full, 1);
+    mbar_init(ds_full, 4);
+    mbar_init(dq_done, 1);
+    fence_mbar_init();
+  }
+  if (warp == 2) {
+    tmem_alloc<1>(tmem_slot, 512);
+    tmem_relinquish<1>();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_S = tmem_base + kColS, tmem_dP = tmem_base + kColdP, tmem_dQ = tmem_base + kColdQ;
+
+  if (warp == 0) {
+    // ------------------------------------ TMA producer ------------------------------------
+    if (elect_one()) {
+      mbar_expect_tx(qdo_full, 2 * kTileBytes);
+      tma_load_4d(smem + kOffQ, &tmQ, qdo_full, 0, h, q0, b);
+      tma_load_4d(smem + kOffQ + kTileBytes / 2, &tmQ, qdo_full, 64, h, q0, b);
+      tma_load_4d(smem + kOffdO, &tmdO, qdo_full, 0, h, q0, b);
+      tma_load_4d(smem + kOffdO + kTileBytes / 2, &tmdO, qdo_full, 64, h, q0, b);
+      for (int j = 0; j < n_kv; ++j) {
+        const int st = j & 1;
+        const uint32_t ph = (j >> 1) & 1;
+        const int kv0 = (j_begin + j) * kTile;
+        mbar_wait(&k_empty[st], ph ^ 1);
+        mbar_expect_tx(&k_full[st], kTileBytes);
+        uint8_t* sk = smem + kOffK + st * kTileBytes;
+        tma_load_4d(sk, &tmK, &k_full[st], 0, hk, kv0, b);
+        tma_load_4d(sk + kTileBytes / 2, &tmK, &k_full[st], 64, hk, kv0, b);
+        mbar_wait(&v_empty[st], ph ^ 1);
+        mbar_expect_tx(&v_full[st], kTileBytes);
+        uint8_t* sv = smem + kOffV + st * kTileBytes;
+        tma_load_4d(sv, &tmV, &v_full[st], 0, hk, kv0, b);
+        tma_load_4d(sv + kTileBytes / 2, &tmV, &v_full[st], 64, hk, kv0, b);
+      }
+    }
+    __syncwarp();
+  } else if (warp == 1) {
+    // ------------------------------------ MMA issuer ------------------------------------
+    if (elect_one()) {
+      constexpr uint32_t idesc_s = make_idesc(1, 1, 128, 128, 0, 0);   // S, dP: [q x d] . [kv x d]^T
+      constexpr uint32_t idesc_dq = make_idesc(1, 1, 128, 128, 0, 1);  // dQ: [q x kv] . [kv x d]  (B = K MN-major)
+      constexpr uint32_t kHi = desc_hi(1024);
+      const uint32_t loQ = desc_lo(smem_u32(smem + kOffQ), 16), lodO = desc_lo(smem_u32(smem + kOffdO), 16);
+      const uint32_t loK0 = desc_lo(smem_u32(smem + kOffK), 16), loKmn0 = desc_lo(smem_u32(smem + kOffK), 16384);
+      const uint32_t loV0 = desc_lo(smem_u32(smem + kOffV), 16);
+      auto mma_kk = [&](uint32_t d, uint32_t a_lo, uint32_t b_lo) {
+#pragma unroll
+        for (int dh = 0; dh < 2; ++dh)
+#pragma unroll
+          for (int ks = 0; ks < 4; ++ks)
+            umma_ss<false, 1>(d, desc_join(a_lo + dh * 1024 + ks * 2, kHi), desc_join(b_lo + dh * 1024 + ks * 2, kHi),
+                              idesc_s, (dh | ks) != 0);
+      };
+      auto issue_s = [&](int j) {
+        const int st = j & 1;
+        const uint32_t ph = (j >> 1) & 1;
+        mbar_wait(&k_full[st], ph);
+        mbar_wait(&s_empty[st], ph ^ 1);
+        tc_fence_after();
+        mma_kk(tmem_S + st * 128, loQ, loK0 + st * (kTileBytes / 16));
+        umma_commit(&s_full[st]);
+      };
+      auto issue_dp = [&](int j) {   // dP buffer: free once the workers have read dP(j - 1) (ds_full waited before)
+        const int st = j & 1;
+        mbar_wait(&v_full[st], (j >> 1) & 1);
+        tc_fence_after();
+        mma_kk(tmem_dP, lodO, loV0 + st * (kTileBytes / 16));
+        umma_commit(dp_full);
+        umma_commit(&v_empty[st]);
+      };
+      mbar_wait(qdo_full, 0);
+      issue_s(0);
+      issue_dp(0);
+      for (int j = 0; j < n_kv; ++j) {
+        const int st = j & 1;
+        if (j + 1 < n_kv) issue_s(j + 1);
+        mbar_wait(ds_full, j & 1);
+        tc_fence_after();
+        const uint32_t loKmn = loKmn0 + st * (kTileBytes / 16);
+#pragma unroll
+        for (int kb = 0; kb < 2; ++kb)
+#pragma unroll
+          for (int ks = 0; ks < 4; ++ks)
+            // A = dS from TMEM: bf16 pairs, 8 columns per 16-wide k-step (16 kv rows of K)
+            umma_ts_f16(tmem_dQ, tmem_S + st * 128 + (kb * 4 + ks) * 8, desc_join(loKmn + (kb * 64 + ks * 16) * 8, kHi),
+                        idesc_dq, (j | kb | ks) != 0);
+        umma_commit(&s_empty[st]);
+        umma_commit(&k_empty[st]);
+        if (j + 1 < n_kv) issue_dp(j + 1);
+      }
+      umma_commit(dq_done);
+    }
+    __syncwarp();
+  } else if (warp >= 4) {
+    // ------------------------------------ dS workers: thread = query row ------------------------------------
+    const int r = threadIdx.x - 128;
+    const uint32_t lane_off = uint32_t((warp - 4) * 32) << 16;
+    const int q = q0 + r;
+    const bool row_ok = q < p.S;
+    const int64_t sidx = ((int64_t)b * p.Hq + h) * p.S + q;
+    const float lse2 = row_ok ? p.lse[sidx] * kLog2e : INFINITY;   // rows past the end: P = 0
+    const float dlt = row_ok ? p.delta[sidx] * p.scale : 0.f;
+    const int ds_row = kDocs ? p.doc_start[(int64_t)b * p.S + min(q, p.S - 1)] : 0;
+    const int ds_tile = kDocs ? p.doc_start[(int64_t)b * p.S + min(q0 + kTile - 1, p.S - 1)] : 0;
+    for (int j = 0; j < n_kv; ++j) {
+      const int st = j & 1;
+      const int kv0 = (j_begin + j) * kTile;
+      const bool full_tile = q_tile_full(p.S, Pb, ds_tile, q0, kv0);
+      mbar_wait(&s_full[st], (j >> 1) & 1);
+      tc_fence_after();
+      const uint32_t tS = tmem_S + st * 128 + lane_off;
+      uint32_t pr[64];   // P of this row: 128 kv columns as bf16 pairs
+      {
+        uint32_t sv[4][32];
+#pragma unroll
+        for (int c = 0; c < 4; ++c) tmem_ld_32x32(tS + c * 32, sv[c]);
+        tmem_wait_ld_regs(sv[0]);
+        tmem_wait_ld_regs(sv[1]);
+        tmem_wait_ld_regs(sv[2]);
+        tmem_wait_ld_regs(sv[3]);
+        if (!full_tile) {   // the visible keys of a row are one interval of the tile's columns (see attn_fwd_kernel)
+          const int lo = kDocs ? ds_row - kv0 : 0;
+          const uint32_t width = (uint32_t)max(min(p.S, max(Pb, q + 1)) - kv0 - lo, 0);
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if ((uint32_t)(c * 32 + i - lo) >= width) sv[c][i] = 0xff800000u;  // -inf
+        }
+#pragma unroll
+        for (int c = 0; c < 4; ++c)
+#pragma unroll
+          for (int i = 0; i < 32; i += 2)
+            pr[c * 16 + i / 2] = pack_bf16(ex2(fmaf(__uint_as_float(sv[c][i]), p.scale_log2, -lse2)),
+                                           ex2(fmaf(__uint_as_float(sv[c][i + 1]), p.scale_log2, -lse2)));
+      }
+      mbar_wait(dp_full, j & 1);
+      tc_fence_after();
+#pragma unroll
+      for (int c = 0; c < 4; ++c) {
+        uint32_t dv[32], dsr[16];
+        tmem_ld_32x32(tmem_dP + lane_off + c * 32, dv);
+        tmem_wait_ld_regs(dv);
+#pragma unroll
+        for (int i = 0; i < 32; i += 2) {
+          const uint32_t p01 = pr[c * 16 + i / 2];
+          dsr[i / 2] = pack_bf16(bf16_lo(p01) * fmaf(__uint_as_float(dv[i]), p.scale, -dlt),
+                                 bf16_hi(p01) * fmaf(__uint_as_float(dv[i + 1]), p.scale, -dlt));
+        }
+        // dS (bf16 pairs) over the score columns of this row: A operand of dQ(j), read straight from TMEM
+        tmem_st_32x16(tS + c * 16, dsr);
+      }
+      tmem_wait_st();
+      tc_fence_before();
+      __syncwarp();
+      if (lane_id() == 0) mbar_arrive(ds_full);
+    }
+    // epilogue: dQ row (fp32, TMEM) -> RoPE backward -> bf16
+    mbar_wait(dq_done, 0);
+    tc_fence_after();
+    __nv_bfloat16* drow = dq + ((int64_t)b * p.S + q) * lddq + (int64_t)h * kD;
+#pragma unroll 1
+    for (int c = 0; c < kD / 32; ++c) {
+      uint32_t v[32];
+      tmem_ld_32x32(tmem_dQ + lane_off + c * 32, v);
+      tmem_wait_ld_regs(v);
+      if (row_ok && p.rope != nullptr) {
+        const float4* cs = reinterpret_cast<const float4*>(p.rope + ((int64_t)q * (kD / 2) + c * 16) * 2);
+#pragma unroll
+        for (int i = 0; i < 32; i += 4) {
+          const float4 t4 = cs[i / 4];   // (c0, s0, c1, s1)
+          const float g0 = __uint_as_float(v[i]), g1 = __uint_as_float(v[i + 1]);
+          const float g2 = __uint_as_float(v[i + 2]), g3 = __uint_as_float(v[i + 3]);
+          v[i] = __float_as_uint(g0 * t4.x + g1 * t4.y);
+          v[i + 1] = __float_as_uint(g1 * t4.x - g0 * t4.y);
+          v[i + 2] = __float_as_uint(g2 * t4.z + g3 * t4.w);
+          v[i + 3] = __float_as_uint(g3 * t4.z - g2 * t4.w);
+        }
+      }
+      if (row_ok) {
+#pragma unroll
+        for (int i = 0; i < 32; i += 8) {
+          uint4 o4;
+          o4.x = pack_bf16(__uint_as_float(v[i]), __uint_as_float(v[i + 1]));
+          o4.y = pack_bf16(__uint_as_float(v[i + 2]), __uint_as_float(v[i + 3]));
+          o4.z = pack_bf16(__uint_as_float(v[i + 4]), __uint_as_float(v[i + 5]));
+          o4.w = pack_bf16(__uint_as_float(v[i + 6]), __uint_as_float(v[i + 7]));
+          stg_v4(drow + c * 32 + i, o4);
+        }
+      }
+    }
+    tc_fence_before();
   }
 
   tc_fence_before();
@@ -2381,15 +2679,19 @@ int llamax_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
   return 0;
 }
 
-int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
-                    const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
-                    int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* dq_accum, void* delta,
-                    int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
-                    const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
-                    const void* rope_inverse, void* stream) {
+}  // extern "C"
+
+// dq_accum == NULL: deterministic mode (attn_bwd_dq_kernel writes dq, attn_bwd_kernel<.., kNoDQ> dk / dv)
+static int attn_bwd_run(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                        const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
+                        int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* dq_accum, void* delta,
+                        int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
+                        const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
+                        const void* rope_inverse, void* stream) {
+  const bool det = dq_accum == nullptr;
   if ((doc_start == nullptr) != (doc_end == nullptr))
     return set_error(LLAMAX_ERR_ARG, "attn_bwd: doc_start and doc_end go together");
-  if (!q || !k || !v || !lse || !dout || !dq || !dk || !dv || !dq_accum || !delta)   // o may be NULL: delta is given
+  if (!q || !k || !v || !lse || !dout || !dq || !dk || !dv || !delta)   // o may be NULL: delta is given
     return set_error(LLAMAX_ERR_ARG, "attn_bwd: null pointer");
   int rc = check_attn_args(B, S, Hq, Hkv, D, prefix_len, "attn_bwd");
   if (rc) return rc;
@@ -2397,8 +2699,10 @@ int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
     return set_error(LLAMAX_ERR_ARG, "attn_bwd: pitches must be multiples of 8");
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t rows = B * S;
-  cudaError_t e = cudaMemsetAsync(dq_accum, 0, (size_t)rows * Hq * D * sizeof(float), st);
-  if (e != cudaSuccess) return set_cuda_error(e, "attn_bwd: memset");
+  if (!det) {
+    cudaError_t e = cudaMemsetAsync(dq_accum, 0, (size_t)rows * Hq * D * sizeof(float), st);
+    if (e != cudaSuccess) return set_cuda_error(e, "attn_bwd: memset");
+  }
   if (o != nullptr) {
     const int groups = (int)ceil_div(Hq, 32 / (D / 8));   // warps per row
     dim3 dgrid((unsigned)rows, (unsigned)ceil_div(groups, 8));
@@ -2415,8 +2719,10 @@ int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
   if ((rc = make_head_tmap(&tdo, dout, lddo, B, S, Hq, D, bwd::kQ))) return rc;
   if ((rc = make_head_tmap(&tk, k, ldk, B, S, Hkv, D, bwd::kKV))) return rc;
   if ((rc = make_head_tmap(&tv, v, ldv, B, S, Hkv, D, bwd::kKV))) return rc;
-  auto kern = doc_start ? (D == 128 ? attn_bwd_kernel<true, 128> : attn_bwd_kernel<true, 64>)
-                        : (D == 128 ? attn_bwd_kernel<false, 128> : attn_bwd_kernel<false, 64>);
+  auto kern = det ? (doc_start ? (D == 128 ? attn_bwd_kernel<true, 128, true> : attn_bwd_kernel<true, 64, true>)
+                               : (D == 128 ? attn_bwd_kernel<false, 128, true> : attn_bwd_kernel<false, 64, true>))
+                  : (doc_start ? (D == 128 ? attn_bwd_kernel<true, 128> : attn_bwd_kernel<true, 64>)
+                               : (D == 128 ? attn_bwd_kernel<false, 128> : attn_bwd_kernel<false, 64>));
   if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), bwd::kSmemBytes, "attn_bwd: cudaFuncSetAttribute"))) return rc;
   AttnBwdParams p;
   p.lse = (const float*)lse;
@@ -2434,8 +2740,18 @@ int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
   p.rope = (const float*)rope_inverse;
   p.prefix_b = (const int32_t*)prefix_len_b;
   dim3 grid(Hkv, (unsigned)ceil_div(S, bwd::kKV), (unsigned)B);
-  kern<<<grid, bwd::kThreads, bwd::kSmemBytes, st>>>(tq, tk, tv, tdo, p);
+  kern<<<grid, det ? bwd::kThreadsNoDQ : bwd::kThreads, bwd::kSmemBytes, st>>>(tq, tk, tv, tdo, p);
   LX_CHECK_LAUNCH("attn_bwd");
+  if (det) {
+    auto kdq = doc_start ? (D == 128 ? attn_bwd_dq_kernel<true, 128> : attn_bwd_dq_kernel<true, 64>)
+                         : (D == 128 ? attn_bwd_dq_kernel<false, 128> : attn_bwd_dq_kernel<false, 64>);
+    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kdq), bwdq::kSmemBytes, "attn_bwd: cudaFuncSetAttribute")))
+      return rc;
+    dim3 qgrid(Hq, (unsigned)B, (unsigned)ceil_div(S, bwdq::kTile));
+    kdq<<<qgrid, bwdq::kThreads, bwdq::kSmemBytes, st>>>(tq, tk, tv, tdo, p, (__nv_bfloat16*)dq, lddq);
+    LX_CHECK_LAUNCH("attn_bwd: dq");
+    return 0;
+  }
   {
     dim3 cgrid((unsigned)(B * Hq), (unsigned)ceil_div(S * (D / 8), 512));
     if (D == 128)
@@ -2447,6 +2763,29 @@ int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
     LX_CHECK_LAUNCH("attn_bwd: dq convert");
   }
   return 0;
+}
+
+extern "C" {
+
+int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                    const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
+                    int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* dq_accum, void* delta,
+                    int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
+                    const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
+                    const void* rope_inverse, void* stream) {
+  if (!dq_accum) return set_error(LLAMAX_ERR_ARG, "attn_bwd: null pointer");
+  return attn_bwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, dout, lddo, dq, lddq, dk, lddk, dv, lddv, dq_accum, delta,
+                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, stream);
+}
+
+int llamax_attn_bwd_deterministic(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                                  const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
+                                  int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* delta, int64_t B,
+                                  int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
+                                  const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
+                                  const void* rope_inverse, void* stream) {
+  return attn_bwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, dout, lddo, dq, lddq, dk, lddk, dv, lddv, nullptr, delta,
+                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, stream);
 }
 
 }  // extern "C"

@@ -8,6 +8,7 @@
 #include <algorithm>
 
 #include <cstdlib>
+#include <type_traits>
 
 #include "llamax_b200.h"
 
@@ -847,13 +848,21 @@ rmsnorm_bwd_ring_kernel(const __nv_bfloat16* __restrict__ dy, const __nv_bfloat1
   }
 }
 
-__global__ void reduce_partials_kernel(const float* __restrict__ partial, __nv_bfloat16* __restrict__ out, int nparts,
-                                       int64_t D) {
+// out[d] = sum_p partial[p, d], summed in part order: bf16 out (RMSNorm dw), fp32 out (deterministic lora_wgrad)
+template <typename T = __nv_bfloat16>
+__global__ void reduce_partials_kernel(const float* __restrict__ partial, T* __restrict__ out, int nparts, int64_t D) {
   const int64_t d = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (d >= D) return;
   float s = 0.f;
   for (int p = 0; p < nparts; ++p) s += partial[(int64_t)p * D + d];
-  out[d] = __float2bfloat16_rn(s);
+  if constexpr (std::is_same_v<T, float>) out[d] = s;
+  else out[d] = __float2bfloat16_rn(s);
+}
+
+int launch_reduce_partials_f32(const float* partial, float* out, int nparts, int64_t D, cudaStream_t stream) {
+  reduce_partials_kernel<float><<<(unsigned)((D + 255) / 256), 256, 0, stream>>>(partial, out, nparts, D);
+  LX_CHECK_LAUNCH("reduce_partials");
+  return 0;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -970,6 +979,9 @@ dequant_transpose_kernel(const int8_t* __restrict__ w8, const __nv_bfloat16* __r
 // logits <- (softmax - onehot(label)) * inv_n   (0 for ignored rows, label == -100).
 // One CTA per row: one HBM read (online max/sum), one L2 re-read + one write. No fp32 [M, vocab] tensor.
 // ------------------------------------------------------------------------------------------------
+// kRowLoss (deterministic mode): loss_sum is an fp32 [M] buffer that receives each row's loss (0 for ignored rows),
+// summed in a fixed order by the caller, instead of one scalar accumulated with fp32 atomics in CTA completion order.
+template <bool kRowLoss = false>
 __global__ void __launch_bounds__(512)
 cross_entropy_kernel(__nv_bfloat16* __restrict__ logits, int64_t ld, const int64_t* __restrict__ labels,
                      float* __restrict__ loss_sum, const float* __restrict__ inv_n, int V, int write_grad) {
@@ -979,6 +991,9 @@ cross_entropy_kernel(__nv_bfloat16* __restrict__ logits, int64_t ld, const int64
   const int64_t label = labels[row];
   const int nvec = V / 8;
   if (label < 0) {  // ignore_index
+    if constexpr (kRowLoss) {
+      if (threadIdx.x == 0) loss_sum[row] = 0.f;
+    }
     if (write_grad)
       for (int i = threadIdx.x; i < nvec; i += blockDim.x) *reinterpret_cast<uint4*>(lr + (int64_t)i * 8) = make_uint4(0, 0, 0, 0);
     return;
@@ -1013,7 +1028,11 @@ cross_entropy_kernel(__nv_bfloat16* __restrict__ logits, int64_t ld, const int64
   float S_ = 0.f;
   for (int i = 0; i < nw; ++i) S_ += (sm_m[i] == -INFINITY) ? 0.f : sm_s[i] * __expf(sm_m[i] - M_);
   const float lse = M_ + logf(S_);
-  if (threadIdx.x == 0) atomicAdd(loss_sum, lse - __bfloat162float(lr[label]));
+  if constexpr (kRowLoss) {
+    if (threadIdx.x == 0) loss_sum[row] = lse - __bfloat162float(lr[label]);
+  } else {
+    if (threadIdx.x == 0) atomicAdd(loss_sum, lse - __bfloat162float(lr[label]));
+  }
   if (!write_grad) return;
   const float scale = *inv_n;
   __syncthreads();  // every thread has read lr[label]-independent data; row is rewritten below
@@ -1381,6 +1400,18 @@ int llamax_cross_entropy(void* logits, int64_t ld, const void* labels, void* los
   cross_entropy_kernel<<<(unsigned)M, 512, 0, (cudaStream_t)stream>>>((bf16*)logits, ld, (const int64_t*)labels,
                                                                       (float*)loss_sum, (const float*)inv_n, (int)V,
                                                                       write_grad);
+  LX_CHECK_LAUNCH("cross_entropy");
+  return 0;
+}
+
+int llamax_cross_entropy_rows(void* logits, int64_t ld, const void* labels, void* loss_rows, const void* inv_n,
+                              int64_t M, int64_t V, int write_grad, void* stream) {
+  if (!logits || !labels || !loss_rows || (write_grad && !inv_n)) return set_error(LLAMAX_ERR_ARG, "cross_entropy: null pointer");
+  if (V % 8 || ld % 8) return set_error(LLAMAX_ERR_ARG, "cross_entropy: V and ld must be multiples of 8");
+  if (M == 0) return 0;
+  cross_entropy_kernel<true><<<(unsigned)M, 512, 0, (cudaStream_t)stream>>>((bf16*)logits, ld, (const int64_t*)labels,
+                                                                            (float*)loss_rows, (const float*)inv_n,
+                                                                            (int)V, write_grad);
   LX_CHECK_LAUNCH("cross_entropy");
   return 0;
 }

@@ -1312,6 +1312,9 @@ constexpr int kStageBytes = kABytes + kBBytes;
 constexpr int kSmem = kStages * kStageBytes + (2 * kStages + 1) * 8 + 16 + 1024;
 }  // namespace wg
 
+// kPartials (deterministic mode): split s stores its partial with plain stores into out[s, P, R]; the splits are then
+// summed in split order by reduce_partials_kernel instead of with order-dependent fp32 atomics.
+template <bool kPartials = false>
 __global__ void __launch_bounds__(192, 1)
 lora_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmHt,
                      float* __restrict__ out, int P, int R, int M, int k_per_split, float alpha) {
@@ -1389,7 +1392,21 @@ lora_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
     // epilogue warps 2..5: TMEM lanes 32*(warp % 4)
     const int lq = warp & 3;
     const int row = p0 + lq * 32 + lane_id();
-    if (num_kb > 0) {
+    if constexpr (kPartials) {
+      uint32_t v[32] = {};
+      if (num_kb > 0) {
+        mbar_wait(done_bar, 0);
+        tc_fence_after();
+        tmem_ld_32x32(tmem_base + (uint32_t(lq * 32) << 16), v);
+        tmem_wait_ld_regs(v);
+      }
+      if (row < P) {
+        float* dst = out + ((int64_t)blockIdx.y * P + row) * R;
+#pragma unroll
+        for (int r = 0; r < 32; ++r)
+          if (r < R) dst[r] = alpha * __uint_as_float(v[r]);
+      }
+    } else if (num_kb > 0) {
       mbar_wait(done_bar, 0);
       tc_fence_after();
       uint32_t v[32];
@@ -1842,36 +1859,21 @@ int llamax_bf16_gemm(const void* A, int64_t lda, const void* B, int64_t ldb, voi
                         : launch_gemm<false, 1>(A, lda, B, ldb, p, (cudaStream_t)stream);
 }
 
-int llamax_lora_wgrad(const void* X, int64_t ldx, const void* Ht, int64_t ldht, void* out, int64_t M, int64_t P,
-                      int32_t R, float alpha, void* stream) {
-  if (!X || !Ht || !out) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: null pointer");
-  if (R < 1 || R > 32) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: rank must be in [1, 32]");
-  if (M <= 0 || P <= 0) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: empty problem");
-  if (ldx % 8 || ldht % 8 || (reinterpret_cast<uintptr_t>(X) % 16) || (reinterpret_cast<uintptr_t>(Ht) % 16))
-    return set_error(LLAMAX_ERR_ARG, "lora_wgrad: X / H^T must be 16-byte aligned with pitches multiple of 8");
-  cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t e = cudaMemsetAsync(out, 0, (size_t)P * R * sizeof(float), st);
-  if (e != cudaSuccess) return set_cuda_error(e, "lora_wgrad: memset");
-  CUtensorMap tmX, tmHt;
-  int rc = make_tmap_2d(&tmX, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, X, P, M, ldx, 64, 64);
-  if (rc) return rc;
-  rc = make_tmap_2d(&tmHt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, Ht, M, R, ldht, 64, 32);
-  if (rc) return rc;
-  if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(lora_wgrad_tc_kernel), wg::kSmem, "lora_wgrad: cudaFuncSetAttribute")))
-    return rc;
-  const int p_tiles = (int)((P + 127) / 128);
-  // Token splits: one CTA per SM is resident (147 KB ring), so the kernel lasts waves x (tokens per split + a fixed
-  // fill/drain cost of ~5 stages). Pick the split count that minimises that: "just enough CTAs to cover the SMs" left a
-  // nearly empty second wave (P = 4096: 32 tiles x 5 splits = 160 CTAs on 148 SMs; 9 splits = 288 CTAs, two full waves
-  // of half the length). LLAMAX_WGRAD_SPLITS_OLD=1 keeps the old rule (A/B).
+}  // extern "C"
+
+// Token splits of lora_wgrad: one CTA per SM is resident (147 KB ring), so the kernel lasts waves x (tokens per split + a
+// fixed fill/drain cost of ~5 stages). Pick the split count that minimises that: "just enough CTAs to cover the SMs" left
+// a nearly empty second wave (P = 4096: 32 tiles x 5 splits = 160 CTAs on 148 SMs; 9 splits = 288 CTAs, two full waves
+// of half the length). LLAMAX_WGRAD_SPLITS_OLD=1 keeps the old rule (A/B). At most LLAMAX_LORA_WGRAD_MAX_SPLITS splits.
+static void lora_wgrad_splits(int64_t M, int p_tiles, int& splits, int& k_per_split) {
   static const bool old_rule = getenv("LLAMAX_WGRAD_SPLITS_OLD") != nullptr;
-  int splits = std::max(1, std::min(32, (sm_count() + p_tiles - 1) / p_tiles));
-  int k_per_split = (int)((M + splits - 1) / splits);
+  splits = std::max(1, std::min(LLAMAX_LORA_WGRAD_MAX_SPLITS, (sm_count() + p_tiles - 1) / p_tiles));
+  k_per_split = (int)((M + splits - 1) / splits);
   k_per_split = ((k_per_split + 63) / 64) * 64;
   splits = (int)((M + k_per_split - 1) / k_per_split);
   if (!old_rule && p_tiles * 2 <= sm_count()) {   // wide outputs (P = 14336) stream at HBM rate either way: 79 vs 81 us
     int64_t best_cost = INT64_MAX;
-    for (int s = 1; s <= 32; ++s) {
+    for (int s = 1; s <= LLAMAX_LORA_WGRAD_MAX_SPLITS; ++s) {
       int kp = (int)((M + s - 1) / s);
       kp = ((kp + 63) / 64) * 64;
       const int s_eff = (int)((M + kp - 1) / kp);
@@ -1881,10 +1883,51 @@ int llamax_lora_wgrad(const void* X, int64_t ldx, const void* Ht, int64_t ldht, 
       if (cost < best_cost) { best_cost = cost; splits = s; k_per_split = kp; }
     }
   }
+}
+
+// workspace == NULL: splits are reduced into `out` with fp32 atomics; else the deterministic form (partials + ordered sum)
+static int lora_wgrad_run(const void* X, int64_t ldx, const void* Ht, int64_t ldht, void* out, void* workspace, int64_t M,
+                          int64_t P, int32_t R, float alpha, void* stream) {
+  if (!X || !Ht || !out) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: null pointer");
+  if (R < 1 || R > 32) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: rank must be in [1, 32]");
+  if (M <= 0 || P <= 0) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: empty problem");
+  if (ldx % 8 || ldht % 8 || (reinterpret_cast<uintptr_t>(X) % 16) || (reinterpret_cast<uintptr_t>(Ht) % 16))
+    return set_error(LLAMAX_ERR_ARG, "lora_wgrad: X / H^T must be 16-byte aligned with pitches multiple of 8");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (workspace == nullptr) {
+    cudaError_t e = cudaMemsetAsync(out, 0, (size_t)P * R * sizeof(float), st);
+    if (e != cudaSuccess) return set_cuda_error(e, "lora_wgrad: memset");
+  }
+  CUtensorMap tmX, tmHt;
+  int rc = make_tmap_2d(&tmX, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, X, P, M, ldx, 64, 64);
+  if (rc) return rc;
+  rc = make_tmap_2d(&tmHt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, Ht, M, R, ldht, 64, 32);
+  if (rc) return rc;
+  auto kern = workspace ? lora_wgrad_tc_kernel<true> : lora_wgrad_tc_kernel<false>;
+  if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), wg::kSmem, "lora_wgrad: cudaFuncSetAttribute")))
+    return rc;
+  const int p_tiles = (int)((P + 127) / 128);
+  int splits, k_per_split;
+  lora_wgrad_splits(M, p_tiles, splits, k_per_split);
   dim3 grid(p_tiles, splits);
-  lora_wgrad_tc_kernel<<<grid, 192, wg::kSmem, st>>>(tmX, tmHt, (float*)out, (int)P, R, (int)M, k_per_split, alpha);
+  kern<<<grid, 192, wg::kSmem, st>>>(tmX, tmHt, (float*)(workspace ? workspace : out), (int)P, R, (int)M, k_per_split,
+                                     alpha);
   LX_CHECK_LAUNCH("lora_wgrad");
+  if (workspace) return launch_reduce_partials_f32((const float*)workspace, (float*)out, splits, P * R, st);
   return 0;
+}
+
+extern "C" {
+
+int llamax_lora_wgrad(const void* X, int64_t ldx, const void* Ht, int64_t ldht, void* out, int64_t M, int64_t P,
+                      int32_t R, float alpha, void* stream) {
+  return lora_wgrad_run(X, ldx, Ht, ldht, out, nullptr, M, P, R, alpha, stream);
+}
+
+int llamax_lora_wgrad_deterministic(const void* X, int64_t ldx, const void* Ht, int64_t ldht, void* out,
+                                    void* workspace, int64_t M, int64_t P, int32_t R, float alpha, void* stream) {
+  if (!workspace) return set_error(LLAMAX_ERR_ARG, "lora_wgrad: null pointer");
+  return lora_wgrad_run(X, ldx, Ht, ldht, out, workspace, M, P, R, alpha, stream);
 }
 
 int llamax_lora_bwd_pair(const void* dY, int64_t lddy, const void* Bt, int64_t ldbt, const void* Ht, int64_t ldht,

@@ -25,6 +25,9 @@ int make_tmap_4d(CUtensorMap* map, CUtensorMapDataType dt, int esz, const void* 
 // second GPU of the same thread with the 48 KB default).
 int ensure_dyn_smem(const void* kernel, int bytes, const char* who);
 
+// out[d] (fp32) = sum_p partial[p, d] in part order (elementwise.cu; the deterministic lora_wgrad's split reduction)
+int launch_reduce_partials_f32(const float* partial, float* out, int nparts, int64_t D, cudaStream_t stream);
+
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 }  // namespace lx

@@ -329,14 +329,20 @@ def _lora_prepare(items, M: int, device, groups=()):
 
 def _group_mergeable(specs) -> bool:
     r_tot = sum(s.R for s in specs)
-    return (_LORA_PAIR and _LORA_GROUP_PAIR and len(specs) > 1 and all(s.R > 0 for s in specs) and r_tot <= 32
+    return (_lora_pair() and _LORA_GROUP_PAIR and len(specs) > 1 and all(s.R > 0 for s in specs) and r_tot <= 32
             and all(s.lora_scale == specs[0].lora_scale for s in specs) and all(s.N % 8 == 0 for s in specs))
+
+
+def _lora_pair() -> bool:
+    """lora_bwd_pair reduces dB and dh across CTAs with fp32 atomics: under torch.use_deterministic_algorithms the
+    two-pass form runs instead (the skinny dh GEMM streams each contraction in one CTA; lora_wgrad's deterministic form)."""
+    return _LORA_PAIR and not ops.deterministic_mode()
 
 
 def _lora_dh_dB(dy: Tensor, bt: Tensor, ht: Tensor, out_dh: Tensor, scale: float, out_dht: Tensor) -> Tensor:
     """out_dh = dy @ bt^T (bt already carries the LoRA scale), out_dht = out_dh^T (operand of the dA weight
     gradient), returns dB = scale * dy^T h (fp32)."""
-    if _LORA_PAIR:
+    if _lora_pair():
         return ops.lora_bwd_pair(dy, bt, None, out_dh, scale, Ht=ht, out_dht=out_dht)
     ops.bf16_gemm(dy, bt, out=out_dh)
     out_dht.copy_(out_dh.t())

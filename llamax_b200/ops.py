@@ -124,6 +124,13 @@ def make_epilogue(lora_h=None, lora_b=None, lora_scale=1.0, resid=None, lora_seg
     return ep, keep
 
 
+def deterministic_mode(deterministic: bool | None = None) -> bool:
+    """Whether a launch takes its deterministic form: `deterministic` when given, else PyTorch's own switch
+    (torch.use_deterministic_algorithms). Deterministic forms give bitwise identical results from run to run on the same
+    GPU: no fp32 reduction whose order depends on which CTA finishes first."""
+    return torch.are_deterministic_algorithms_enabled() if deterministic is None else bool(deterministic)
+
+
 def set_gemm_cta_group(cg: int):
     check(_lib.load().llamax_set_gemm_cta_group(cg), "llamax_set_gemm_cta_group")
 
@@ -460,9 +467,13 @@ def transposed_rank_buffer(R: int, M: int, device) -> Tensor:
     return torch.zeros(R, Mp, device=device, dtype=torch.bfloat16)[:, :M]
 
 
-def lora_wgrad(X: Tensor, H: Tensor | None, alpha: float = 1.0, *, Ht: Tensor | None = None) -> Tensor:
+def lora_wgrad(X: Tensor, H: Tensor | None, alpha: float = 1.0, *, Ht: Tensor | None = None,
+               deterministic: bool | None = None) -> Tensor:
     """out[P,R] (fp32) = alpha * X[M,P]^T @ H[M,R]  (tensor cores; X is consumed in place). Pass Ht = H^T [R,M]
-    (from transposed_rank_buffer) when it already exists; otherwise it is made here (a tiny copy)."""
+    (from transposed_rank_buffer) when it already exists; otherwise it is made here (a tiny copy).
+    deterministic (None: torch.are_deterministic_algorithms_enabled()): the token splits store partials into a
+    workspace that is summed in split order, instead of fp32 atomics."""
+    det = deterministic_mode(deterministic)
     lib, st = _prep(X)
     assert X.dtype is torch.bfloat16 and X.stride(1) == 1
     M, Pn = X.shape
@@ -473,8 +484,14 @@ def lora_wgrad(X: Tensor, H: Tensor | None, alpha: float = 1.0, *, Ht: Tensor | 
     R = Ht.shape[0]
     assert Ht.dtype is torch.bfloat16 and Ht.shape[1] == M and Ht.stride(1) == 1
     if R > 32:   # the kernel's accumulator is 32 columns wide: wider rank groups (e.g. q|k|v at rank 16) go in chunks
-        return torch.cat([lora_wgrad(X, None, alpha, Ht=Ht[r0 : r0 + 32]) for r0 in range(0, R, 32)], 1)
+        return torch.cat([lora_wgrad(X, None, alpha, Ht=Ht[r0 : r0 + 32], deterministic=det) for r0 in range(0, R, 32)], 1)
     out = torch.empty(Pn, R, device=X.device, dtype=torch.float32)
+    if det:
+        ws = torch.empty(_lib.LORA_WGRAD_MAX_SPLITS, Pn, R, device=X.device, dtype=torch.float32)
+        _call(lib, "llamax_lora_wgrad_deterministic",
+              (_p(X), X.stride(0), _p(Ht), Ht.stride(0), _p(out), _p(ws), M, Pn, R, float(alpha), st),
+              "lora_wgrad_det", 2.0 * M * Pn * R, 2.0 * M * (Pn + R))
+        return out
     _call(lib, "llamax_lora_wgrad",
           (_p(X), X.stride(0), _p(Ht), Ht.stride(0), _p(out), M, Pn, R, float(alpha), st),
           "lora_wgrad", 2.0 * M * Pn * R, 2.0 * M * (Pn + R))
@@ -561,14 +578,24 @@ def batched_copy(jobs) -> None:
         _call(lib, "llamax_batched_copy", (arr, len(chunk), st), "batched_copy", 0.0, 0.0)
 
 
-def cross_entropy_(logits: Tensor, labels: Tensor, loss_sum: Tensor, inv_n: Tensor | None, write_grad: bool):
+def cross_entropy_(logits: Tensor, labels: Tensor, loss_sum: Tensor, inv_n: Tensor | None, write_grad: bool, *,
+                   deterministic: bool | None = None):
     """In place: accumulates sum of per-row CE into loss_sum (fp32 scalar tensor); if write_grad, overwrites logits
-    with (softmax - onehot) * inv_n (rows with label -100 -> 0)."""
+    with (softmax - onehot) * inv_n (rows with label -100 -> 0).
+    deterministic (None: torch.are_deterministic_algorithms_enabled()): the row losses go to an fp32 [M] buffer and are
+    summed in a fixed order, instead of fp32 atomics in CTA completion order."""
     lib, st = _prep(logits)
     assert logits.dtype is torch.bfloat16 and logits.dim() == 2 and logits.stride(1) == 1
     assert labels.dtype is torch.int64 and labels.is_contiguous() and labels.numel() == logits.shape[0]
     assert loss_sum.dtype is torch.float32 and (inv_n is None or inv_n.dtype is torch.float32)
     M, V = logits.shape
+    if deterministic_mode(deterministic):
+        rows = torch.empty(M, device=logits.device, dtype=torch.float32)
+        _call(lib, "llamax_cross_entropy_rows",
+              (_p(logits), logits.stride(0), _p(labels), _p(rows), _p(inv_n), M, V, int(write_grad), st),
+              "cross_entropy_det", 0.0, (4.0 if write_grad else 2.0) * M * V)
+        loss_sum += rows.sum()   # fixed-order tree reduction for a given M
+        return
     _call(lib, "llamax_cross_entropy",
           (_p(logits), logits.stride(0), _p(labels), _p(loss_sum), _p(inv_n), M, V, int(write_grad), st),
           "cross_entropy", 0.0, (4.0 if write_grad else 2.0) * M * V)
@@ -625,16 +652,19 @@ def attn_fwd(q: Tensor, k: Tensor, v: Tensor, B: int, S: int, Hq: int, Hkv: int,
 
 
 def attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, prefix_len, scale=None, doc_start=None,
-             doc_end=None, rope_inverse=None, delta=None):
+             doc_end=None, rope_inverse=None, delta=None, *, deterministic: bool | None = None):
     """Writes dq/dk/dv (row views like q/k/v). rope_inverse: fp32 [>= S, D/2, 2] table -> dq, dk come back already
     rotated through the RoPE backward (no separate rope_(..., inverse=True) pass needed). delta: fp32 [B, Hq, S] =
-    sum_d dout * o already computed (bf16_gemm_rowdot): o is then not read and may be None."""
+    sum_d dout * o already computed (bf16_gemm_rowdot): o is then not read and may be None.
+    deterministic (None: torch.are_deterministic_algorithms_enabled()): dq from a kernel that sums the kv tiles of each
+    query tile in a fixed order (it recomputes the S and dP products) instead of fp32 atomics; dk, dv are unchanged."""
+    det = deterministic_mode(deterministic)
     if rope_inverse is not None:
         assert rope_inverse.dtype is torch.float32 and rope_inverse.is_contiguous()
         assert rope_inverse.shape[0] >= S and rope_inverse.shape[1] == D // 2
     lib, st = _prep(q)
     dout = _rows(dout)
-    dq_accum = torch.empty(B * S, Hq * D, device=q.device, dtype=torch.float32)
+    dq_accum = None if det else torch.empty(B * S, Hq * D, device=q.device, dtype=torch.float32)
     if delta is None:
         delta = torch.empty(B, Hq, S, device=q.device, dtype=torch.float32)
     else:
@@ -642,6 +672,11 @@ def attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, prefix_len, sc
         o = None
     scale = float(scale) if scale is not None else D ** -0.5
     p_scalar, p_b = _prefix_args(prefix_len, B, q.device)
+    if det:
+        _call(lib, "llamax_attn_bwd_deterministic",
+              (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0) if o is not None else 0, _p(lse), _p(dout), dout.stride(0), _p(dq), dq.stride(0), _p(dk), dk.stride(0), _p(dv), dv.stride(0), _p(delta), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), _p(doc_end), scale, _p(rope_inverse), st,),
+              "attn_bwd_det", 14.0 * B * Hq * D * _pairs(S, prefix_len), 0.0)
+        return dq, dk, dv
     _call(lib, "llamax_attn_bwd",
           (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0) if o is not None else 0, _p(lse), _p(dout), dout.stride(0), _p(dq), dq.stride(0), _p(dk), dk.stride(0), _p(dv), dv.stride(0), _p(dq_accum), _p(delta), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), _p(doc_end), scale, _p(rope_inverse), st,),
           "attn_bwd", 10.0 * B * Hq * D * _pairs(S, prefix_len), 0.0)
