@@ -9,13 +9,13 @@
 //
 // Optional packed-sequence document mask: additionally kv >= doc_start[q] (tiles outside a row's document skipped).
 //
-// Forward  : default = attn_fwd5_kernel, persistent: one CTA per SM walks a length-balanced list of items (pair of
-//            128-row query tiles, query head, sequence); warp0 TMA, warps1-2 MMA issue (one per tile), two softmax
-//            warpgroups (thread = row). Per tile S = Q K^T in TMEM is read once into registers, P (bf16 pairs) is written
-//            back over the score columns in four chunks and consumed by the PV MMA straight from TMEM, O accumulates
-//            in TMEM with lazy rescaling; exp2-domain online softmax, LSE saved in natural log. Older forms kept behind
-//            LLAMAX_ATTN_FWD (1: one tile per CTA, 2: two tiles / one issuer — also the packed-document path, 3: two
-//            threads per row, 4: v5 without the persistent loop).
+// Forward  : two 128-row query tiles per CTA, two softmax warpgroups (thread = row). Per tile S = Q K^T in TMEM is read
+//            once into registers, P (bf16 pairs) is written back over the score columns and consumed by the PV MMA
+//            straight from TMEM, O accumulates in TMEM with lazy rescaling; exp2-domain online softmax, LSE saved in
+//            natural log. attn_fwd5_kernel is persistent: one CTA per SM walks a length-balanced list of items (pair of
+//            query tiles, query head, sequence); warp0 TMA, warps1-2 MMA issue (one per tile), P handed over in four
+//            chunks. With packed documents attn_fwd2_kernel runs instead: one CTA per pair of query tiles, one MMA
+//            issuer, each tile starting at its own document's first kv tile.
 // Backward : CTA = (128 kv rows, 1 kv head), loops over the group's query heads x 128-row query tiles; every MMA is
 //            128 x 128 x 16. S^T = K Q^T and dP^T = V dO^T in TMEM (thread = kv row); P^T goes back to TMEM as bf16 pairs
 //            (A operand of dV += P^T dO straight from TMEM), dS^T through smem (dK += dS^T Q, dQ^T = K^T dS^T); dV, dK
@@ -78,344 +78,42 @@ struct AttnFwdParams {
   const int32_t* prefix_b;   // null, or [B]: per-sequence prefix length (overrides P)
 };
 
+// Layout and thread roles of both forward kernels: a CTA holds two 128-row query tiles, each with its own softmax
+// warpgroup, and double-buffered K / V tiles; warpgroup 0 does TMA, MMA issue and TMEM allocation.
 namespace fwd {
 constexpr int kTile = 128;
-constexpr int kTileBytes = kTile * kHD * 2;       // 32 KB: two 16 KB boxes of [128 rows x 128 B]
-constexpr int kOffQ = 0;
-constexpr int kOffK = kOffQ + kTileBytes;         // kNB stages of K, then kNB stages of V
-constexpr int kNumBars = 1 + 4 + 4 + 4 + 2;       // q_full, k full/empty[2], v full/empty[2], s full/empty[2], p_full, pv_done
-constexpr int smem_bytes(int nb) { return kTileBytes * (1 + 2 * nb) + kNumBars * 8 + 16 + 1024; }
-constexpr int kNB = 2;                             // smem stages of K and V, TMEM score buffers
-constexpr int kThreads = 256;                     // warp0 TMA, warp1 MMA, warp2 TMEM alloc, warps 4-7 softmax
-}  // namespace fwd
-
-// Tile classification of a 128-row query tile starting at q0 (attn_fwd_kernel, attn_bwd_dq_kernel): the kv tiles it
-// visits are [j_begin, j_begin + n_kv) — up to max(P, q0 + 128), and, with packed documents, from the start of the first
-// row's document on; a visited tile needs no element test when every (q, kv) pair of it is visible and in range.
-template <bool kDocs>
-__device__ __forceinline__ void q_tile_kv_range(int S, int Pb, const int32_t* doc_start, int b, int q0, int& j_begin,
-                                                int& n_kv) {
-  const int kv_end = min(S, max(Pb, q0 + 128));
-  j_begin = kDocs ? doc_start[(int64_t)b * S + q0] / 128 : 0;
-  n_kv = (kv_end + 127) / 128 - j_begin;
-}
-// ds_tile: document start of the tile's last row (0 without documents)
-__device__ __forceinline__ bool q_tile_full(int S, int Pb, int ds_tile, int q0, int kv0) {
-  return (kv0 + 128 <= S) && ((kv0 + 128 <= Pb) || (kv0 + 127 <= q0)) && (kv0 >= ds_tile);
-}
-
-// kDocs: packed-document mask compiled in; kD: real head dim (64 runs on zero-padded 128-wide tiles).
-// (A variant with two softmax warpgroups per query tile — column halves, row maxima exchanged through smem — was
-// measured 10 % slower than this single-warpgroup version on B200: the extra 256-thread barrier per tile and the
-// doubled TMEM read contention cost more than the halved per-thread work saves.)
-// K/V are double-buffered in smem and S in TMEM (kNB = 2), one CTA per SM (160 KB smem, 512 TMEM columns).
-// P is handed to the PV MMA through TMEM: bf16 pairs written over the score columns just read, consumed by
-// tcgen05.mma with the A operand in TMEM (+9 % over staging P in 128B-swizzled smem).
-// Rejected after measurement: single buffers with two CTAs per SM and setmaxnreg register rebalancing (-12 %), and two
-// softmax warpgroups per query tile (-10 %).
-template <bool kDocs, int kD>
-__global__ void __launch_bounds__(fwd::kThreads, 1)
-attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p) {
-  using namespace fwd;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  constexpr int kOffV = kOffK + kNB * kTileBytes;
-  constexpr int kOffBar = kOffV + kNB * kTileBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
-  uint64_t* q_full = bars;
-  uint64_t* k_full = bars + 1;
-  uint64_t* k_empty = bars + 3;
-  uint64_t* v_full = bars + 5;
-  uint64_t* v_empty = bars + 7;
-  uint64_t* s_full = bars + 9;
-  uint64_t* s_empty = bars + 11;
-  uint64_t* p_full = bars + 13;
-  uint64_t* pv_done = bars + 14;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars);
-
-  const int warp = threadIdx.x >> 5;
-#ifdef LX_ATTN_TRACE
-  const bool tr_cta = (blockIdx.x | blockIdx.y | blockIdx.z) == 0 && (threadIdx.x & 31) == 0 && (warp == 1 || warp == 4);
-#endif
-  // grid = (query heads, batch, query tiles): the tile index is the slowest one and runs backwards, so CTAs are
-  // dispatched longest-first (the last query tile visits every kv tile); the 4 heads of a GQA group run together
-  const int qt = gridDim.z - 1 - blockIdx.z;
-  const int h = blockIdx.x, b = blockIdx.y;
-  const int Pb = p.prefix_b ? min(max(p.prefix_b[b], 0), p.S) : p.P;   // prefix length of this sequence
-  const int hk = h / (p.Hq / p.Hkv);
-  const int q0 = qt * kTile;
-  int j_begin, n_kv;   // visited kv tiles
-  q_tile_kv_range<kDocs>(p.S, Pb, p.doc_start, b, q0, j_begin, n_kv);
-
-  if (warp == 0 && elect_one()) {
-    tma_prefetch_desc(&tmQ);
-    tma_prefetch_desc(&tmK);
-    tma_prefetch_desc(&tmV);
-  }
-  if (warp == 1 && elect_one()) {
-    mbar_init(q_full, 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&k_full[i], 1);
-      mbar_init(&k_empty[i], 1);
-      mbar_init(&v_full[i], 1);
-      mbar_init(&v_empty[i], 1);
-      mbar_init(&s_full[i], 1);
-      mbar_init(&s_empty[i], 4);
-    }
-    mbar_init(p_full, 4);
-    mbar_init(pv_done, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) {
-    tmem_alloc<1>(tmem_slot, 256 * kNB);
-    tmem_relinquish<1>();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tmem_S = tmem_base;              // kNB x 128 columns
-  const uint32_t tmem_O = tmem_base + kNB * 128;  // 128 columns
-
-  if (warp == 0) {
-    // ------------------------------------ TMA producer ------------------------------------
-    if (elect_one()) {
-      mbar_expect_tx(q_full, kTileBytes);
-      tma_load_4d(smem + kOffQ, &tmQ, q_full, 0, h, q0, b);
-      tma_load_4d(smem + kOffQ + kTileBytes / 2, &tmQ, q_full, 64, h, q0, b);
-      for (int j = 0; j < n_kv; ++j) {
-        const int st = kNB == 2 ? (j & 1) : 0;
-        const uint32_t ph = (kNB == 2 ? (j >> 1) : j) & 1;
-        mbar_wait(&k_empty[st], ph ^ 1);
-        mbar_expect_tx(&k_full[st], kTileBytes);
-        uint8_t* sk = smem + kOffK + st * kTileBytes;
-        tma_load_4d(sk, &tmK, &k_full[st], 0, hk, (j_begin + j) * kTile, b);
-        tma_load_4d(sk + kTileBytes / 2, &tmK, &k_full[st], 64, hk, (j_begin + j) * kTile, b);
-        mbar_wait(&v_empty[st], ph ^ 1);
-        mbar_expect_tx(&v_full[st], kTileBytes);
-        uint8_t* sv = smem + kOffV + st * kTileBytes;
-        tma_load_4d(sv, &tmV, &v_full[st], 0, hk, (j_begin + j) * kTile, b);
-        tma_load_4d(sv + kTileBytes / 2, &tmV, &v_full[st], 64, hk, (j_begin + j) * kTile, b);
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    // ------------------------------------ MMA issuer ------------------------------------
-    if (elect_one()) {
-      constexpr uint32_t idesc_s = make_idesc(1, 1, 128, 128, 0, 0);
-      constexpr uint32_t idesc_pv = make_idesc(1, 1, 128, 128, 0, 1);  // B = V is MN-major
-      constexpr uint32_t kHi = desc_hi(1024);
-      const uint32_t loQ = desc_lo(smem_u32(smem + kOffQ), 16);
-      const uint32_t loK0 = desc_lo(smem_u32(smem + kOffK), 16), loV0 = desc_lo(smem_u32(smem + kOffV), 16384);
-      auto issue_s = [&](int j) {
-        const int st = kNB == 2 ? (j & 1) : 0;
-        const uint32_t ph = (kNB == 2 ? (j >> 1) : j) & 1;
-        mbar_wait(&k_full[st], ph);
-        mbar_wait(&s_empty[st], ph ^ 1);
-        tc_fence_after();
-        const uint32_t loK = loK0 + st * (kTileBytes / 16);
-#pragma unroll
-        for (int dh = 0; dh < 2; ++dh)
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks)
-            umma_ss<false, 1>(tmem_S + st * 128, desc_join(loQ + dh * 1024 + ks * 2, kHi),
-                              desc_join(loK + dh * 1024 + ks * 2, kHi), idesc_s, (dh | ks) != 0);
-        umma_commit(&s_full[st]);
-        umma_commit(&k_empty[st]);
-      };
-      mbar_wait(q_full, 0);
-      issue_s(0);
-      for (int j = 0; j < n_kv; ++j) {
-        if (kNB == 2 && j + 1 < n_kv) issue_s(j + 1);  // next scores into the other TMEM buffer
-        const int st = kNB == 2 ? (j & 1) : 0;
-        LX_TR(tr_cta, j, 0);
-        mbar_wait(&v_full[st], (kNB == 2 ? (j >> 1) : j) & 1);
-        mbar_wait(p_full, j & 1);
-        tc_fence_after();
-        LX_TR(tr_cta, j, 1);
-        const uint32_t loV = loV0 + st * (kTileBytes / 16);
-#pragma unroll
-        for (int kb = 0; kb < 2; ++kb)
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks) {
-            const uint64_t bd = desc_join(loV + (kb * 64 + ks * 16) * 8, kHi);
-            // A = P read from TMEM: bf16 pairs, 8 columns per 16-wide k-step, aliasing the score buffer
-            umma_ts_f16(tmem_O, tmem_S + st * 128 + (kb * 4 + ks) * 8, bd, idesc_pv, (j | kb | ks) != 0);
-          }
-        umma_commit(pv_done);
-        umma_commit(&v_empty[st]);
-        if (kNB == 1 && j + 1 < n_kv) issue_s(j + 1);  // single score buffer: free once PV_j (in order) consumed P_j
-      }
-    }
-    __syncwarp();
-  } else if (warp >= 4) {
-    // ------------------------------------ softmax / correction / epilogue ------------------------------------
-    const int r = threadIdx.x - 128;  // row in tile == TMEM lane
-    const int ew = warp - 4;
-    const uint32_t lane_off = uint32_t(ew * 32) << 16;
-    const int q = q0 + r;
-    float m_used = -INFINITY, l = 0.f;
-    const int ds_row = kDocs ? p.doc_start[(int64_t)b * p.S + min(q, p.S - 1)] : 0;
-    const int ds_tile = kDocs ? p.doc_start[(int64_t)b * p.S + min(q0 + kTile - 1, p.S - 1)] : 0;
-    for (int j = 0; j < n_kv; ++j) {
-      const int st = kNB == 2 ? (j & 1) : 0;
-      const int kv0 = (j_begin + j) * kTile;
-      const bool full_tile = q_tile_full(p.S, Pb, ds_tile, q0, kv0);
-      LX_TR(tr_cta, j, 4);
-      mbar_wait(&s_full[st], (kNB == 2 ? (j >> 1) : j) & 1);
-      tc_fence_after();
-      LX_TR(tr_cta, j, 5);
-      const uint32_t tS = tmem_S + st * 128 + lane_off;
-      // single pass over TMEM: the whole score row (128 fp32) lives in registers
-      uint32_t sv[4][32];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) tmem_ld_32x32(tS + c * 32, sv[c]);
-      tmem_wait_ld_regs(sv[0]);
-      tmem_wait_ld_regs(sv[1]);
-      tmem_wait_ld_regs(sv[2]);
-      tmem_wait_ld_regs(sv[3]);
-      LX_TR(tr_cta, j, 6);
-      // S is in registers: release the TMEM buffer for the next QK^T right away
-      tc_fence_before();
-      __syncwarp();
-      if (lane_id() == 0) mbar_arrive(&s_empty[st]);
-      if (!full_tile) {
-        // the visible keys of a row are ONE interval of the tile's columns, [lo, lo + width): the prefix-LM mask keeps
-        // kv < max(P, q + 1) (and kv < S), packed documents additionally cut the head (kv >= ds_row) — one unsigned
-        // compare against a per-row constant and a select per element instead of three compares
-        const int lo = kDocs ? ds_row - kv0 : 0;
-        const uint32_t width = (uint32_t)max(min(p.S, max(Pb, q + 1)) - kv0 - lo, 0);
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-#pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if ((uint32_t)(c * 32 + i - lo) >= width) sv[c][i] = 0xff800000u;  // -inf
-      }
-      // four independent max chains (one per 32-column chunk): a single chain of 64 dependent FMNMX3 is ~300 cycles of
-      // pure latency for the one softmax warp a scheduler has
-      float mx4[4];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        mx4[c] = __uint_as_float(sv[c][0]);
-#pragma unroll
-        for (int i = 1; i < 32; ++i) mx4[c] = fmaxf(mx4[c], __uint_as_float(sv[c][i]));
-      }
-      const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      const float m_tile = mx * p.scale_log2;
-      float alpha = 1.f;
-      if (m_tile > m_used + 8.f) {  // lazy rescale: only when the running max grows by more than 2^8
-        alpha = ex2(m_used - m_tile);
-        m_used = m_tile;
-      }
-      uint32_t preg[64];
-      float rowsum = 0.f;
-      // a row may see nothing in a visited tile (packed documents): keep the exponent finite so that exp2(-inf) = 0
-      const float m_exp = (m_used == -INFINITY) ? 0.f : m_used;
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-#pragma unroll
-        for (int i = 0; i < 32; i += 2) {
-          const float p0 = ex2(fmaf(__uint_as_float(sv[c][i]), p.scale_log2, -m_exp));      // -inf -> 0
-          const float p1 = ex2(fmaf(__uint_as_float(sv[c][i + 1]), p.scale_log2, -m_exp));
-          rowsum += p0 + p1;
-          preg[c * 16 + i / 2] = pack_bf16(p0, p1);
-        }
-
-      l = l * alpha + rowsum;
-      LX_TR(tr_cta, j, 7);
-
-      if (j > 0) {
-        mbar_wait(pv_done, (j - 1) & 1);  // O stable, P buffer free
-        tc_fence_after();
-        LX_TR(tr_cta, j, 8);
-        if (__any_sync(0xffffffffu, alpha != 1.f)) {
-#pragma unroll 1
-          for (int c = 0; c < 4; ++c) {
-            uint32_t v[32];
-            tmem_ld_32x32(tmem_O + lane_off + c * 32, v);
-            tmem_wait_ld();
-#pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(__uint_as_float(v[i]) * alpha);
-            tmem_st_32x32(tmem_O + lane_off + c * 32, v);
-          }
-          tmem_wait_st();
-        }
-      }
-      {
-        // P (bf16 pairs) -> TMEM, over the first 64 columns of the score buffer this row was just read from
-        uint32_t(&p0)[32] = *reinterpret_cast<uint32_t(*)[32]>(&preg[0]);
-        uint32_t(&p1)[32] = *reinterpret_cast<uint32_t(*)[32]>(&preg[32]);
-        tmem_st_32x32(tS, p0);
-        tmem_st_32x32(tS + 32, p1);
-        tmem_wait_st();
-      }
-      LX_TR(tr_cta, j, 9);
-      tc_fence_before();
-      __syncwarp();
-      if (lane_id() == 0) mbar_arrive(p_full);
-    }
-    // epilogue
-    mbar_wait(pv_done, (n_kv - 1) & 1);
-    tc_fence_after();
-    const float inv_l = 1.f / l;
-    const bool row_ok = q < p.S;
-    __nv_bfloat16* orow = p.o + ((int64_t)b * p.S + q) * p.ldo + (int64_t)h * kD;
-#pragma unroll 1
-    for (int c = 0; c < kD / 32; ++c) {
-      uint32_t v[32];
-      tmem_ld_32x32(tmem_O + lane_off + c * 32, v);
-      tmem_wait_ld();
-      if (row_ok) {
-#pragma unroll
-        for (int i = 0; i < 32; i += 8) {
-          uint4 o4;
-          o4.x = pack_bf16(__uint_as_float(v[i]) * inv_l, __uint_as_float(v[i + 1]) * inv_l);
-          o4.y = pack_bf16(__uint_as_float(v[i + 2]) * inv_l, __uint_as_float(v[i + 3]) * inv_l);
-          o4.z = pack_bf16(__uint_as_float(v[i + 4]) * inv_l, __uint_as_float(v[i + 5]) * inv_l);
-          o4.w = pack_bf16(__uint_as_float(v[i + 6]) * inv_l, __uint_as_float(v[i + 7]) * inv_l);
-          stg_v4(orow + c * 32 + i, o4);
-        }
-      }
-    }
-    if (row_ok) p.lse[((int64_t)b * p.Hq + h) * p.S + q] = (m_used + log2f(l)) * kLn2;
-    tc_fence_before();
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) tmem_dealloc<1>(tmem_base, 256 * kNB);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Forward, two query tiles per CTA ("ping-pong"). tools/attn_trace.py on the one-tile kernel above: the softmax
-// warpgroup needs ~2400 cycles per 128x128 tile (128 ex2 per thread on the 16-lane XU pipe = 1024, the max, TMEM
-// round-trips, barriers — one warp per scheduler, nothing to overlap with) against 1364 cycles of MMA work, and the
-// chain softmax(j) -> PV(j) is serial. Here a CTA owns TWO 128-row query tiles with one softmax warpgroup each: while
-// one group is in its exp phase the other waits for its MMAs, so XU pipe and tensor pipe are both kept busy and each
-// K/V tile is loaded once for 256 query rows.
-//   TMEM (512 columns): S0 | S1 (P written over the score columns read, A operand of PV from TMEM) | O0 | O1
-//   MMA issue order   : S0(j0), S1(j0);  then per kv tile j:  PV0(j), S0(j+1) | PV1(j), S1(j+1)
-// ------------------------------------------------------------------------------------------------
-namespace fwd2 {
-constexpr int kTile = 128;
-constexpr int kTileBytes = kTile * kHD * 2;        // 32 KB
+constexpr int kTileBytes = kTile * kHD * 2;        // 32 KB: two 16 KB boxes of [128 rows x 128 B]
 constexpr int kOffQ = 0;                           // 2 query tiles
 constexpr int kOffK = kOffQ + 2 * kTileBytes;      // 2 stages
 constexpr int kOffV = kOffK + 2 * kTileBytes;      // 2 stages
-constexpr int kOffBar = kOffV + 2 * kTileBytes;
-// q_full, k full/empty[2], v full/empty[2], s_full[2 tiles], p_full[2 tiles], pv_done[2 tiles]
-constexpr int kNumBars = 1 + 4 + 4 + 2 + 2 + 2;
-constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 16 + 1024;
-constexpr int kThreads = 384;                      // warpgroup 0: TMA / MMA / TMEM alloc; warpgroups 1, 2: softmax of tile 0, 1
-constexpr int kRegsCtrl = 56, kRegsSoftmax = 224;  // 56 + 2 * 224 = 504 <= 512
-}  // namespace fwd2
+constexpr int kOffBar = kOffV + 2 * kTileBytes;    // mbarriers, then the TMEM address slot
+// attn_fwd2_kernel: q_full, k full/empty[2], v full/empty[2], s_full[2 tiles], p_full[2 tiles], pv_done[2 tiles]
+constexpr int kNumBars2 = 1 + 4 + 4 + 2 + 2 + 2;
+// attn_fwd5_kernel: q_full, k full/empty[2], v full/empty[2], s_full[2 tiles], p_chunk[2 tiles][4], pv_done[2 tiles],
+// xu_tok[2 item parities][2 tiles], q_empty
+constexpr int kNumBars5 = 1 + 4 + 4 + 2 + 8 + 2 + 4 + 1;
+constexpr int kSmemBytes2 = kOffBar + kNumBars2 * 8 + 16 + 1024;   // + 1 KB alignment slack
+constexpr int kSmemBytes5 = kOffBar + kNumBars5 * 8 + 16 + 1024;
+constexpr int kThreads = 384;                      // warpgroup 0: control; warpgroups 1, 2: softmax of tile 0, 1
+constexpr int kRegsCtrl = 56, kRegsSoftmax = 224;  // 128 * 56 + 256 * 224 = 384 * 168
+}  // namespace fwd
 
-template <bool kDocs, int kD>
-__global__ void __launch_bounds__(fwd2::kThreads, 1)
+// ------------------------------------------------------------------------------------------------
+// Packed-document forward: two query tiles per CTA ("ping-pong"), one MMA-issuing thread. Traced with one query tile per
+// CTA (round 1, tools/attn_trace.py), the softmax warpgroup needs ~2400 cycles per 128x128 tile (128 ex2 per thread on
+// the 16-lane XU pipe = 1024, the max, TMEM round-trips, barriers — one warp per scheduler, nothing to overlap with)
+// against 1364 cycles of MMA work, and the chain softmax(j) -> PV(j) is serial. Here a CTA owns TWO 128-row query tiles
+// with one softmax warpgroup each: while one group is in its exp phase the other waits for its MMAs, so XU pipe and
+// tensor pipe are both kept busy and each K/V tile is loaded once for 256 query rows. Each tile starts at the kv tile of
+// its first row's document, so the two tiles may start at different kv tiles, which attn_fwd5_kernel cannot handle.
+//   TMEM (512 columns): S0 | S1 (P written over the score columns read, A operand of PV from TMEM) | O0 | O1
+//   MMA issue order   : S0(j0), S1(j0);  then per kv tile j:  PV0(j), S0(j+1) | PV1(j), S1(j+1)
+// ------------------------------------------------------------------------------------------------
+template <int kD>
+__global__ void __launch_bounds__(fwd::kThreads, 1)
 attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                  const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p) {
-  using namespace fwd2;
+  using namespace fwd;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
@@ -427,12 +125,9 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
   uint64_t* s_full = bars + 9;     // [tile]
   uint64_t* p_full = bars + 11;    // [tile]
   uint64_t* pv_done = bars + 13;   // [tile]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars2);
 
   const int warp = threadIdx.x >> 5;
-#ifdef LX_ATTN_TRACE
-  const bool tr_cta = (blockIdx.x | blockIdx.y | blockIdx.z) == 0 && (threadIdx.x & 31) == 0 && (warp == 1 || warp == 4);
-#endif
   // grid = (query heads, batch, pairs of query tiles): pairs run backwards so CTAs are dispatched longest-first
   const int pr = gridDim.z - 1 - blockIdx.z;
   const int h = blockIdx.x, b = blockIdx.y;
@@ -446,7 +141,7 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
     if (q0 < p.S) {
       const int kv_end = min(p.S, max(Pb, q0 + kTile));
       je_[x] = (kv_end + kTile - 1) / kTile;
-      jb_[x] = kDocs ? p.doc_start[(int64_t)b * p.S + q0] / kTile : 0;
+      jb_[x] = p.doc_start[(int64_t)b * p.S + q0] / kTile;
     } else {
       jb_[x] = je_[x] = 0;
     }
@@ -544,11 +239,9 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
           for (int x = 0; x < 2; ++x) {
             if (!active(x, j)) continue;
             if (j == jb_[x] && j != jb) issue_s(x, j);   // a tile whose document starts later than its partner's
-            if (x == 0) LX_TR(tr_cta, j, 0);
             mbar_wait(&v_full[st], ((j - jb) >> 1) & 1);
             mbar_wait(&p_full[x], it[x] & 1);
             tc_fence_after();
-            if (x == 0) LX_TR(tr_cta, j, 1);
             const uint32_t loV = loV0 + st * (kTileBytes / 16);
 #pragma unroll
             for (int kb = 0; kb < 2; ++kb)
@@ -579,16 +272,14 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
     const uint32_t tS = tmem_base + x * 128 + lane_off;
     const uint32_t tO = tmem_base + 256 + x * 128 + lane_off;
     float m_used = -INFINITY, l = 0.f;
-    const int ds_row = kDocs ? p.doc_start[(int64_t)b * p.S + min(q, p.S - 1)] : 0;
-    const int ds_tile = kDocs ? p.doc_start[(int64_t)b * p.S + min(q0 + kTile - 1, p.S - 1)] : 0;
+    const int ds_row = p.doc_start[(int64_t)b * p.S + min(q, p.S - 1)];
+    const int ds_tile = p.doc_start[(int64_t)b * p.S + min(q0 + kTile - 1, p.S - 1)];
     for (int i = 0; i < n_kv; ++i) {
       const int kv0 = (jb_x + i) * kTile;
       // tile needs the element test unless every (q, kv) pair is visible and in range
       const bool full_tile = (kv0 + kTile <= p.S) && ((kv0 + kTile <= Pb) || (kv0 + kTile - 1 <= q0)) && (kv0 >= ds_tile);
-      if (x == 0) LX_TR(tr_cta, jb_x + i, 4);
       mbar_wait(&s_full[x], i & 1);
       tc_fence_after();
-      if (x == 0) LX_TR(tr_cta, jb_x + i, 5);
       // single pass over TMEM: the whole score row (128 fp32) lives in registers
       uint32_t sv[4][32];
 #pragma unroll
@@ -597,12 +288,11 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       tmem_wait_ld_regs(sv[1]);
       tmem_wait_ld_regs(sv[2]);
       tmem_wait_ld_regs(sv[3]);
-      if (x == 0) LX_TR(tr_cta, jb_x + i, 6);
       if (!full_tile) {
         // the visible keys of a row are ONE interval of the tile's columns, [lo, lo + width): the prefix-LM mask keeps
         // kv < max(P, q + 1) (and kv < S), packed documents additionally cut the head (kv >= ds_row) — one unsigned
         // compare against a per-row constant and a select per element instead of three compares
-        const int lo = kDocs ? ds_row - kv0 : 0;
+        const int lo = ds_row - kv0;
         const uint32_t width = (uint32_t)max(min(p.S, max(Pb, q + 1)) - kv0 - lo, 0);
 #pragma unroll
         for (int c = 0; c < 4; ++c)
@@ -638,11 +328,9 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
           preg[c * 16 + e / 2] = pack_bf16(p0, p1);
         }
       l = l * alpha + rowsum;
-      if (x == 0) LX_TR(tr_cta, jb_x + i, 7);
       if (i > 0) {
         mbar_wait(&pv_done[x], (i - 1) & 1);  // O stable
         tc_fence_after();
-        if (x == 0) LX_TR(tr_cta, jb_x + i, 8);
         if (__any_sync(0xffffffffu, alpha != 1.f)) {
 #pragma unroll 1
           for (int c = 0; c < 4; ++c) {
@@ -664,7 +352,6 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         tmem_st_32x32(tS + 32, p1);
         tmem_wait_st();
       }
-      if (x == 0) LX_TR(tr_cta, jb_x + i, 9);
       tc_fence_before();
       __syncwarp();
       if (lane_id() == 0) mbar_arrive(&p_full[x]);
@@ -704,683 +391,22 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
 }
 
 // ------------------------------------------------------------------------------------------------
-// Forward v3: two query tiles per CTA as above, but every score row is shared by TWO threads (column halves), i.e. four
-// softmax warpgroups per CTA. Measured (tools/xu_bench.cu, profiles/r2_xu_bench.txt): one warp issues a MUFU.EX2 at most
-// every 8 cycles, while two warps on the same scheduler together reach one per ~5.5 cycles — a thread-per-row softmax is
-// bound by its own 128 dependent-free ex2 (>= 1024 cycles per tile) no matter how idle the XU pipe is, and that softmax
-// sits on the serial chain S(j) -> softmax(j) -> PV(j) -> S(j+1) of its tile (P aliases S in TMEM, so the chain cannot
-// be broken), which is what paces the kernel: 4250 cycles per pair of tiles against 2728 cycles of MMA work.
-// With 64 columns per thread the per-warp ex2 floor halves, four warps per scheduler fill the XU pipe, the O rescale and
-// the epilogue split by head-dim halves, and PV starts on the first 64 kv columns while the second half is still in exp.
-//   row maxima / row sums of the two halves are exchanged through shared memory (double-buffered slots, one 64-thread
-//   named barrier per lane quarter and tile); both halves take identical rescale decisions (same inputs).
-//   TMEM (512 columns): S0 | S1 | O0 | O1; P half h (bf16 pairs, 32 columns) is written over the first 32 columns of
-//   the 64 score columns its own warpgroup has just read.
-// ------------------------------------------------------------------------------------------------
-namespace fwd3 {
-constexpr int kTile = 128;
-constexpr int kTileBytes = kTile * kHD * 2;        // 32 KB
-constexpr int kOffQ = 0;                           // 2 query tiles
-constexpr int kOffK = kOffQ + 2 * kTileBytes;      // 2 stages
-constexpr int kOffV = kOffK + 2 * kTileBytes;      // 2 stages
-constexpr int kOffStat = kOffV + 2 * kTileBytes;   // exchange slots: [2 buffers][2 tiles][2 halves][128 rows] fp32
-constexpr int kStatBytes = 2 * 2 * 2 * kTile * 4;
-constexpr int kOffBar = kOffStat + kStatBytes;
-// q_full, k full/empty[2], v full/empty[2], s_full[2 tiles], p_full[2 tiles][2 halves], pv_done[2 tiles]
-constexpr int kNumBars = 1 + 4 + 4 + 2 + 4 + 2;
-constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 16 + 1024;
-// warps 0-15: four softmax warpgroups (tile 0 halves 0, 1; tile 1 halves 0, 1); warp 16: TMA producer + TMEM allocator;
-// warp 17: MMA issuer. 18 warps get 112 registers each straight from the launch (65536 / 576 = 113): no setmaxnreg —
-// it can only trade registers inside the CTA's launch allocation, and 640 threads would start at 96 registers with
-// nothing to take the 16 extra per softmax thread from but a 32-register control warpgroup (measured: spills around
-// every MMA group of the issuer).
-constexpr int kThreads = 576;
-static_assert(kSmemBytes <= 232448, "attention forward shared memory budget");
-}  // namespace fwd3
-
-template <bool kDocs, int kD>
-__global__ void __launch_bounds__(fwd3::kThreads, 1)
-attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                 const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p) {
-  using namespace fwd3;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  float* s_stat = reinterpret_cast<float*>(smem + kOffStat);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
-  uint64_t* q_full = bars;
-  uint64_t* k_full = bars + 1;
-  uint64_t* k_empty = bars + 3;
-  uint64_t* v_full = bars + 5;
-  uint64_t* v_empty = bars + 7;
-  uint64_t* s_full = bars + 9;     // [tile]
-  uint64_t* p_full = bars + 11;    // [tile * 2 + half]
-  uint64_t* pv_done = bars + 15;   // [tile]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars);
-
-  const int warp = threadIdx.x >> 5;
-  // grid = (query heads, batch, pairs of query tiles): pairs run backwards so CTAs are dispatched longest-first
-  const int pr = gridDim.z - 1 - blockIdx.z;
-  const int h = blockIdx.x, b = blockIdx.y;
-  const int Pb = p.prefix_b ? min(max(p.prefix_b[b], 0), p.S) : p.P;   // prefix length of this sequence
-  const int hk = h / (p.Hq / p.Hkv);
-  // per-tile kv tile ranges [jb_x, je_x); a tile past the end of the sequence has an empty range
-  int jb_[2], je_[2];
-#pragma unroll
-  for (int x = 0; x < 2; ++x) {
-    const int q0 = (2 * pr + x) * kTile;
-    if (q0 < p.S) {
-      const int kv_end = min(p.S, max(Pb, q0 + kTile));
-      je_[x] = (kv_end + kTile - 1) / kTile;
-      jb_[x] = kDocs ? p.doc_start[(int64_t)b * p.S + q0] / kTile : 0;
-    } else {
-      jb_[x] = je_[x] = 0;
-    }
-  }
-  const bool act1 = je_[1] > jb_[1];
-  const int jb = act1 ? min(jb_[0], jb_[1]) : jb_[0];
-  const int je = max(je_[0], je_[1]);
-
-  if (warp == 16 && elect_one()) {
-    tma_prefetch_desc(&tmQ);
-    tma_prefetch_desc(&tmK);
-    tma_prefetch_desc(&tmV);
-  }
-  if (warp == 17 && elect_one()) {
-    mbar_init(q_full, 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&k_full[i], 1);
-      mbar_init(&k_empty[i], 1);
-      mbar_init(&v_full[i], 1);
-      mbar_init(&v_empty[i], 1);
-      mbar_init(&s_full[i], 1);
-      mbar_init(&pv_done[i], 1);
-    }
-    for (int i = 0; i < 4; ++i) mbar_init(&p_full[i], 4);
-    fence_mbar_init();
-  }
-  if (warp == 16) {
-    tmem_alloc<1>(tmem_slot, 512);
-    tmem_relinquish<1>();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp >= 16) {
-    if (warp == 16) {
-      // ------------------------------------ TMA producer ------------------------------------
-      if (elect_one()) {
-        mbar_expect_tx(q_full, 2 * kTileBytes);
-#pragma unroll
-        for (int x = 0; x < 2; ++x) {   // rows past the end of the sequence are zero-filled
-          tma_load_4d(smem + kOffQ + x * kTileBytes, &tmQ, q_full, 0, h, (2 * pr + x) * kTile, b);
-          tma_load_4d(smem + kOffQ + x * kTileBytes + kTileBytes / 2, &tmQ, q_full, 64, h, (2 * pr + x) * kTile, b);
-        }
-        for (int j = jb; j < je; ++j) {
-          const int st = (j - jb) & 1;
-          const uint32_t ph = ((j - jb) >> 1) & 1;
-          mbar_wait(&k_empty[st], ph ^ 1);
-          mbar_expect_tx(&k_full[st], kTileBytes);
-          uint8_t* sk = smem + kOffK + st * kTileBytes;
-          tma_load_4d(sk, &tmK, &k_full[st], 0, hk, j * kTile, b);
-          tma_load_4d(sk + kTileBytes / 2, &tmK, &k_full[st], 64, hk, j * kTile, b);
-          mbar_wait(&v_empty[st], ph ^ 1);
-          mbar_expect_tx(&v_full[st], kTileBytes);
-          uint8_t* sv = smem + kOffV + st * kTileBytes;
-          tma_load_4d(sv, &tmV, &v_full[st], 0, hk, j * kTile, b);
-          tma_load_4d(sv + kTileBytes / 2, &tmV, &v_full[st], 64, hk, j * kTile, b);
-        }
-      }
-      __syncwarp();
-    } else {
-      // ------------------------------------ MMA issuer ------------------------------------
-      if (elect_one()) {
-        constexpr uint32_t idesc_s = make_idesc(1, 1, 128, 128, 0, 0);
-        constexpr uint32_t idesc_pv = make_idesc(1, 1, 128, 128, 0, 1);  // B = V is MN-major
-        constexpr uint32_t kHi = desc_hi(1024);
-        const uint32_t loQ0 = desc_lo(smem_u32(smem + kOffQ), 16);
-        const uint32_t loK0 = desc_lo(smem_u32(smem + kOffK), 16), loV0 = desc_lo(smem_u32(smem + kOffV), 16384);
-        auto active = [&](int x, int j) { return j >= jb_[x] && j < je_[x]; };
-        // S_x(j) = Q_x K(j)^T; releases K(j) if x is the last tile that reads it
-        auto issue_s = [&](int x, int j) {
-          const int st = (j - jb) & 1;
-          mbar_wait(&k_full[st], ((j - jb) >> 1) & 1);
-          tc_fence_after();
-          const uint32_t loQ = loQ0 + x * (kTileBytes / 16), loK = loK0 + st * (kTileBytes / 16);
-#pragma unroll
-          for (int dh = 0; dh < 2; ++dh)
-#pragma unroll
-            for (int ks = 0; ks < 4; ++ks)
-              umma_ss<false, 1>(tmem_base + x * 128, desc_join(loQ + dh * 1024 + ks * 2, kHi),
-                                desc_join(loK + dh * 1024 + ks * 2, kHi), idesc_s, (dh | ks) != 0);
-          umma_commit(&s_full[x]);
-          if (x == 1 || !active(1, j)) umma_commit(&k_empty[st]);
-        };
-        mbar_wait(q_full, 0);
-        int it[2] = {0, 0};   // iterations done per tile
-#pragma unroll
-        for (int x = 0; x < 2; ++x)
-          if (active(x, jb)) issue_s(x, jb);
-        for (int j = jb; j < je; ++j) {
-          const int st = (j - jb) & 1;
-#pragma unroll
-          for (int x = 0; x < 2; ++x) {
-            if (!active(x, j)) continue;
-            if (j == jb_[x] && j != jb) issue_s(x, j);   // a tile whose document starts later than its partner's
-            mbar_wait(&v_full[st], ((j - jb) >> 1) & 1);
-            const uint32_t loV = loV0 + st * (kTileBytes / 16);
-            // O_x += P_x V in two halves of the kv range: half hh of P comes from warpgroup hh of the tile and lives in
-            // the first 32 columns of that warpgroup's 64 score columns
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-              mbar_wait(&p_full[x * 2 + hh], it[x] & 1);
-              tc_fence_after();
-#pragma unroll
-              for (int ks = 0; ks < 4; ++ks)
-                umma_ts_f16(tmem_base + 256 + x * 128, tmem_base + x * 128 + hh * 64 + ks * 8,
-                            desc_join(loV + (hh * 64 + ks * 16) * 8, kHi), idesc_pv, (it[x] | hh | ks) != 0);
-            }
-            umma_commit(&pv_done[x]);
-            if (x == 1 || !active(1, j)) umma_commit(&v_empty[st]);
-            ++it[x];
-            if (active(x, j + 1)) issue_s(x, j + 1);     // in order behind PV_x(j), which reads P from the same columns
-          }
-        }
-      }
-      __syncwarp();
-    }
-  } else {
-    // ------------------------------------ softmax / correction / epilogue: two warpgroups per query tile ------------
-    const int wg = warp >> 2;           // 0..3
-    const int x = wg >> 1;              // query tile
-    const int hf = wg & 1;              // column half (scores: kv columns; O / epilogue: head-dim columns)
-    const int ew = warp & 3;            // TMEM lane quarter (hardware: warp % 4)
-    const int r = ew * 32 + lane_id();  // row in tile == TMEM lane
-    const uint32_t lane_off = uint32_t(ew * 32) << 16;
-    const int q0 = (2 * pr + x) * kTile;
-    const int q = q0 + r;
-    const int jb_x = x ? jb_[1] : jb_[0], je_x = x ? je_[1] : je_[0];
-    const int n_kv = je_x - jb_x;
-    const uint32_t tS = tmem_base + x * 128 + hf * 64 + lane_off;         // my 64 score columns (P over the first 32)
-    const uint32_t tO = tmem_base + 256 + x * 128 + hf * 64 + lane_off;   // my 64 O columns
-    const uint32_t bar_id = 1 + x * 4 + ew;                               // the 64 threads that share my 32 rows
-    float* my_slot = s_stat + (x * 2 + hf) * kTile + r;                   // + buffer * 4 * kTile
-    float* peer_slot = s_stat + (x * 2 + (hf ^ 1)) * kTile + r;
-    float m_used = -INFINITY, l = 0.f;
-    const int ds_row = kDocs ? p.doc_start[(int64_t)b * p.S + min(q, p.S - 1)] : 0;
-    const int ds_tile = kDocs ? p.doc_start[(int64_t)b * p.S + min(q0 + kTile - 1, p.S - 1)] : 0;
-    for (int i = 0; i < n_kv; ++i) {
-      const int kv0 = (jb_x + i) * kTile;
-      // tile needs the element test unless every (q, kv) pair is visible and in range
-      const bool full_tile = (kv0 + kTile <= p.S) && ((kv0 + kTile <= Pb) || (kv0 + kTile - 1 <= q0)) && (kv0 >= ds_tile);
-      mbar_wait(&s_full[x], i & 1);
-      tc_fence_after();
-      uint32_t sv[2][32];
-      tmem_ld_32x32(tS, sv[0]);
-      tmem_ld_32x32(tS + 32, sv[1]);
-      tmem_wait_ld_regs(sv[0]);
-      tmem_wait_ld_regs(sv[1]);
-      if (!full_tile) {
-        // the visible keys of a row are ONE interval of the tile's columns, [lo, lo + width): the prefix-LM mask keeps
-        // kv < max(P, q + 1) (and kv < S), packed documents additionally cut the head (kv >= ds_row) — one unsigned
-        // compare against a per-row constant and a select per element instead of three compares
-        const int lo = kDocs ? ds_row - kv0 : 0;
-        const uint32_t width = (uint32_t)max(min(p.S, max(Pb, q + 1)) - kv0 - lo, 0);
-#pragma unroll
-        for (int c = 0; c < 2; ++c)
-#pragma unroll
-          for (int e = 0; e < 32; ++e)
-            if ((uint32_t)(hf * 64 + c * 32 + e - lo) >= width) sv[c][e] = 0xff800000u;  // -inf
-      }
-      float mx4[4];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        mx4[c] = __uint_as_float(sv[c >> 1][(c & 1) * 16]);
-#pragma unroll
-        for (int e = 1; e < 16; ++e) mx4[c] = fmaxf(mx4[c], __uint_as_float(sv[c >> 1][(c & 1) * 16 + e]));
-      }
-      float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      // row maximum over both column halves (double-buffered slot: the peer reads slot i & 1 after barrier i, my next
-      // write to it is after barrier i + 1)
-      my_slot[(i & 1) * 4 * kTile] = mx;
-      named_bar_sync(bar_id, 64);
-      mx = fmaxf(mx, peer_slot[(i & 1) * 4 * kTile]);
-      const float m_tile = mx * p.scale_log2;
-      float alpha = 1.f;
-      if (m_tile > m_used + 8.f) {  // lazy rescale: only when the running max grows by more than 2^8
-        alpha = ex2(m_used - m_tile);
-        m_used = m_tile;
-      }
-      uint32_t preg[32];
-      float rs0 = 0.f, rs1 = 0.f;
-      // a row may see nothing in a visited tile (packed documents): keep the exponent finite so that exp2(-inf) = 0
-      const float m_exp = (m_used == -INFINITY) ? 0.f : m_used;
-#pragma unroll
-      for (int c = 0; c < 2; ++c)
-#pragma unroll
-        for (int e = 0; e < 32; e += 2) {
-          const float p0 = ex2(fmaf(__uint_as_float(sv[c][e]), p.scale_log2, -m_exp));      // -inf -> 0
-          const float p1 = ex2(fmaf(__uint_as_float(sv[c][e + 1]), p.scale_log2, -m_exp));
-          rs0 += p0;
-          rs1 += p1;
-          preg[c * 16 + e / 2] = pack_bf16(p0, p1);
-        }
-      l = l * alpha + (rs0 + rs1);
-      if (i > 0) {
-        mbar_wait(&pv_done[x], (i - 1) & 1);  // O stable
-        tc_fence_after();
-        if (__any_sync(0xffffffffu, alpha != 1.f)) {   // the peer warp sees the same maxima: same decision
-#pragma unroll 1
-          for (int c = 0; c < 2; ++c) {
-            uint32_t v[32];
-            tmem_ld_32x32(tO + c * 32, v);
-            tmem_wait_ld();
-#pragma unroll
-            for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * alpha);
-            tmem_st_32x32(tO + c * 32, v);
-          }
-          tmem_wait_st();
-        }
-      }
-      tmem_st_32x32(tS, preg);   // P half (bf16 pairs) over the first 32 of my 64 score columns
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane_id() == 0) mbar_arrive(&p_full[x * 2 + hf]);
-    }
-    // epilogue: row sum over both halves, then my 64 head-dim columns of O
-    if (n_kv > 0) {
-      float* eslot = s_stat + (n_kv & 1) * 4 * kTile;   // the buffer the last iteration did NOT use
-      eslot[(x * 2 + hf) * kTile + r] = l;
-      named_bar_sync(bar_id, 64);
-      l += eslot[(x * 2 + (hf ^ 1)) * kTile + r];
-      mbar_wait(&pv_done[x], (n_kv - 1) & 1);
-      tc_fence_after();
-      const float inv_l = 1.f / l;
-      const bool row_ok = q < p.S;
-      __nv_bfloat16* orow = p.o + ((int64_t)b * p.S + q) * p.ldo + (int64_t)h * kD + hf * 64;
-      if (hf * 64 < kD) {
-#pragma unroll 1
-        for (int c = 0; c < 2; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32(tO + c * 32, v);
-          tmem_wait_ld();
-          if (row_ok) {
-#pragma unroll
-            for (int e = 0; e < 32; e += 8) {
-              uint4 o4;
-              o4.x = pack_bf16(__uint_as_float(v[e]) * inv_l, __uint_as_float(v[e + 1]) * inv_l);
-              o4.y = pack_bf16(__uint_as_float(v[e + 2]) * inv_l, __uint_as_float(v[e + 3]) * inv_l);
-              o4.z = pack_bf16(__uint_as_float(v[e + 4]) * inv_l, __uint_as_float(v[e + 5]) * inv_l);
-              o4.w = pack_bf16(__uint_as_float(v[e + 6]) * inv_l, __uint_as_float(v[e + 7]) * inv_l);
-              stg_v4(orow + c * 32 + e, o4);
-            }
-          }
-        }
-      }
-      if (row_ok && hf == 0) p.lse[((int64_t)b * p.Hq + h) * p.S + q] = (m_used + log2f(l)) * kLn2;
-    }
-    tc_fence_before();
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 16) tmem_dealloc<1>(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Forward v4: the v2 structure (two query tiles per CTA, one softmax warpgroup per tile, thread = row) with the serial
-// chain of a tile cut where it can be:  S(j) -> softmax(j) -> PV(j) -> S(j+1)  cannot be broken (P aliases S in TMEM, 512
-// columns are S0 | S1 | O0 | O1), and that chain — not a pipe — paces v2: 1364 cycles of the tile's own MMAs + ~2500 of
-// softmax latency + hand-offs = the measured ~4250 cycles per pair of tiles, with the tensor pipe busy 64 % of the time.
+// Persistent forward, used without packed documents. It keeps attn_fwd2_kernel's structure (two query tiles per CTA,
+// one softmax warpgroup per tile, thread = row) and cuts the serial chain of a tile where it can be cut. The chain
+// S(j) -> softmax(j) -> PV(j) -> S(j+1) cannot be broken (P aliases S in TMEM, 512 columns are S0 | S1 | O0 | O1), and
+// it, not a pipe, paces attn_fwd2_kernel: 1364 cycles of the tile's own MMAs + ~2500 of softmax latency + hand-offs =
+// the measured ~4250 cycles per pair of tiles, with the tensor pipe busy 64 % of the time.
 //   * P is handed over in FOUR 32-column chunks, each with its own mbarrier: the two PV MMAs of a chunk run while the
 //     softmax warpgroup is in the exponentials of the next chunks, so of PV only the last chunk's MMAs stay on the chain;
 //   * one MMA-issuing warp PER TILE: with chunked hand-offs a single issuer thread would sit in tile 0's chunk waits
 //     while tile 1's chunks are ready (head-of-line blocking); the K / V stages are released by BOTH issuers (count 2);
-//   * the per-step wait on pv_done is gone: S(j) is issued behind PV(j-1) by the same thread, so s_full(j) implies it.
-// ------------------------------------------------------------------------------------------------
-namespace fwd4 {
-constexpr int kTile = 128;
-constexpr int kTileBytes = kTile * kHD * 2;        // 32 KB
-constexpr int kOffQ = 0;                           // 2 query tiles
-constexpr int kOffK = kOffQ + 2 * kTileBytes;      // 2 stages
-constexpr int kOffV = kOffK + 2 * kTileBytes;      // 2 stages
-constexpr int kOffBar = kOffV + 2 * kTileBytes;
-// q_full, k full/empty[2], v full/empty[2], s_full[2 tiles], p_chunk[2 tiles][4], pv_done[2 tiles], xu_tok[2 tiles]
-constexpr int kNumBars = 1 + 4 + 4 + 2 + 8 + 2 + 2;
-constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 16 + 1024;
-constexpr int kThreads = 384;                      // warp 0 TMA, warps 1-2 MMA issue (tile 0, 1), warp 3 TMEM alloc; warpgroups 1, 2: softmax
-constexpr int kRegsCtrl = 56, kRegsSoftmax = 224;  // 128 * 56 + 256 * 224 = 384 * 168
-}  // namespace fwd4
-
-template <bool kDocs, int kD, bool kAluPack, bool kStagger>
-__global__ void __launch_bounds__(fwd4::kThreads, 1)
-attn_fwd4_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                 const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p) {
-  using namespace fwd4;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
-  uint64_t* q_full = bars;
-  uint64_t* k_full = bars + 1;
-  uint64_t* k_empty = bars + 3;
-  uint64_t* v_full = bars + 5;
-  uint64_t* v_empty = bars + 7;
-  uint64_t* s_full = bars + 9;     // [tile]
-  uint64_t* p_chunk = bars + 11;   // [tile * 4 + chunk]
-  uint64_t* pv_done = bars + 19;   // [tile]
-  uint64_t* xu_tok = bars + 21;    // [tile]: "tile x may run its next exp phase" (arrived on by the OTHER tile's 4 warps)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars);
-
-  const int warp = threadIdx.x >> 5;
-#ifdef LX_ATTN_TRACE
-  const bool tr_cta = (blockIdx.x | blockIdx.y | blockIdx.z) == 0 && (threadIdx.x & 31) == 0 &&
-                      (warp == 1 || warp == 2 || warp == 4 || warp == 8);
-#endif
-  // grid = (query heads, batch, pairs of query tiles): pairs run backwards so CTAs are dispatched longest-first
-  const int pr = gridDim.z - 1 - blockIdx.z;
-  const int h = blockIdx.x, b = blockIdx.y;
-  const int Pb = p.prefix_b ? min(max(p.prefix_b[b], 0), p.S) : p.P;   // prefix length of this sequence
-  const int hk = h / (p.Hq / p.Hkv);
-  // per-tile kv tile ranges [jb_x, je_x); a tile past the end of the sequence has an empty range
-  int jb_[2], je_[2];
-#pragma unroll
-  for (int x = 0; x < 2; ++x) {
-    const int q0 = (2 * pr + x) * kTile;
-    if (q0 < p.S) {
-      const int kv_end = min(p.S, max(Pb, q0 + kTile));
-      je_[x] = (kv_end + kTile - 1) / kTile;
-      jb_[x] = kDocs ? p.doc_start[(int64_t)b * p.S + q0] / kTile : 0;
-    } else {
-      jb_[x] = je_[x] = 0;
-    }
-  }
-  const bool act1 = je_[1] > jb_[1];
-  const int jb = act1 ? min(jb_[0], jb_[1]) : jb_[0];
-  const int je = max(je_[0], je_[1]);
-
-  if (warp == 0 && elect_one()) {
-    tma_prefetch_desc(&tmQ);
-    tma_prefetch_desc(&tmK);
-    tma_prefetch_desc(&tmV);
-  }
-  if (warp == 1 && elect_one()) {
-    mbar_init(q_full, 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&k_full[i], 1);
-      mbar_init(&k_empty[i], 2);   // one commit from each tile's issuer
-      mbar_init(&v_full[i], 1);
-      mbar_init(&v_empty[i], 2);
-      mbar_init(&s_full[i], 1);
-      mbar_init(&pv_done[i], 1);
-    }
-    for (int i = 0; i < 8; ++i) mbar_init(&p_chunk[i], 4);
-    for (int i = 0; i < 2; ++i) mbar_init(&xu_tok[i], 4);
-    fence_mbar_init();
-  }
-  if (warp == 3) {
-    tmem_alloc<1>(tmem_slot, 512);
-    tmem_relinquish<1>();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp < 4) {
-    setmaxnreg_dec<kRegsCtrl>();
-    if (warp == 0) {
-      // ------------------------------------ TMA producer ------------------------------------
-      if (elect_one()) {
-        mbar_expect_tx(q_full, 2 * kTileBytes);
-#pragma unroll
-        for (int x = 0; x < 2; ++x) {   // rows past the end of the sequence are zero-filled
-          tma_load_4d(smem + kOffQ + x * kTileBytes, &tmQ, q_full, 0, h, (2 * pr + x) * kTile, b);
-          tma_load_4d(smem + kOffQ + x * kTileBytes + kTileBytes / 2, &tmQ, q_full, 64, h, (2 * pr + x) * kTile, b);
-        }
-        for (int j = jb; j < je; ++j) {
-          const int st = (j - jb) & 1;
-          const uint32_t ph = ((j - jb) >> 1) & 1;
-          mbar_wait(&k_empty[st], ph ^ 1);
-          mbar_expect_tx(&k_full[st], kTileBytes);
-          uint8_t* sk = smem + kOffK + st * kTileBytes;
-          tma_load_4d(sk, &tmK, &k_full[st], 0, hk, j * kTile, b);
-          tma_load_4d(sk + kTileBytes / 2, &tmK, &k_full[st], 64, hk, j * kTile, b);
-          mbar_wait(&v_empty[st], ph ^ 1);
-          mbar_expect_tx(&v_full[st], kTileBytes);
-          uint8_t* sv = smem + kOffV + st * kTileBytes;
-          tma_load_4d(sv, &tmV, &v_full[st], 0, hk, j * kTile, b);
-          tma_load_4d(sv + kTileBytes / 2, &tmV, &v_full[st], 64, hk, j * kTile, b);
-        }
-      }
-      __syncwarp();
-    } else if (warp <= 2) {
-      // ------------------------------------ MMA issuer of tile x ------------------------------------
-      // Walks EVERY kv tile of the CTA's range, also those its own query tile does not visit (causal: the first tile of a
-      // pair skips the last kv tile; packed documents: later start): there it only waits for the stage and releases it,
-      // so the K / V barriers always see two arrivals and neither issuer can run a stage ahead of the other.
-      const int x = warp - 1;
-      if (elect_one()) {
-        constexpr uint32_t idesc_s = make_idesc(1, 1, 128, 128, 0, 0);
-        constexpr uint32_t idesc_pv = make_idesc(1, 1, 128, 128, 0, 1);  // B = V is MN-major
-        constexpr uint32_t kHi = desc_hi(1024);
-        const uint32_t loQ = desc_lo(smem_u32(smem + kOffQ), 16) + x * (kTileBytes / 16);
-        const uint32_t loK0 = desc_lo(smem_u32(smem + kOffK), 16), loV0 = desc_lo(smem_u32(smem + kOffV), 16384);
-        const int jb_x = x ? jb_[1] : jb_[0], je_x = x ? je_[1] : je_[0];
-        const uint32_t tSx = tmem_base + x * 128, tOx = tmem_base + 256 + x * 128;
-        auto issue_s = [&](int j) {
-          const int st = (j - jb) & 1;
-          mbar_wait(&k_full[st], ((j - jb) >> 1) & 1);
-          if (j >= jb_x && j < je_x) {
-            tc_fence_after();
-            const uint32_t loK = loK0 + st * (kTileBytes / 16);
-#pragma unroll
-            for (int dh = 0; dh < 2; ++dh)
-#pragma unroll
-              for (int ks = 0; ks < 4; ++ks)
-                umma_ss<false, 1>(tSx, desc_join(loQ + dh * 1024 + ks * 2, kHi), desc_join(loK + dh * 1024 + ks * 2, kHi),
-                                  idesc_s, (dh | ks) != 0);
-            umma_commit(&s_full[x]);
-          }
-          umma_commit(&k_empty[st]);
-        };
-        mbar_wait(q_full, 0);
-        int it = 0;   // PV steps done
-        issue_s(jb);
-        for (int j = jb; j < je; ++j) {
-          const int st = (j - jb) & 1;
-          mbar_wait(&v_full[st], ((j - jb) >> 1) & 1);
-          if (j >= jb_x && j < je_x) {
-            const uint32_t loV = loV0 + st * (kTileBytes / 16);
-            LX_TR(tr_cta, j, x * 16 + 0);
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-              mbar_wait(&p_chunk[x * 4 + c], it & 1);
-              tc_fence_after();
-              if (c == 0) LX_TR(tr_cta, j, x * 16 + 1);
-#pragma unroll
-              for (int k2 = 0; k2 < 2; ++k2) {
-                const int ks = c * 2 + k2;   // 16 kv rows per MMA: P columns 8 ks .. 8 ks + 7, V rows 16 ks .. 16 ks + 15
-                umma_ts_f16(tOx, tSx + ks * 8, desc_join(loV + ((ks >> 2) * 64 + (ks & 3) * 16) * 8, kHi), idesc_pv,
-                            (it | ks) != 0);
-              }
-            }
-            umma_commit(&pv_done[x]);
-            LX_TR(tr_cta, j, x * 16 + 2);
-            ++it;
-          }
-          umma_commit(&v_empty[st]);
-          if (j + 1 < je) issue_s(j + 1);   // in order behind PV_x(j), which reads P from the same columns
-        }
-      }
-      __syncwarp();
-    }
-  } else {
-    // ------------------------------------ softmax / correction / epilogue: one warpgroup per query tile ------------
-    setmaxnreg_inc<kRegsSoftmax>();
-    const int x = (warp - 4) >> 2;
-    const int ew = warp & 3;
-    const int r = ew * 32 + lane_id();  // row in tile == TMEM lane
-    const uint32_t lane_off = uint32_t(ew * 32) << 16;
-    const int q0 = (2 * pr + x) * kTile;
-    const int q = q0 + r;
-    const int jb_x = x ? jb_[1] : jb_[0], je_x = x ? je_[1] : je_[0];
-    const int n_kv = je_x - jb_x;
-    const uint32_t tS = tmem_base + x * 128 + lane_off;
-    const uint32_t tO = tmem_base + 256 + x * 128 + lane_off;
-    float m_used = -INFINITY, l = 0.f;
-    const int ds_row = kDocs ? p.doc_start[(int64_t)b * p.S + min(q, p.S - 1)] : 0;
-    const int ds_tile = kDocs ? p.doc_start[(int64_t)b * p.S + min(q0 + kTile - 1, p.S - 1)] : 0;
-    for (int i = 0; i < n_kv; ++i) {
-      const int kv0 = (jb_x + i) * kTile;
-      // tile needs the element test unless every (q, kv) pair is visible and in range
-      const bool full_tile = (kv0 + kTile <= p.S) && ((kv0 + kTile <= Pb) || (kv0 + kTile - 1 <= q0)) && (kv0 >= ds_tile);
-      LX_TR(tr_cta, jb_x + i, x * 16 + 4);
-      mbar_wait(&s_full[x], i & 1);   // also: PV(i-1) has completed (same issuing thread, in order): O is stable
-      tc_fence_after();
-      LX_TR(tr_cta, jb_x + i, x * 16 + 5);
-      // single pass over TMEM: the whole score row (128 fp32) lives in registers
-      uint32_t sv[4][32];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) tmem_ld_32x32(tS + c * 32, sv[c]);
-      tmem_wait_ld_regs(sv[0]);
-      tmem_wait_ld_regs(sv[1]);
-      tmem_wait_ld_regs(sv[2]);
-      tmem_wait_ld_regs(sv[3]);
-      LX_TR(tr_cta, jb_x + i, x * 16 + 6);
-      if (!full_tile) {
-        // the visible keys of a row are ONE interval of the tile's columns, [lo, lo + width): the prefix-LM mask keeps
-        // kv < max(P, q + 1) (and kv < S), packed documents additionally cut the head (kv >= ds_row) — one unsigned
-        // compare against a per-row constant and a select per element instead of three compares
-        const int lo = kDocs ? ds_row - kv0 : 0;
-        const uint32_t width = (uint32_t)max(min(p.S, max(Pb, q + 1)) - kv0 - lo, 0);
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-#pragma unroll
-          for (int e = 0; e < 32; ++e)
-            if ((uint32_t)(c * 32 + e - lo) >= width) sv[c][e] = 0xff800000u;  // -inf
-      }
-      float mx4[4];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        mx4[c] = __uint_as_float(sv[c][0]);
-#pragma unroll
-        for (int e = 1; e < 32; ++e) mx4[c] = fmaxf(mx4[c], __uint_as_float(sv[c][e]));
-      }
-      const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      const float m_tile = mx * p.scale_log2;
-      float alpha = 1.f;
-      if (m_tile > m_used + 8.f) {  // lazy rescale: only when the running max grows by more than 2^8
-        alpha = ex2(m_used - m_tile);
-        m_used = m_tile;
-      }
-      if (i > 0 && __any_sync(0xffffffffu, alpha != 1.f)) {
-#pragma unroll 1
-        for (int c = 0; c < 4; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32(tO + c * 32, v);
-          tmem_wait_ld();
-#pragma unroll
-          for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) * alpha);
-          tmem_st_32x32(tO + c * 32, v);
-        }
-        tmem_wait_st();
-      }
-      LX_TR(tr_cta, jb_x + i, x * 16 + 7);
-      // The exponentials of the two tiles share the XU pipe (16 ex2 / clk / SM = 8 cycles per warp instruction per
-      // scheduler). tools/attn_trace.py: left alone, the two tiles drift INTO phase within two steps, whatever their initial
-      // offset — both sit in their exp phase together (~2200 cycles each instead of ~1100 alone) and then both sit in
-      // their XU-idle part together (wait for S, TMEM load, row max: ~1700 cycles): ~3900 cycles per step. A token makes
-      // the exp phases mutually exclusive and strictly alternating, t0(0) t1(0) t0(1) t1(1) ..., so that one tile's
-      // XU-idle part hides under the other's exponentials. Without packed documents both tiles start at kv tile 0 and
-      // tile 1 has at least as many steps as tile 0, so the chain of waits is acyclic; with packed documents a tile may
-      // start several kv tiles after its partner and the token could wait on a K / V stage that waits on the token: off.
-      if (kStagger && !kDocs) {
-        // tile 1's exp i follows tile 0's exp i (if tile 0 has one); tile 0's exp i follows tile 1's exp i - 1 (if any)
-        if (x == 1 ? (i < je_[0] - jb_[0]) : (i > 0 && i - 1 < je_[1] - jb_[1])) mbar_wait(&xu_tok[x], (x == 1 ? i : i - 1) & 1);
-      }
-      float m_exp = (m_used == -INFINITY) ? 0.f : m_used;
-      asm volatile("" : "+f"(m_exp));   // pins the exponentials behind the wait (they are pure: ptxas hoists them otherwise)
-      // (a row may see nothing in a visited tile (packed documents): m_exp keeps the exponent finite, exp2(-inf) = 0)
-      float rowsum = 0.f;   // same summation order as v2 (packed-document masks run on v2): bit-identical outputs
-      // chunk c: exponentials of kv columns 32 c .. 32 c + 31 -> 16 bf16 pairs -> P columns 16 c .. 16 c + 15 (over score
-      // columns this thread holds in registers). The store of chunk c completes under the exponentials of chunk c + 1.
-      uint32_t pc[2][16];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-#pragma unroll
-        for (int e = 0; e < 32; e += 2) {
-#ifdef LX_FAKE_EXP   // what-if build (tools only): no MUFU in the loop, results are meaningless
-          const float p0 = fmaf(__uint_as_float(sv[c][e]), p.scale_log2, -m_exp);
-          const float p1 = fmaf(__uint_as_float(sv[c][e + 1]), p.scale_log2, -m_exp);
-#else
-          const float p0 = ex2(fmaf(__uint_as_float(sv[c][e]), p.scale_log2, -m_exp));      // -inf -> 0
-          const float p1 = ex2(fmaf(__uint_as_float(sv[c][e + 1]), p.scale_log2, -m_exp));
-#endif
-          rowsum += p0 + p1;
-          pc[c & 1][e / 2] = kAluPack ? pack_bf16_alu(p0, p1) : pack_bf16(p0, p1);
-        }
-        if (c > 0) {   // chunk c - 1 is in TMEM: hand it to the issuer
-          tmem_wait_st();
-          tc_fence_before();
-          __syncwarp();
-          if (lane_id() == 0) mbar_arrive(&p_chunk[x * 4 + c - 1]);
-          if (c == 1) LX_TR(tr_cta, jb_x + i, x * 16 + 8);
-        }
-        tmem_st_32x16(tS + c * 16, pc[c & 1]);
-      }
-      if (kStagger && !kDocs) {   // exponentials done: the other tile may start its own
-        __syncwarp();
-        if (lane_id() == 0) mbar_arrive(&xu_tok[x ^ 1]);
-      }
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane_id() == 0) mbar_arrive(&p_chunk[x * 4 + 3]);
-      LX_TR(tr_cta, jb_x + i, x * 16 + 9);
-      l = l * alpha + rowsum;
-    }
-    // epilogue
-    if (n_kv > 0) {
-      mbar_wait(&pv_done[x], (n_kv - 1) & 1);
-      tc_fence_after();
-      const float inv_l = 1.f / l;
-      const bool row_ok = q < p.S;
-      __nv_bfloat16* orow = p.o + ((int64_t)b * p.S + q) * p.ldo + (int64_t)h * kD;
-#pragma unroll 1
-      for (int c = 0; c < kD / 32; ++c) {
-        uint32_t v[32];
-        tmem_ld_32x32(tO + c * 32, v);
-        tmem_wait_ld();
-        if (row_ok) {
-#pragma unroll
-          for (int e = 0; e < 32; e += 8) {
-            uint4 o4;
-            o4.x = pack_bf16(__uint_as_float(v[e]) * inv_l, __uint_as_float(v[e + 1]) * inv_l);
-            o4.y = pack_bf16(__uint_as_float(v[e + 2]) * inv_l, __uint_as_float(v[e + 3]) * inv_l);
-            o4.z = pack_bf16(__uint_as_float(v[e + 4]) * inv_l, __uint_as_float(v[e + 5]) * inv_l);
-            o4.w = pack_bf16(__uint_as_float(v[e + 6]) * inv_l, __uint_as_float(v[e + 7]) * inv_l);
-            stg_v4(orow + c * 32 + e, o4);
-          }
-        }
-      }
-      if (row_ok) p.lse[((int64_t)b * p.Hq + h) * p.S + q] = (m_used + log2f(l)) * kLn2;
-    }
-    tc_fence_before();
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 3) tmem_dealloc<1>(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Forward v5 = v4 made PERSISTENT. One CTA per SM walks a static, length-balanced list of work items (pair of query
-// tiles, head, sequence) and every ring — K / V stages, the S / P / O hand-offs, the XU token — keeps running across
-// items, so that of an item's fixed cost only the O drain stays exposed:
-//   * v4 pays per item (= per CTA): launch, barrier init, TMEM allocation, then Q and the first K from global memory and
-//     the first S MMA before any softmax can start (~2400 cycles, tools/attn_trace.py), and at the end one tile alone in
+//   * no per-step wait on pv_done: S(j) is issued behind PV(j-1) by the same thread, so s_full(j) implies it;
+//   * an XU token makes the exp phases of the two tiles strictly alternate (see the softmax loop).
+// The kernel is PERSISTENT: one CTA per SM walks a static, length-balanced list of work items (pair of query tiles, head,
+// sequence) and every ring — K / V stages, the S / P / O hand-offs, the XU token — keeps running across items, so that
+// of an item's fixed cost only the O drain stays exposed:
+//   * with one CTA per item, every item pays launch, barrier init, TMEM allocation, then Q and the first K from global
+//     memory and the first S MMA before any softmax can start (~2400 cycles, traced), and at the end one tile alone in
 //     its last step, the O drain and the tear-down — ~8-12k cycles on items that average ~9 steps of ~3550 cycles at
 //     S = 2048 causal (13.8 items per SM): a quarter of the kernel;
 //   * here the producer loads the next item's Q as soon as both issuers have committed the item's last S MMA (q_empty),
@@ -1391,20 +417,15 @@ attn_fwd4_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
 // Items are ordered longest first (pairs from the end of the sequence, heads of one kv head adjacent) and dealt to the
 // CTAs in boustrophedon order (round r forwards, round r + 1 backwards), which levels the per-CTA sums of a monotone
 // length list to within one step without a work counter. XU-token arrivals are made conditional so that every arrival
-// has exactly one wait (v4 leaves unmatched arrivals behind at the end of a CTA; here the barrier lives on).
-// Packed-document masks stay on v2 (the token's wait chain is only acyclic when both tiles start at kv tile 0).
+// has exactly one wait: the barriers live on across items, so no arrival may be left unmatched.
+// Packed-document masks run on attn_fwd2_kernel (the token's wait chain is only acyclic when both tiles start at kv
+// tile 0).
 // ------------------------------------------------------------------------------------------------
-namespace fwd5 {
-using namespace fwd4;   // same shared-memory layout, thread roles and register split
-constexpr int kNumBars5 = fwd4::kNumBars + 1 + 2;   // + q_empty, + a second pair of XU-token barriers
-constexpr int kSmemBytes5 = fwd4::kOffBar + kNumBars5 * 8 + 16 + 1024;
-}  // namespace fwd5
-
 template <int kD>
-__global__ void __launch_bounds__(fwd4::kThreads, 1)
+__global__ void __launch_bounds__(fwd::kThreads, 1)
 attn_fwd5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                  const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p, int n_pairs) {
-  using namespace fwd5;
+  using namespace fwd;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
@@ -1656,16 +677,22 @@ attn_fwd5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
           }
           tmem_wait_st();
         }
-        // XU token (see v4): within an item the exp phases alternate t0(0) t1(0) t0(1) t1(1) ...; tile 1's exp i follows
-        // tile 0's exp i (if tile 0 has one), tile 0's exp i follows tile 1's exp i - 1. Every arrival below has exactly
-        // one wait here, so the barrier phases can be counted across items.
+        // XU token. The exponentials of the two tiles share the XU pipe (16 ex2 / clk / SM = 8 cycles per warp instruction
+        // per scheduler). Traced, the two tiles left alone drift INTO phase within two steps, whatever their initial offset:
+        // both sit in their exp phase together (~2200 cycles each instead of ~1100 alone) and then both sit in their
+        // XU-idle part together (wait for S, TMEM load, row max: ~1700 cycles), ~3900 cycles per step. The token makes the
+        // exp phases mutually exclusive and strictly alternating, so that one tile's XU-idle part hides under the other's
+        // exponentials. Within an item the exp phases run t0(0) t1(0) t0(1) t1(1) ...; tile 1's exp i follows tile 0's
+        // exp i (if tile 0 has one), tile 0's exp i follows tile 1's exp i - 1. Both tiles start at kv tile 0 and tile 1
+        // has at least as many steps as tile 0, so the chain of waits is acyclic. Every arrival below has exactly one wait
+        // here, so the barrier phases can be counted across items.
         if (x == 1 ? (i < n0) : (i > 0 && i - 1 < n1)) {
           mbar_wait(&xu_tok[(r & 1) * 2 + x], tokw[r & 1] & 1);
           ++tokw[r & 1];
         }
         float m_exp = (m_used == -INFINITY) ? 0.f : m_used;
         asm volatile("" : "+f"(m_exp));   // pins the exponentials behind the wait (they are pure: ptxas hoists them otherwise)
-        float rowsum = 0.f;
+        float rowsum = 0.f;   // same summation order as attn_fwd2_kernel: bit-identical outputs
         uint32_t pc[2][16];
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
@@ -2202,9 +1229,24 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
   if (warp == 2) tmem_dealloc<1>(tmem_base, 512);
 }
 
+// Tile classification of a 128-row query tile starting at q0 (attn_bwd_dq_kernel): the kv tiles it visits are
+// [j_begin, j_begin + n_kv) — up to max(P, q0 + 128), and, with packed documents, from the start of the first row's
+// document on; a visited tile needs no element test when every (q, kv) pair of it is visible and in range.
+template <bool kDocs>
+__device__ __forceinline__ void q_tile_kv_range(int S, int Pb, const int32_t* doc_start, int b, int q0, int& j_begin,
+                                                int& n_kv) {
+  const int kv_end = min(S, max(Pb, q0 + 128));
+  j_begin = kDocs ? doc_start[(int64_t)b * S + q0] / 128 : 0;
+  n_kv = (kv_end + 127) / 128 - j_begin;
+}
+// ds_tile: document start of the tile's last row (0 without documents)
+__device__ __forceinline__ bool q_tile_full(int S, int Pb, int ds_tile, int q0, int kv0) {
+  return (kv0 + 128 <= S) && ((kv0 + 128 <= Pb) || (kv0 + 127 <= q0)) && (kv0 >= ds_tile);
+}
+
 // ------------------------------------------------------------------------------------------------
 // Deterministic dQ (torch.use_deterministic_algorithms): CTA = (128 query rows, 1 query head), the forward's structure.
-// The CTA walks the visible kv tiles of its rows in ascending order (attn_fwd_kernel's tile range and full-tile test)
+// The CTA walks the visible kv tiles of its rows in ascending order (q_tile_kv_range, q_tile_full)
 // and accumulates dQ in TMEM, so the summation order is fixed by construction: no fp32 atomics, no dq_accum.
 // Per kv tile j (every MMA 128 x 128 x 16):
 //   S = Q K^T, dP = dO V^T          (TMEM, thread = query row)
@@ -2253,7 +1295,7 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + kNumBars);
 
   const int warp = threadIdx.x >> 5;
-  // grid = (query heads, batch, query tiles), longest tiles first (as attn_fwd_kernel)
+  // grid = (query heads, batch, query tiles): the tile index runs backwards, so the longest tiles are dispatched first
   const int qt = gridDim.z - 1 - blockIdx.z;
   const int h = blockIdx.x, b = blockIdx.y;
   const int Pb = p.prefix_b ? min(max(p.prefix_b[b], 0), p.S) : p.P;
@@ -2402,7 +1444,7 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
         tmem_wait_ld_regs(sv[1]);
         tmem_wait_ld_regs(sv[2]);
         tmem_wait_ld_regs(sv[3]);
-        if (!full_tile) {   // the visible keys of a row are one interval of the tile's columns (see attn_fwd_kernel)
+        if (!full_tile) {   // the visible keys of a row are one interval of the tile's columns (see attn_fwd2_kernel)
           const int lo = kDocs ? ds_row - kv0 : 0;
           const uint32_t width = (uint32_t)max(min(p.S, max(Pb, q + 1)) - kv0 - lo, 0);
 #pragma unroll
@@ -2607,61 +1649,6 @@ int llamax_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
   if ((rc = make_head_tmap(&tq, q, ldq, B, S, Hq, D, fwd::kTile))) return rc;
   if ((rc = make_head_tmap(&tk, k, ldk, B, S, Hkv, D, fwd::kTile))) return rc;
   if ((rc = make_head_tmap(&tv, v, ldv, B, S, Hkv, D, fwd::kTile))) return rc;
-  // A/B switch: LLAMAX_ATTN_FWD = 1 (one query tile per CTA), 2 (two tiles, thread per row, one issuer), 3 (two tiles,
-  // two threads per row), 4 (two tiles, thread per row, chunked P hand-off, one issuer per tile), 5 (default: v4 made
-  // persistent, one CTA per SM over a static item list)
-  static const int version = [] {
-    const char* e = getenv("LLAMAX_ATTN_FWD");
-    if (getenv("LLAMAX_ATTN_FWD_ONE_TILE") && getenv("LLAMAX_ATTN_FWD_ONE_TILE")[0] == '1') return 1;
-    return (e != nullptr && e[0] >= '1' && e[0] <= '5') ? e[0] - '0' : 5;
-  }();
-  // packed documents: the XU token of v4 / v5 is off there (see the kernels) and without it they lose to v2 -> v2
-  const int version_eff = (version >= 4 && doc_start != nullptr) ? 2 : version;
-  if (version_eff == 5) {   // persistent: one CTA per SM over a static item list
-    auto kern5 = D == 128 ? attn_fwd5_kernel<128> : attn_fwd5_kernel<64>;
-    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern5), fwd5::kSmemBytes5, "attn_fwd: cudaFuncSetAttribute"))) return rc;
-    AttnFwdParams p5;
-    p5.o = (__nv_bfloat16*)o;
-    p5.ldo = ldo;
-    p5.lse = (float*)lse;
-    p5.B = (int)B; p5.S = (int)S; p5.Hq = Hq; p5.Hkv = Hkv;
-    p5.P = (int)std::min<int64_t>(prefix_len, S);
-    p5.D = D;
-    p5.scale_log2 = scale * kLog2e;
-    p5.doc_start = nullptr;
-    p5.prefix_b = (const int32_t*)prefix_len_b;
-    const int n_pairs = (int)((ceil_div(S, fwd::kTile) + 1) / 2);
-    const int64_t n_items = (int64_t)n_pairs * B * Hq;
-    const int grid5 = (int)std::min<int64_t>(n_items, sm_count());
-    kern5<<<grid5, fwd4::kThreads, fwd5::kSmemBytes5, (cudaStream_t)stream>>>(tq, tk, tv, p5, n_pairs);
-    LX_CHECK_LAUNCH("attn_fwd");
-    return 0;
-  }
-  const bool one_tile = version_eff == 1;
-  auto kern1 = doc_start ? (D == 128 ? attn_fwd_kernel<true, 128> : attn_fwd_kernel<true, 64>)
-                         : (D == 128 ? attn_fwd_kernel<false, 128> : attn_fwd_kernel<false, 64>);
-  auto kern2 = doc_start ? (D == 128 ? attn_fwd2_kernel<true, 128> : attn_fwd2_kernel<true, 64>)
-                         : (D == 128 ? attn_fwd2_kernel<false, 128> : attn_fwd2_kernel<false, 64>);
-  auto kern3 = doc_start ? (D == 128 ? attn_fwd3_kernel<true, 128> : attn_fwd3_kernel<true, 64>)
-                         : (D == 128 ? attn_fwd3_kernel<false, 128> : attn_fwd3_kernel<false, 64>);
-  static const bool alu_pack = getenv("LLAMAX_ATTN_ALU_PACK") && getenv("LLAMAX_ATTN_ALU_PACK")[0] == '1';
-  static const bool stagger = !(getenv("LLAMAX_ATTN_STAGGER") && getenv("LLAMAX_ATTN_STAGGER")[0] == '0');
-  auto pick4 = [&](auto docs_tag, auto d_tag) {
-    constexpr bool kDc = decltype(docs_tag)::value;
-    constexpr int kDd = decltype(d_tag)::value;
-    return alu_pack ? (stagger ? attn_fwd4_kernel<kDc, kDd, true, true> : attn_fwd4_kernel<kDc, kDd, true, false>)
-                    : (stagger ? attn_fwd4_kernel<kDc, kDd, false, true> : attn_fwd4_kernel<kDc, kDd, false, false>);
-  };
-  auto kern4 = doc_start ? (D == 128 ? pick4(std::true_type{}, std::integral_constant<int, 128>{})
-                                     : pick4(std::true_type{}, std::integral_constant<int, 64>{}))
-                         : (D == 128 ? pick4(std::false_type{}, std::integral_constant<int, 128>{})
-                                     : pick4(std::false_type{}, std::integral_constant<int, 64>{}));
-  auto kern = version_eff == 1 ? kern1 : version_eff == 2 ? kern2 : version_eff == 3 ? kern3 : kern4;
-  const int smem_bytes = version_eff == 1 ? fwd::smem_bytes(fwd::kNB) : version_eff == 2 ? fwd2::kSmemBytes
-                         : version_eff == 3 ? fwd3::kSmemBytes : fwd4::kSmemBytes;
-  const int threads = version_eff == 1 ? fwd::kThreads : version_eff == 2 ? fwd2::kThreads
-                      : version_eff == 3 ? fwd3::kThreads : fwd4::kThreads;
-  if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), smem_bytes, "attn_fwd: cudaFuncSetAttribute"))) return rc;
   AttnFwdParams p;
   p.o = (__nv_bfloat16*)o;
   p.ldo = ldo;
@@ -2672,9 +1659,19 @@ int llamax_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
   p.scale_log2 = scale * kLog2e;
   p.doc_start = (const int32_t*)doc_start;
   p.prefix_b = (const int32_t*)prefix_len_b;
-  const unsigned q_tiles = (unsigned)ceil_div(S, fwd::kTile);
-  dim3 grid(Hq, (unsigned)B, one_tile ? q_tiles : (q_tiles + 1) / 2);
-  kern<<<grid, threads, smem_bytes, (cudaStream_t)stream>>>(tq, tk, tv, p);
+  const int n_pairs = (int)((ceil_div(S, fwd::kTile) + 1) / 2);
+  if (doc_start) {   // packed documents: one CTA per pair of query tiles
+    auto kern = D == 128 ? attn_fwd2_kernel<128> : attn_fwd2_kernel<64>;
+    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), fwd::kSmemBytes2, "attn_fwd: cudaFuncSetAttribute"))) return rc;
+    dim3 grid(Hq, (unsigned)B, (unsigned)n_pairs);
+    kern<<<grid, fwd::kThreads, fwd::kSmemBytes2, (cudaStream_t)stream>>>(tq, tk, tv, p);
+  } else {   // persistent: one CTA per SM over a static item list
+    auto kern = D == 128 ? attn_fwd5_kernel<128> : attn_fwd5_kernel<64>;
+    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), fwd::kSmemBytes5, "attn_fwd: cudaFuncSetAttribute"))) return rc;
+    const int64_t n_items = (int64_t)n_pairs * B * Hq;
+    const int grid = (int)std::min<int64_t>(n_items, sm_count());
+    kern<<<grid, fwd::kThreads, fwd::kSmemBytes5, (cudaStream_t)stream>>>(tq, tk, tv, p, n_pairs);
+  }
   LX_CHECK_LAUNCH("attn_fwd");
   return 0;
 }

@@ -62,13 +62,6 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
   __nv_bfloat162 r = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&r);
 }
-// Two finite fp32 -> packed bf16 with round-half-away (differs from nearest-even only on exact ties): two integer adds
-// and a byte permute on the ALU pipe. The cvt-based pack_bf16 (F2FP) issues on the 16-lane/clk XU pipe, which it
-// shares with ex2: in the attention softmax loops that made XU, not the tensor pipe, the limiter
-// (tools/attn_trace.py: 1610 cycles per 128x128 tile = 128 ex2 + 64 F2FP per thread at 8 cycles each).
-__device__ __forceinline__ uint32_t pack_bf16_alu(float lo, float hi) {
-  return __byte_perm(__float_as_uint(lo) + 0x8000u, __float_as_uint(hi) + 0x8000u, 0x7632);
-}
 // fp32 -> nearest-even bf16 -> fp32, in integer arithmetic (ALU pipe). The cvt.rn.bf16.f32 instruction runs on the
 // 16-lane/clk conversion (XU) pipe, which made the fused norm / SwiGLU passes XU-bound instead of HBM-bound.
 __device__ __forceinline__ float round_bf16(float v) {

@@ -1,4 +1,4 @@
-"""Pipeline-phase timeline of ONE attention CTA (debug build with -DLX_ATTN_TRACE; SM-clock timestamps).
+"""Pipeline-phase timeline of ONE attention-backward CTA (debug build with -DLX_ATTN_TRACE; SM-clock timestamps).
 
     python tools/attn_trace.py --build      # here (nvcc cross-compiles): csrc/libllamax_b200_trace.so
     python tools/attn_trace.py              # on the GPU box: prints per-step phase durations (cycles)
@@ -55,25 +55,7 @@ def show(name, slots, first, last):
         print(f"{s:4d} " + " ".join(f"{x:9d}" for x in row) + f"   {per:6d}")
 
 
-for _ in range(2):
-    o, lse = ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P)
-torch.cuda.synchronize()
-trace.zero_()
-o, lse = ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P)
-torch.cuda.synchronize()
-if os.environ.get("LLAMAX_ATTN_FWD", "4") == "4":
-    show("forward v4 (CTA = last pair of q tiles, head 0), tile 0: softmax warp 4, issuer warp 1",
-         [(4, "top"), (5, "s_full"), (6, "S_in_reg"), (7, "max_done"), (8, "chunk0"), (9, "chunk3"), (0, "mma:top"), (1, "mma:c0"), (2, "mma:pv_iss")],
-         0, 16)
-    show("forward v4, tile 1: softmax warp 8, issuer warp 2 (same clock origin as above: subtract)",
-         [(4, "top"), (20, "top1"), (21, "s_full1"), (22, "S_in_reg1"), (23, "max_done1"), (24, "chunk0_1"), (25, "chunk3_1"), (16, "mma1:top"), (17, "mma1:c0"), (18, "mma1:pv_iss")],
-         0, 16)
-else:
-    show("forward (CTA q-tile 15, head 0): mma thread 0/1, softmax warp 4..9",
-         [(4, "top"), (5, "s_full"), (6, "S_in_reg"), (7, "exp_done"), (8, "pv_done"), (9, "P_stored"), (0, "mma:top"), (1, "mma:p_full")],
-         0, 16)
-if "fwd" in sys.argv:
-    sys.exit(0)
+o, lse = ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P)   # operands of the backward
 for _ in range(2):
     ops.attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, P)
 torch.cuda.synchronize()

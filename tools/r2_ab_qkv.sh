@@ -10,4 +10,3 @@ PY
 run qkv1 A=1
 run qkv3 LLAMAX_QKV_ONE_LAUNCH=0
 run qkv1b A=1
-run fwd4 LLAMAX_ATTN_FWD=4
