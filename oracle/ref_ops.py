@@ -203,6 +203,54 @@ def attention_ref_grads(q, k, v, dout, prefix_len, dtype=torch.float64, doc_ids=
     return out.detach(), q_.grad, k_.grad, v_.grad
 
 
+def attention_ref_grouped(q, k, v, dout, prefix_len, doc_ids=None, scale=None, delta_from_bf16_o=False):
+    """The math of `attention_ref_grads` in fp64, written out and evaluated one (sequence, kv head) group at a time on
+    the device of the inputs, so that it scales to full-size shapes on a GPU (fp64 matmuls ignore the TF32 flags).
+
+    q, dout [B,Hq,S,D], k, v [B,Hkv,S,D] (any float dtype); prefix_len: int, or a sequence / tensor of B lengths;
+    doc_ids: int [B, S] packed-document ids or None; scale: softmax scale (default D**-0.5).
+    delta_from_bf16_o: take delta = rowsum(bf16(o) * dout) instead of rowsum(o * dout), i.e. the rounding a kernel that
+    reads its own bf16 output for delta cannot avoid.
+    Returns fp64 (o [B,Hq,S,D], lse [B,Hq,S] (natural log), dq [B,Hq,S,D], dk, dv [B,Hkv,S,D])."""
+    B, Hq, S, D = q.shape
+    Hkv = k.shape[1]
+    G = Hq // Hkv
+    scale = D ** -0.5 if scale is None else float(scale)
+    dev, f64 = q.device, torch.float64
+    prefix = [int(p) for p in prefix_len] if isinstance(prefix_len, (list, tuple, Tensor)) else [int(prefix_len)] * B
+    o = torch.empty(B, Hq, S, D, dtype=f64, device=dev)
+    lse = torch.empty(B, Hq, S, dtype=f64, device=dev)
+    dq = torch.empty(B, Hq, S, D, dtype=f64, device=dev)
+    dk = torch.empty(B, Hkv, S, D, dtype=f64, device=dev)
+    dv = torch.empty(B, Hkv, S, D, dtype=f64, device=dev)
+    idx = torch.arange(S, device=dev)
+    for b in range(B):
+        if doc_ids is None:
+            mask = (idx[None, :] < prefix[b]) | (idx[:, None] >= idx[None, :])
+        else:
+            d = doc_ids[b].to(dev)
+            mask = (d[:, None] == d[None, :]) & (idx[:, None] >= idx[None, :])
+        for hk in range(Hkv):
+            hs = slice(hk * G, (hk + 1) * G)
+            qg, dog = q[b, hs].to(f64), dout[b, hs].to(f64)          # [G, S, D]
+            kg, vg = k[b, hk].to(f64), v[b, hk].to(f64)              # [S, D]
+            s = (qg @ kg.T) * scale
+            s.masked_fill_(~mask, float("-inf"))
+            m = s.amax(-1, keepdim=True)
+            p = torch.exp(s - m)
+            l = p.sum(-1, keepdim=True)
+            p /= l
+            og = p @ vg
+            o[b, hs], lse[b, hs] = og, (m + l.log()).squeeze(-1)
+            ob = og.to(torch.bfloat16).to(f64) if delta_from_bf16_o else og
+            delta = (ob * dog).sum(-1, keepdim=True)
+            ds = p * (dog @ vg.T - delta)                            # dS = P o (dP - delta), then dS * scale below
+            dq[b, hs] = (ds @ kg) * scale
+            dk[b, hk] = torch.einsum("gqk,gqd->kd", ds, qg) * scale
+            dv[b, hk] = torch.einsum("gqk,gqd->kd", p, dog)
+    return o, lse, dq, dk, dv
+
+
 # ------------------------------------------------------------------------------------------------
 # a1/a3/a12  decoder block                                            modelling/llama.py:93-174
 # ------------------------------------------------------------------------------------------------
