@@ -202,6 +202,32 @@ int llamax_attn_bwd_deterministic(const void* q, int64_t ldq, const void* k, int
                                   int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
                                   const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
                                   const void* rope_inverse, void* stream);
+/* Attention dropout (F.scaled_dot_product_attention(dropout_p) semantics): the three calls above with
+ * O = (P o Z / (1 - p)) V, where P is the masked softmax and Z a keep mask per (batch, query head, q, kv); lse stays that
+ * of the undropped softmax, and the backward regenerates the same Z from (seed, offset). 0 <= dropout_p < 1, anything
+ * else (NaN too) is LLAMAX_ERR_ARG. Z is Philox4x32-10 (Random123 / curand) with key = seed and counter
+ * (kv / 16, q, b * Hq + hq, offset / 4): key kv is kept when byte kv % 16 of the four output words (little-endian) is
+ * >= t = round(256 * dropout_p), and kept values are scaled by 256 / (256 - t): the drop rate is t / 256, exactly.
+ * t = 0 runs the calls above unchanged; t = 256 drops everything (zero outputs and gradients). q and kv are positions
+ * in the (packed) sequence. */
+int llamax_attn_fwd_dropout(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, void* o,
+                            int64_t ldo, void* lse, int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D,
+                            int64_t prefix_len, const void* prefix_len_b, const void* doc_start, float scale,
+                            float dropout_p, uint64_t seed, uint64_t offset, void* stream);
+int llamax_attn_bwd_dropout(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                            const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
+                            int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* dq_accum, void* delta,
+                            int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
+                            const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
+                            const void* rope_inverse, float dropout_p, uint64_t seed, uint64_t offset, void* stream);
+int llamax_attn_bwd_deterministic_dropout(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v,
+                                          int64_t ldv, const void* o, int64_t ldo, const void* lse, const void* dout,
+                                          int64_t lddo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv,
+                                          int64_t lddv, void* delta, int64_t B, int64_t S, int32_t Hq, int32_t Hkv,
+                                          int32_t D, int64_t prefix_len, const void* prefix_len_b,
+                                          const void* doc_start, const void* doc_end, float scale,
+                                          const void* rope_inverse, float dropout_p, uint64_t seed, uint64_t offset,
+                                          void* stream);
 
 /* ---- audio stem (modelling/audio.py:26-31,51-60): Conv1d(k3,s1)+GELU, Conv1d(k3,s2)+GELU -------------------------
  * The convolutions run on llamax_bf16_gemm: with channels-last activations padded by one zero row on each side of a

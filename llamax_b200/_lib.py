@@ -7,7 +7,7 @@ loudly with the build command.
 import ctypes
 import os
 import threading
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int64, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int64, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # LLAMAX_B200_LIB: load another build of the same library (tools/attn_trace.py uses an instrumented one)
@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("LLAMAX_B200_LIB") or os.path.join(_HERE, "csrc", "lib
 P = c_void_p
 I64 = c_int64
 I32 = c_int32
+U64 = c_uint64
 
 
 class Epilogue(Structure):
@@ -84,6 +85,12 @@ SIGNATURES = {
                         I64, I64, I32, I32, I32, I64, P, P, P, c_float, P, P],
     "llamax_attn_bwd_deterministic": [P, I64, P, I64, P, I64, P, I64, P, P, I64, P, I64, P, I64, P, I64, P,
                                       I64, I64, I32, I32, I32, I64, P, P, P, c_float, P, P],
+    "llamax_attn_fwd_dropout": [P, I64, P, I64, P, I64, P, I64, P, I64, I64, I32, I32, I32, I64, P, P, c_float,
+                                c_float, U64, U64, P],
+    "llamax_attn_bwd_dropout": [P, I64, P, I64, P, I64, P, I64, P, P, I64, P, I64, P, I64, P, I64, P, P,
+                                I64, I64, I32, I32, I32, I64, P, P, P, c_float, P, c_float, U64, U64, P],
+    "llamax_attn_bwd_deterministic_dropout": [P, I64, P, I64, P, I64, P, I64, P, P, I64, P, I64, P, I64, P, I64, P,
+                                              I64, I64, I32, I32, I32, I64, P, P, P, c_float, P, c_float, U64, U64, P],
     "llamax_lora_wgrad": [P, I64, P, I64, P, I64, I64, I32, c_float, P],
     "llamax_lora_wgrad_deterministic": [P, I64, P, I64, P, P, I64, I64, I32, c_float, P],
     "llamax_lora_bwd_pair": [P, I64, P, I64, P, I64, P, I64, P, I64, P, P, I64, I64, I32, c_float, P],

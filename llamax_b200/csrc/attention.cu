@@ -64,6 +64,53 @@ __device__ __forceinline__ void sts_v4(uint32_t addr, uint32_t a, uint32_t b, ui
   asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 
+// ------------------------------------------------------------------------------------------------
+// Attention dropout (the semantics of F.scaled_dot_product_attention(dropout_p = p)). The keep mask Z of (batch b,
+// query head hq, query q, key kv) comes from Philox4x32-10 (Random123 / curand), key = the 64-bit seed, counter =
+// (kv / 16, q, b * Hq + hq, call): one call decides 16 consecutive keys of one query row, key kv is kept when byte
+// kv % 16 of the four output words (little-endian) is >= t = round(p * 256), and kept values are scaled by
+// 256 / (256 - t), so the expectation is exact and the drop rate is t / 256. The forward, both backward kernels and
+// tests/attention_dropout_ref.py build the same Z, regenerated, never stored. The LSE is that of the undropped softmax.
+// ------------------------------------------------------------------------------------------------
+struct AttnDrop {
+  uint32_t key0, key1;   // seed: low / high word
+  uint32_t call;         // counter word 3 (generator offset / 4)
+  uint32_t t4;           // t in each of the four bytes (t = 256: 0xffffffff, with scale 0)
+  float scale;           // 256 / (256 - t); 0 when t = 256 (everything dropped)
+};
+
+__device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
+                                               uint32_t k1) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r > 0) {
+      k0 += 0x9E3779B9u;
+      k1 += 0xBB67AE85u;
+    }
+    const uint32_t lo0 = 0xD2511F53u * c0, hi0 = __umulhi(0xD2511F53u, c0);
+    const uint32_t lo1 = 0xCD9E8D57u * c2, hi1 = __umulhi(0xCD9E8D57u, c2);
+    c0 = hi1 ^ c1 ^ k0;
+    c1 = lo1;
+    c2 = hi0 ^ c3 ^ k1;
+    c3 = lo0;
+  }
+  return make_uint4(c0, c1, c2, c3);
+}
+
+// keep mask of the 16 keys [16 g, 16 g + 16) of query row q: 0xff in each kept byte, 0x00 in each dropped one
+__device__ __forceinline__ void drop_keep16(const AttnDrop& d, uint32_t g, uint32_t q, uint32_t bh, uint32_t (&z)[4]) {
+  const uint4 r = philox4x32_10(g, q, bh, d.call, d.key0, d.key1);
+  z[0] = __vcmpgeu4(r.x, d.t4);
+  z[1] = __vcmpgeu4(r.y, d.t4);
+  z[2] = __vcmpgeu4(r.z, d.t4);
+  z[3] = __vcmpgeu4(r.w, d.t4);
+}
+
+// bf16-pair mask of bytes b, b + 1 (b even) of a keep word: AND it into a packed pair of P values
+__device__ __forceinline__ uint32_t drop_pair_mask(uint32_t z, int b) { return __byte_perm(z, 0, b ? 0x3322 : 0x1100); }
+// all-ones / all-zeros word from byte b of a keep word: AND it into an fp32 value
+__device__ __forceinline__ uint32_t drop_elem_mask(uint32_t z, int b) { return __byte_perm(z, 0, b * 0x1111); }
+
 // ================================================================================================
 // forward
 // ================================================================================================
@@ -109,10 +156,10 @@ constexpr int kRegsCtrl = 56, kRegsSoftmax = 224;  // 128 * 56 + 256 * 224 = 384
 //   TMEM (512 columns): S0 | S1 (P written over the score columns read, A operand of PV from TMEM) | O0 | O1
 //   MMA issue order   : S0(j0), S1(j0);  then per kv tile j:  PV0(j), S0(j+1) | PV1(j), S1(j+1)
 // ------------------------------------------------------------------------------------------------
-template <int kD>
+template <int kD, bool kDrop = false>
 __global__ void __launch_bounds__(fwd::kThreads, 1)
 attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                 const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p) {
+                 const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p, const AttnDrop drop) {
   using namespace fwd;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -319,14 +366,21 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       // a row may see nothing in a visited tile (packed documents): keep the exponent finite so that exp2(-inf) = 0
       const float m_exp = (m_used == -INFINITY) ? 0.f : m_used;
 #pragma unroll
-      for (int c = 0; c < 4; ++c)
+      for (int c = 0; c < 4; ++c) {
+        uint32_t z[8];   // dropout: keep bytes of the chunk's 32 keys (the sum l stays that of the undropped P)
+        if constexpr (kDrop) {
+          drop_keep16(drop, (kv0 + c * 32) >> 4, q, b * p.Hq + h, *reinterpret_cast<uint32_t(*)[4]>(&z[0]));
+          drop_keep16(drop, (kv0 + c * 32 + 16) >> 4, q, b * p.Hq + h, *reinterpret_cast<uint32_t(*)[4]>(&z[4]));
+        }
 #pragma unroll
         for (int e = 0; e < 32; e += 2) {
           const float p0 = ex2(fmaf(__uint_as_float(sv[c][e]), p.scale_log2, -m_exp));      // -inf -> 0
           const float p1 = ex2(fmaf(__uint_as_float(sv[c][e + 1]), p.scale_log2, -m_exp));
           rowsum += p0 + p1;
           preg[c * 16 + e / 2] = pack_bf16(p0, p1);
+          if constexpr (kDrop) preg[c * 16 + e / 2] &= drop_pair_mask(z[e / 4], e & 2);
         }
+      }
       l = l * alpha + rowsum;
       if (i > 0) {
         mbar_wait(&pv_done[x], (i - 1) & 1);  // O stable
@@ -360,7 +414,7 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
     if (n_kv > 0) {
       mbar_wait(&pv_done[x], (n_kv - 1) & 1);
       tc_fence_after();
-      const float inv_l = 1.f / l;
+      const float inv_l = kDrop ? drop.scale / l : 1.f / l;
       const bool row_ok = q < p.S;
       __nv_bfloat16* orow = p.o + ((int64_t)b * p.S + q) * p.ldo + (int64_t)h * kD;
 #pragma unroll 1
@@ -421,10 +475,10 @@ attn_fwd2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
 // Packed-document masks run on attn_fwd2_kernel (the token's wait chain is only acyclic when both tiles start at kv
 // tile 0).
 // ------------------------------------------------------------------------------------------------
-template <int kD>
+template <int kD, bool kDrop = false>
 __global__ void __launch_bounds__(fwd::kThreads, 1)
 attn_fwd5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                 const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p, int n_pairs) {
+                 const __grid_constant__ CUtensorMap tmV, const AttnFwdParams p, int n_pairs, const AttnDrop drop) {
   using namespace fwd;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -696,12 +750,19 @@ attn_fwd5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         uint32_t pc[2][16];
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
+          uint32_t z[8];   // dropout: keep bytes of the chunk's 32 keys (the sum l stays that of the undropped P)
+          if constexpr (kDrop) {
+            const uint32_t bh = it.b * p.Hq + it.h;
+            drop_keep16(drop, (kv0 + c * 32) >> 4, q, bh, *reinterpret_cast<uint32_t(*)[4]>(&z[0]));
+            drop_keep16(drop, (kv0 + c * 32 + 16) >> 4, q, bh, *reinterpret_cast<uint32_t(*)[4]>(&z[4]));
+          }
 #pragma unroll
           for (int e = 0; e < 32; e += 2) {
             const float p0 = ex2(fmaf(__uint_as_float(sv[c][e]), p.scale_log2, -m_exp));      // -inf -> 0
             const float p1 = ex2(fmaf(__uint_as_float(sv[c][e + 1]), p.scale_log2, -m_exp));
             rowsum += p0 + p1;
             pc[c & 1][e / 2] = pack_bf16(p0, p1);
+            if constexpr (kDrop) pc[c & 1][e / 2] &= drop_pair_mask(z[e / 4], e & 2);
           }
           if (c > 0) {   // chunk c - 1 is in TMEM: hand it to the issuer
             tmem_wait_st();
@@ -726,7 +787,7 @@ attn_fwd5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       if (n_kv > 0) {
         mbar_wait(&pv_done[x], (sc - 1) & 1);   // PV steps == S steps of this tile
         tc_fence_after();
-        const float inv_l = 1.f / l;
+        const float inv_l = kDrop ? drop.scale / l : 1.f / l;
         const bool row_ok = q < p.S;
         __nv_bfloat16* orow = p.o + ((int64_t)it.b * p.S + q) * p.ldo + (int64_t)it.h * kD;
 #pragma unroll 1
@@ -793,7 +854,7 @@ constexpr int kOffV = kOffK + kTileBytes;
 constexpr int kOffQ = kOffV + kTileBytes;         // 2 stages (Q(s) lives from S^T(s) to dK(s), across S^T(s+1))
 constexpr int kOffdO = kOffQ + 2 * kTileBytes;    // 1 stage  (dO(s): dP^T(s) and dV(s) are adjacent in the MMA order)
 constexpr int kOffdS = kOffdO + kTileBytes;       // dS^T [128 kv][128 q] bf16: two boxes (q halves) of [128 x 128 B]
-constexpr int kOffdQ = kOffdS + kTileBytes;       // fp32 [32 q][128 d] staging for the bulk reduce-add
+constexpr int kOffdQ = kOffdS + kTileBytes;       // 16 KB: with dropout, each worker warp's 2 KB keep-byte exchange
 constexpr int kStageRows = 32;
 constexpr int kdQBytes = kStageRows * kHD * 4;    // 16 KB
 constexpr int kOffStat = kOffdQ + kdQBytes;       // lse2 / delta*scale / doc_start: 2 buffers x 3 x 128 words
@@ -820,11 +881,11 @@ constexpr int kColdV = 0, kColdK = 128, kColX = 256, kColY = 384;
 // and dP^T(s+1) waits only for dS^T(s); dV and dK accumulate in the same MMA order, so they are bitwise those of the
 // default instantiation. Without the drain warpgroup the CTA has 384 threads and no setmaxnreg rebalancing (the 168
 // registers a thread gets need no spills).
-template <bool kDocs, int kD, bool kNoDQ = false>
+template <bool kDocs, int kD, bool kNoDQ = false, bool kDrop = false>
 __global__ void __launch_bounds__(kNoDQ ? bwd::kThreadsNoDQ : bwd::kThreads, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                 const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
-                const AttnBwdParams p) {
+                const AttnBwdParams p, const AttnDrop drop) {
   using namespace bwd;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -1058,6 +1119,39 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       const int ds_tile = kDocs ? p.doc_start[(int64_t)b * p.S + min(q0 + kQ - 1, p.S - 1)] : 0;
       const bool full_tile = (kv0 + kKV <= p.S) && (q0 + kQ <= p.S) && ((kv0 + kKV <= Pb) || (kv0 + kKV - 1 <= q0)) &&
                              (kv0 >= ds_tile);
+      // dropout: a thread (kv row x 64 query columns) holds the transpose of the Philox layout (one call = 16 keys of
+      // one query). The 16 lanes that share kv / 16 make the 64 calls of their query columns, 4 each, and swap the keep
+      // bytes through the warp's 2 KB of shared memory (a 128 B line per kv row, 16 B slots XOR-swizzled by the row:
+      // the stores and the v4 loads are free of bank conflicts). zr[w] byte j: query column 4 w + j. Made before the
+      // wait for S^T, under the MMAs.
+      uint32_t zr[16];
+      if constexpr (kDrop) {
+        const int hh = lane_id() >> 4, L = lane_id() & 15;
+        const uint32_t bh = b * p.Hq + hk * G + s / steps_per_head;
+        const uint32_t blk = smem_u32(smem + kOffdQ) + (warp - 4) * 2048;
+        uint32_t zk[4][4];   // [call j: query column 4 L + j][word w: kv rows 4 w .. 4 w + 3 of the 16]
+#pragma unroll
+        for (int j = 0; j < 4; ++j) drop_keep16(drop, kv >> 4, q0 + grp * 64 + 4 * L + j, bh, zk[j]);
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {   // 4 x 4 byte transpose: word bb -> kv row 4 w + bb, byte j = call j
+          const uint32_t a01l = __byte_perm(zk[0][w], zk[1][w], 0x5140), a01h = __byte_perm(zk[0][w], zk[1][w], 0x7362);
+          const uint32_t a23l = __byte_perm(zk[2][w], zk[3][w], 0x5140), a23h = __byte_perm(zk[2][w], zk[3][w], 0x7362);
+          const uint32_t tw[4] = {__byte_perm(a01l, a23l, 0x5410), __byte_perm(a01l, a23l, 0x7632),
+                                  __byte_perm(a01h, a23h, 0x5410), __byte_perm(a01h, a23h, 0x7632)};
+#pragma unroll
+          for (int bb = 0; bb < 4; ++bb) {
+            const int m = 4 * w + bb;
+            asm volatile("st.shared.u32 [%0], %1;" ::"r"(blk + m * 128 + (((hh * 4 + (L >> 2)) ^ (m & 7)) << 4) + (L & 3) * 4),
+                         "r"(tw[bb]) : "memory");
+          }
+        }
+        __syncwarp();
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+          asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
+                       : "=r"(zr[4 * k]), "=r"(zr[4 * k + 1]), "=r"(zr[4 * k + 2]), "=r"(zr[4 * k + 3])
+                       : "r"(blk + L * 128 + (((hh * 4 + k) ^ (L & 7)) << 4)) : "memory");
+      }
       mbar_wait(s_full, s & 1);
       tc_fence_after();
       LX_TR(tr_cta, s, 7);
@@ -1107,8 +1201,16 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         if (full_tile) block(std::false_type{});
         else block(std::true_type{});
       }
-      // P^T -> the first 32 of the 64 X columns this warp has just read (no other warp touches them)
-      tmem_st_32x32(tXw, pr);
+      // P^T -> the first 32 of the 64 X columns this warp has just read (no other warp touches them); with dropout
+      // (P o Z)^T, the A operand of dV (pr itself stays undropped for dS)
+      if constexpr (kDrop) {
+        uint32_t pz[32];
+#pragma unroll
+        for (int k = 0; k < 32; ++k) pz[k] = pr[k] & drop_pair_mask(zr[k / 2], (k & 1) * 2);
+        tmem_st_32x32(tXw, pz);
+      } else {
+        tmem_st_32x32(tXw, pr);
+      }
       tmem_wait_st();
       tc_fence_before();
       __syncwarp();
@@ -1127,10 +1229,16 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         for (int i = 0; i < 32; i += 4) {
           const float4 d4 = lds_f4(stat_u + kQ * 4 + (c * 32 + i) * 4);          // delta * scale
           const uint32_t p01 = pr[c * 16 + i / 2], p23 = pr[c * 16 + i / 2 + 1];
-          const float ds0 = bf16_lo(p01) * fmaf(__uint_as_float(dv[i]), p.scale, -d4.x);
-          const float ds1 = bf16_hi(p01) * fmaf(__uint_as_float(dv[i + 1]), p.scale, -d4.y);
-          const float ds2 = bf16_lo(p23) * fmaf(__uint_as_float(dv[i + 2]), p.scale, -d4.z);
-          const float ds3 = bf16_hi(p23) * fmaf(__uint_as_float(dv[i + 3]), p.scale, -d4.w);
+          if constexpr (kDrop) {   // dS = P o (Z / (1 - p) o dP - delta)
+            const uint32_t zw = zr[c * 8 + i / 4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) dv[i + e] &= drop_elem_mask(zw, e);
+          }
+          const float dsc = kDrop ? p.scale * drop.scale : p.scale;
+          const float ds0 = bf16_lo(p01) * fmaf(__uint_as_float(dv[i]), dsc, -d4.x);
+          const float ds1 = bf16_hi(p01) * fmaf(__uint_as_float(dv[i + 1]), dsc, -d4.y);
+          const float ds2 = bf16_lo(p23) * fmaf(__uint_as_float(dv[i + 2]), dsc, -d4.z);
+          const float ds3 = bf16_hi(p23) * fmaf(__uint_as_float(dv[i + 3]), dsc, -d4.w);
           dsr[i / 2] = pack_bf16(ds0, ds1);
           dsr[i / 2 + 1] = pack_bf16(ds2, ds3);
         }
@@ -1157,6 +1265,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       uint32_t v[32];
       tmem_ld_32x32(tmem_base + (grp == 0 ? kColdV : kColdK) + lane_off + c * 32, v);
       tmem_wait_ld_regs(v);
+      if (kDrop && grp == 0) {   // dV = (P o Z)^T dO / (1 - p)
+#pragma unroll
+        for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(__uint_as_float(v[i]) * drop.scale);
+      }
       if (row_ok && grp == 1 && p.rope != nullptr) {
         // dK through the RoPE backward: (g0, g1) -> (g0 c + g1 s, g1 c - g0 s) per adjacent pair, position = kv row
         const float4* cs = reinterpret_cast<const float4*>(p.rope + ((int64_t)kv * (kD / 2) + c * 16) * 2);
@@ -1273,11 +1385,11 @@ constexpr int kThreads = 256;                      // warp 0 TMA, warp 1 MMA, wa
 constexpr int kColS = 0, kColdP = 256, kColdQ = 384;
 }  // namespace bwdq
 
-template <bool kDocs, int kD>
+template <bool kDocs, int kD, bool kDrop = false>
 __global__ void __launch_bounds__(bwdq::kThreads, 1)
 attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                    const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmdO,
-                   const AttnBwdParams p, __nv_bfloat16* __restrict__ dq, int64_t lddq) {
+                   const AttnBwdParams p, __nv_bfloat16* __restrict__ dq, int64_t lddq, const AttnDrop drop) {
   using namespace bwdq;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -1465,13 +1577,24 @@ attn_bwd_dq_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
         uint32_t dv[32], dsr[16];
-        tmem_ld_32x32(tmem_dP + lane_off + c * 32, dv);
-        tmem_wait_ld_regs(dv);
+        if constexpr (kDrop) {   // dS = P o (Z / (1 - p) o dP - delta): Z of keys kv0 + 32 c .. kv0 + 32 c + 31
+          uint32_t z[8];
+          drop_keep16(drop, (kv0 + c * 32) >> 4, q, b * p.Hq + h, *reinterpret_cast<uint32_t(*)[4]>(&z[0]));
+          drop_keep16(drop, (kv0 + c * 32 + 16) >> 4, q, b * p.Hq + h, *reinterpret_cast<uint32_t(*)[4]>(&z[4]));
+          tmem_ld_32x32(tmem_dP + lane_off + c * 32, dv);
+          tmem_wait_ld_regs(dv);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) dv[i] &= drop_elem_mask(z[i / 4], i & 3);
+        } else {
+          tmem_ld_32x32(tmem_dP + lane_off + c * 32, dv);
+          tmem_wait_ld_regs(dv);
+        }
+        const float dsc = kDrop ? p.scale * drop.scale : p.scale;
 #pragma unroll
         for (int i = 0; i < 32; i += 2) {
           const uint32_t p01 = pr[c * 16 + i / 2];
-          dsr[i / 2] = pack_bf16(bf16_lo(p01) * fmaf(__uint_as_float(dv[i]), p.scale, -dlt),
-                                 bf16_hi(p01) * fmaf(__uint_as_float(dv[i + 1]), p.scale, -dlt));
+          dsr[i / 2] = pack_bf16(bf16_lo(p01) * fmaf(__uint_as_float(dv[i]), dsc, -dlt),
+                                 bf16_hi(p01) * fmaf(__uint_as_float(dv[i + 1]), dsc, -dlt));
         }
         // dS (bf16 pairs) over the score columns of this row: A operand of dQ(j), read straight from TMEM
         tmem_st_32x16(tS + c * 16, dsr);
@@ -1624,6 +1747,19 @@ static int check_attn_args(int64_t B, int64_t S, int Hq, int Hkv, int D, int64_t
   return 0;
 }
 
+// dropout_p -> the kernels' dropout descriptor; *on = false when t = round(256 p) is 0 (the plain kernels run)
+static int make_attn_drop(float dropout_p, uint64_t seed, uint64_t offset, AttnDrop* d, bool* on) {
+  if (!(dropout_p >= 0.f && dropout_p < 1.f)) return set_error(LLAMAX_ERR_ARG, "attention: dropout_p must be in [0, 1)");
+  const int t = (int)lrintf(dropout_p * 256.f);
+  d->key0 = (uint32_t)seed;
+  d->key1 = (uint32_t)(seed >> 32);
+  d->call = (uint32_t)(offset / 4);
+  d->t4 = t >= 256 ? 0xffffffffu : (uint32_t)t * 0x01010101u;
+  d->scale = t >= 256 ? 0.f : 256.f / (float)(256 - t);
+  *on = t > 0;
+  return 0;
+}
+
 }  // namespace lx
 
 using namespace lx;
@@ -1638,9 +1774,33 @@ int llamax_debug_attn_trace(void* buf) {
 }
 #endif
 
-int llamax_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, void* o,
-                    int64_t ldo, void* lse, int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D,
-                    int64_t prefix_len, const void* prefix_len_b, const void* doc_start, float scale, void* stream) {
+}  // extern "C"
+
+template <bool kDrop>
+static int attn_fwd_launch(const CUtensorMap& tq, const CUtensorMap& tk, const CUtensorMap& tv, const AttnFwdParams& p,
+                           int64_t B, int64_t S, int32_t Hq, int32_t D, const AttnDrop& drop, cudaStream_t stream) {
+  int rc;
+  const int n_pairs = (int)((ceil_div(S, fwd::kTile) + 1) / 2);
+  if (p.doc_start) {   // packed documents: one CTA per pair of query tiles
+    auto kern = D == 128 ? attn_fwd2_kernel<128, kDrop> : attn_fwd2_kernel<64, kDrop>;
+    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), fwd::kSmemBytes2, "attn_fwd: cudaFuncSetAttribute"))) return rc;
+    dim3 grid(Hq, (unsigned)B, (unsigned)n_pairs);
+    kern<<<grid, fwd::kThreads, fwd::kSmemBytes2, stream>>>(tq, tk, tv, p, drop);
+  } else {   // persistent: one CTA per SM over a static item list
+    auto kern = D == 128 ? attn_fwd5_kernel<128, kDrop> : attn_fwd5_kernel<64, kDrop>;
+    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), fwd::kSmemBytes5, "attn_fwd: cudaFuncSetAttribute"))) return rc;
+    const int64_t n_items = (int64_t)n_pairs * B * Hq;
+    const int grid = (int)std::min<int64_t>(n_items, sm_count());
+    kern<<<grid, fwd::kThreads, fwd::kSmemBytes5, stream>>>(tq, tk, tv, p, n_pairs, drop);
+  }
+  LX_CHECK_LAUNCH("attn_fwd");
+  return 0;
+}
+
+static int attn_fwd_run(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, void* o,
+                        int64_t ldo, void* lse, int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D,
+                        int64_t prefix_len, const void* prefix_len_b, const void* doc_start, float scale,
+                        const AttnDrop& drop, bool drop_on, void* stream) {
   if (!q || !k || !v || !o || !lse) return set_error(LLAMAX_ERR_ARG, "attn_fwd: null pointer");
   int rc = check_attn_args(B, S, Hq, Hkv, D, prefix_len, "attn_fwd");
   if (rc) return rc;
@@ -1659,24 +1819,46 @@ int llamax_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
   p.scale_log2 = scale * kLog2e;
   p.doc_start = (const int32_t*)doc_start;
   p.prefix_b = (const int32_t*)prefix_len_b;
-  const int n_pairs = (int)((ceil_div(S, fwd::kTile) + 1) / 2);
-  if (doc_start) {   // packed documents: one CTA per pair of query tiles
-    auto kern = D == 128 ? attn_fwd2_kernel<128> : attn_fwd2_kernel<64>;
-    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), fwd::kSmemBytes2, "attn_fwd: cudaFuncSetAttribute"))) return rc;
-    dim3 grid(Hq, (unsigned)B, (unsigned)n_pairs);
-    kern<<<grid, fwd::kThreads, fwd::kSmemBytes2, (cudaStream_t)stream>>>(tq, tk, tv, p);
-  } else {   // persistent: one CTA per SM over a static item list
-    auto kern = D == 128 ? attn_fwd5_kernel<128> : attn_fwd5_kernel<64>;
-    if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), fwd::kSmemBytes5, "attn_fwd: cudaFuncSetAttribute"))) return rc;
-    const int64_t n_items = (int64_t)n_pairs * B * Hq;
-    const int grid = (int)std::min<int64_t>(n_items, sm_count());
-    kern<<<grid, fwd::kThreads, fwd::kSmemBytes5, (cudaStream_t)stream>>>(tq, tk, tv, p, n_pairs);
-  }
-  LX_CHECK_LAUNCH("attn_fwd");
-  return 0;
+  return drop_on ? attn_fwd_launch<true>(tq, tk, tv, p, B, S, Hq, D, drop, (cudaStream_t)stream)
+                 : attn_fwd_launch<false>(tq, tk, tv, p, B, S, Hq, D, drop, (cudaStream_t)stream);
+}
+
+extern "C" {
+
+int llamax_attn_fwd(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, void* o,
+                    int64_t ldo, void* lse, int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D,
+                    int64_t prefix_len, const void* prefix_len_b, const void* doc_start, float scale, void* stream) {
+  return attn_fwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, scale,
+                      AttnDrop{}, false, stream);
+}
+
+int llamax_attn_fwd_dropout(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv, void* o,
+                            int64_t ldo, void* lse, int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D,
+                            int64_t prefix_len, const void* prefix_len_b, const void* doc_start, float scale,
+                            float dropout_p, uint64_t seed, uint64_t offset, void* stream) {
+  AttnDrop drop;
+  bool on;
+  const int rc = make_attn_drop(dropout_p, seed, offset, &drop, &on);
+  if (rc) return rc;
+  return attn_fwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, scale,
+                      drop, on, stream);
 }
 
 }  // extern "C"
+
+template <bool kDrop>
+static auto bwd_kernel_for(bool det, bool docs, int D) {
+  return det ? (docs ? (D == 128 ? attn_bwd_kernel<true, 128, true, kDrop> : attn_bwd_kernel<true, 64, true, kDrop>)
+                     : (D == 128 ? attn_bwd_kernel<false, 128, true, kDrop> : attn_bwd_kernel<false, 64, true, kDrop>))
+             : (docs ? (D == 128 ? attn_bwd_kernel<true, 128, false, kDrop> : attn_bwd_kernel<true, 64, false, kDrop>)
+                     : (D == 128 ? attn_bwd_kernel<false, 128, false, kDrop> : attn_bwd_kernel<false, 64, false, kDrop>));
+}
+
+template <bool kDrop>
+static auto bwd_dq_kernel_for(bool docs, int D) {
+  return docs ? (D == 128 ? attn_bwd_dq_kernel<true, 128, kDrop> : attn_bwd_dq_kernel<true, 64, kDrop>)
+              : (D == 128 ? attn_bwd_dq_kernel<false, 128, kDrop> : attn_bwd_dq_kernel<false, 64, kDrop>);
+}
 
 // dq_accum == NULL: deterministic mode (attn_bwd_dq_kernel writes dq, attn_bwd_kernel<.., kNoDQ> dk / dv)
 static int attn_bwd_run(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
@@ -1684,7 +1866,7 @@ static int attn_bwd_run(const void* q, int64_t ldq, const void* k, int64_t ldk, 
                         int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* dq_accum, void* delta,
                         int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
                         const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
-                        const void* rope_inverse, void* stream) {
+                        const void* rope_inverse, const AttnDrop& drop, bool drop_on, void* stream) {
   const bool det = dq_accum == nullptr;
   if ((doc_start == nullptr) != (doc_end == nullptr))
     return set_error(LLAMAX_ERR_ARG, "attn_bwd: doc_start and doc_end go together");
@@ -1716,10 +1898,7 @@ static int attn_bwd_run(const void* q, int64_t ldq, const void* k, int64_t ldk, 
   if ((rc = make_head_tmap(&tdo, dout, lddo, B, S, Hq, D, bwd::kQ))) return rc;
   if ((rc = make_head_tmap(&tk, k, ldk, B, S, Hkv, D, bwd::kKV))) return rc;
   if ((rc = make_head_tmap(&tv, v, ldv, B, S, Hkv, D, bwd::kKV))) return rc;
-  auto kern = det ? (doc_start ? (D == 128 ? attn_bwd_kernel<true, 128, true> : attn_bwd_kernel<true, 64, true>)
-                               : (D == 128 ? attn_bwd_kernel<false, 128, true> : attn_bwd_kernel<false, 64, true>))
-                  : (doc_start ? (D == 128 ? attn_bwd_kernel<true, 128> : attn_bwd_kernel<true, 64>)
-                               : (D == 128 ? attn_bwd_kernel<false, 128> : attn_bwd_kernel<false, 64>));
+  auto kern = drop_on ? bwd_kernel_for<true>(det, doc_start != nullptr, D) : bwd_kernel_for<false>(det, doc_start != nullptr, D);
   if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), bwd::kSmemBytes, "attn_bwd: cudaFuncSetAttribute"))) return rc;
   AttnBwdParams p;
   p.lse = (const float*)lse;
@@ -1737,15 +1916,14 @@ static int attn_bwd_run(const void* q, int64_t ldq, const void* k, int64_t ldk, 
   p.rope = (const float*)rope_inverse;
   p.prefix_b = (const int32_t*)prefix_len_b;
   dim3 grid(Hkv, (unsigned)ceil_div(S, bwd::kKV), (unsigned)B);
-  kern<<<grid, det ? bwd::kThreadsNoDQ : bwd::kThreads, bwd::kSmemBytes, st>>>(tq, tk, tv, tdo, p);
+  kern<<<grid, det ? bwd::kThreadsNoDQ : bwd::kThreads, bwd::kSmemBytes, st>>>(tq, tk, tv, tdo, p, drop);
   LX_CHECK_LAUNCH("attn_bwd");
   if (det) {
-    auto kdq = doc_start ? (D == 128 ? attn_bwd_dq_kernel<true, 128> : attn_bwd_dq_kernel<true, 64>)
-                         : (D == 128 ? attn_bwd_dq_kernel<false, 128> : attn_bwd_dq_kernel<false, 64>);
+    auto kdq = drop_on ? bwd_dq_kernel_for<true>(doc_start != nullptr, D) : bwd_dq_kernel_for<false>(doc_start != nullptr, D);
     if ((rc = ensure_dyn_smem(reinterpret_cast<const void*>(kdq), bwdq::kSmemBytes, "attn_bwd: cudaFuncSetAttribute")))
       return rc;
     dim3 qgrid(Hq, (unsigned)B, (unsigned)ceil_div(S, bwdq::kTile));
-    kdq<<<qgrid, bwdq::kThreads, bwdq::kSmemBytes, st>>>(tq, tk, tv, tdo, p, (__nv_bfloat16*)dq, lddq);
+    kdq<<<qgrid, bwdq::kThreads, bwdq::kSmemBytes, st>>>(tq, tk, tv, tdo, p, (__nv_bfloat16*)dq, lddq, drop);
     LX_CHECK_LAUNCH("attn_bwd: dq");
     return 0;
   }
@@ -1772,7 +1950,24 @@ int llamax_attn_bwd(const void* q, int64_t ldq, const void* k, int64_t ldk, cons
                     const void* rope_inverse, void* stream) {
   if (!dq_accum) return set_error(LLAMAX_ERR_ARG, "attn_bwd: null pointer");
   return attn_bwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, dout, lddo, dq, lddq, dk, lddk, dv, lddv, dq_accum, delta,
-                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, stream);
+                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, AttnDrop{},
+                      false, stream);
+}
+
+int llamax_attn_bwd_dropout(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                            const void* o, int64_t ldo, const void* lse, const void* dout, int64_t lddo, void* dq,
+                            int64_t lddq, void* dk, int64_t lddk, void* dv, int64_t lddv, void* dq_accum, void* delta,
+                            int64_t B, int64_t S, int32_t Hq, int32_t Hkv, int32_t D, int64_t prefix_len,
+                            const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
+                            const void* rope_inverse, float dropout_p, uint64_t seed, uint64_t offset, void* stream) {
+  AttnDrop drop;
+  bool on;
+  int rc = make_attn_drop(dropout_p, seed, offset, &drop, &on);
+  if (rc) return rc;
+  if (!dq_accum) return set_error(LLAMAX_ERR_ARG, "attn_bwd: null pointer");
+  return attn_bwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, dout, lddo, dq, lddq, dk, lddk, dv, lddv, dq_accum, delta,
+                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, drop, on,
+                      stream);
 }
 
 int llamax_attn_bwd_deterministic(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
@@ -1782,7 +1977,25 @@ int llamax_attn_bwd_deterministic(const void* q, int64_t ldq, const void* k, int
                                   const void* prefix_len_b, const void* doc_start, const void* doc_end, float scale,
                                   const void* rope_inverse, void* stream) {
   return attn_bwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, dout, lddo, dq, lddq, dk, lddk, dv, lddv, nullptr, delta,
-                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, stream);
+                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, AttnDrop{},
+                      false, stream);
+}
+
+int llamax_attn_bwd_deterministic_dropout(const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v,
+                                          int64_t ldv, const void* o, int64_t ldo, const void* lse, const void* dout,
+                                          int64_t lddo, void* dq, int64_t lddq, void* dk, int64_t lddk, void* dv,
+                                          int64_t lddv, void* delta, int64_t B, int64_t S, int32_t Hq, int32_t Hkv,
+                                          int32_t D, int64_t prefix_len, const void* prefix_len_b,
+                                          const void* doc_start, const void* doc_end, float scale,
+                                          const void* rope_inverse, float dropout_p, uint64_t seed, uint64_t offset,
+                                          void* stream) {
+  AttnDrop drop;
+  bool on;
+  const int rc = make_attn_drop(dropout_p, seed, offset, &drop, &on);
+  if (rc) return rc;
+  return attn_bwd_run(q, ldq, k, ldk, v, ldv, o, ldo, lse, dout, lddo, dq, lddq, dk, lddk, dv, lddv, nullptr, delta,
+                      B, S, Hq, Hkv, D, prefix_len, prefix_len_b, doc_start, doc_end, scale, rope_inverse, drop, on,
+                      stream);
 }
 
 }  // extern "C"

@@ -476,7 +476,7 @@ class FusedDecoderBlock(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x: Tensor, rope: Tensor, meta, *trainables):
-        layer, prefix_len, doc_start, doc_end = meta
+        layer, prefix_len, doc_start, doc_end, dropout_p = meta
         att, ff = layer.attention, layer.feed_forward
         B, S, Dm = x.shape
         M = B * S
@@ -518,8 +518,9 @@ class FusedDecoderBlock(torch.autograd.Function):
                 _linear(spec, xn1, xq, xs, h, out=qkv[:, c0:c1])
         if not rope_done:
             ops.rope_(qkv, rope, B, S, Hq + Hkv, D)
+        ctx.attn_rng = ops.attn_dropout_rng(x.device) if dropout_p > 0 else None
         o, lse = ops.attn_fwd(qkv[:, :nq], qkv[:, nq : nq + nk], qkv[:, nq + nk :], B, S, Hq, Hkv, D, prefix_len,
-                              doc_start=doc_start)
+                              doc_start=doc_start, dropout_p=dropout_p, rng=ctx.attn_rng)
         oq = osc = None
         if so.dynamic:
             oq, osc = ops.rowquant_int8(o)
@@ -549,7 +550,7 @@ class FusedDecoderBlock(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dout: Tensor):
-        layer, prefix_len, doc_start, doc_end = ctx.meta
+        layer, prefix_len, doc_start, doc_end, dropout_p = ctx.meta
         att, ff = layer.attention, layer.feed_forward
         if _param_versions(layer) != ctx.versions:
             raise RuntimeError("FusedDecoderBlock: a parameter of this block (LoRA A/B, norm weight or int8 weight) was "
@@ -686,7 +687,8 @@ class FusedDecoderBlock(torch.autograd.Function):
         dqkv = _padded_empty(M, nq + 2 * nk + rqkv, dev)
         ops.attn_bwd(qkv[:, :nq], qkv[:, nq : nq + nk], qkv[:, nq + nk :], o, lse, do,
                      dqkv[:, :nq], dqkv[:, nq : nq + nk], dqkv[:, nq + nk : nq + 2 * nk], B, S, Hq, Hkv, D, prefix_len,
-                     doc_start=doc_start, doc_end=doc_end, rope_inverse=rope, delta=delta)   # dq, dk come back un-rotated
+                     doc_start=doc_start, doc_end=doc_end, rope_inverse=rope, delta=delta,   # dq, dk come back un-rotated
+                     dropout_p=dropout_p, rng=ctx.attn_rng)
         wtqkv, placedqkv = operand("wqkv")
         dxn1, gqkv = _group_backward((sq, sk, sv), dqkv, nq + 2 * nk, xn1, wtqkv, placedqkv, prep, sink,
                                      i8=i8.get("wqkv"), mixed=mixed.get("wqkv"), group_key="wqkv")
@@ -726,7 +728,6 @@ def fused_block_supported(layer, x: Tensor) -> bool:
     mods = (att.wq, att.wk, att.wv, att.wo, ff.w1, ff.w3, ff.w2)
     return (
         x.is_cuda and x.dtype is torch.bfloat16 and att.kv_cache is None and att.head_dim in (64, 128)
-        and not (layer.training and att.attn_dropout > 0)   # falls through to Attention.forward, which raises
         and all(isinstance(m.weight, Int8LinearWeight) and m.bias is None for m in mods)
         and all(getattr(m, "rank", 0) <= 16 and getattr(m, "rank", 0) % 8 == 0 for m in mods)
         and att.wq.weight.dynamic_int8_act == att.wk.weight.dynamic_int8_act == att.wv.weight.dynamic_int8_act

@@ -246,18 +246,22 @@ def apply_rope(x: Tensor, rope: Tensor) -> Tensor:
 
 
 class _PrefixLMAttentionFn(torch.autograd.Function):
-    """o = softmax(q k^T / sqrt(D) + mask) v on [B, S, H, D] tensors (GQA native)."""
+    """o = dropout(softmax(q k^T / sqrt(D) + mask)) v on [B, S, H, D] tensors (GQA native)."""
 
     @staticmethod
-    def forward(ctx, q: Tensor, k: Tensor, v: Tensor, prefix_len: int, doc_start=None, doc_end=None):
+    def forward(ctx, q: Tensor, k: Tensor, v: Tensor, prefix_len: int, doc_start=None, doc_end=None,
+                dropout_p: float = 0.0):
         B, S, Hq, D = q.shape
         Hkv = k.shape[2]
         q2, k2, v2 = (t.reshape(B * S, -1) for t in (q, k, v))
         q2, k2, v2 = (t if t.stride(1) == 1 else t.contiguous() for t in (q2, k2, v2))
-        o, lse = ops.attn_fwd(q2, k2, v2, B, S, Hq, Hkv, D, prefix_len, doc_start=doc_start)
+        rng = ops.attn_dropout_rng(q.device) if dropout_p > 0 else None
+        o, lse = ops.attn_fwd(q2, k2, v2, B, S, Hq, Hkv, D, prefix_len, doc_start=doc_start, dropout_p=dropout_p,
+                              rng=rng)
         ctx.save_for_backward(q2, k2, v2, o, lse)
         ctx.dims = (B, S, Hq, Hkv, D, prefix_len)
         ctx.docs = (doc_start, doc_end)
+        ctx.dropout = (dropout_p, rng)
         return o.view(B, S, Hq, D)
 
     @staticmethod
@@ -266,12 +270,14 @@ class _PrefixLMAttentionFn(torch.autograd.Function):
         B, S, Hq, Hkv, D, prefix_len = ctx.dims
         dq, dk, dv = torch.empty_like(q2), torch.empty_like(k2), torch.empty_like(v2)
         ops.attn_bwd(q2, k2, v2, o, lse, do.reshape(B * S, Hq * D), dq, dk, dv, B, S, Hq, Hkv, D, prefix_len,
-                     doc_start=ctx.docs[0], doc_end=ctx.docs[1])
-        return dq.view(B, S, Hq, D), dk.view(B, S, Hkv, D), dv.view(B, S, Hkv, D), None, None, None
+                     doc_start=ctx.docs[0], doc_end=ctx.docs[1], dropout_p=ctx.dropout[0], rng=ctx.dropout[1])
+        return dq.view(B, S, Hq, D), dk.view(B, S, Hkv, D), dv.view(B, S, Hkv, D), None, None, None, None
 
 
-def prefix_lm_attention(q: Tensor, k: Tensor, v: Tensor, prefix_len: int = 0, doc_start=None, doc_end=None) -> Tensor:
-    return _PrefixLMAttentionFn.apply(q, k, v, prefix_len, doc_start, doc_end)
+def prefix_lm_attention(q: Tensor, k: Tensor, v: Tensor, prefix_len: int = 0, doc_start=None, doc_end=None,
+                        dropout_p: float = 0.0) -> Tensor:
+    """dropout_p > 0: attention dropout with a keep mask drawn from the default CUDA generator (ops.attn_dropout_rng)."""
+    return _PrefixLMAttentionFn.apply(q, k, v, prefix_len, doc_start, doc_end, dropout_p)
 
 
 class Attention(nn.Module):
@@ -292,15 +298,14 @@ class Attention(nn.Module):
                 block_mask=None) -> Tensor:
         if self.kv_cache is not None:
             raise NotImplementedError("llamax_b200: KV-cache decoding is outside the fine-tuning hot path")
-        if self.training and self.attn_dropout > 0:
-            raise NotImplementedError("llamax_b200: attention dropout is not implemented")
         desc = _mask_desc(mask, block_mask, input_pos)
         B, L, _ = x.shape
         q = self.wq(x).view(B, L, self.num_heads, self.head_dim)
         k = self.wk(x).view(B, L, self.num_kv_heads, self.head_dim)
         v = self.wv(x).view(B, L, self.num_kv_heads, self.head_dim)
         q, k = apply_rope(q, rope), apply_rope(k, rope)
-        out = prefix_lm_attention(q, k, v, desc.prefix_len, desc.doc_start, desc.doc_end)
+        out = prefix_lm_attention(q, k, v, desc.prefix_len, desc.doc_start, desc.doc_end,
+                                  self.attn_dropout if self.training else 0.0)
         return self.wo(out.reshape(B, L, self.num_heads * self.head_dim))
 
 
@@ -348,7 +353,8 @@ class TransformerLayer(nn.Module):
                 block_mask=None) -> Tensor:
         if fused_block_supported(self, x):
             desc = _mask_desc(mask, block_mask, input_pos)
-            return FusedDecoderBlock.apply(x, rope, (self, desc.prefix_len, desc.doc_start, desc.doc_end),
+            p = self.attention.attn_dropout if self.training else 0.0
+            return FusedDecoderBlock.apply(x, rope, (self, desc.prefix_len, desc.doc_start, desc.doc_end, p),
                                            *block_trainables(self))
         # unfused composition (e.g. bf16 base weights): same math, module by module
         x = x + self.attention(self.attention_norm(x), rope, mask=mask, input_pos=input_pos, block_mask=block_mask)

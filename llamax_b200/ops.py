@@ -634,10 +634,40 @@ def doc_bounds(doc_ids: Tensor):
     return start.to(torch.int32).contiguous(), end.to(torch.int32).contiguous()
 
 
+# generator offset consumed by one attention call with dropout: the kernels use offset / 4 as a Philox counter word
+ATTN_DROPOUT_OFFSET_STEP = 4
+
+
+def attn_dropout_rng(device) -> tuple[int, int]:
+    """(seed, offset) of one attention call with dropout, drawn from the device's default CUDA generator, which is then
+    advanced: torch.manual_seed repeats the masks, every call gets a fresh one, and torch.utils.checkpoint (which
+    restores the generator state) replays the same mask in its recompute. Not available under CUDA-graph capture."""
+    if torch.cuda.is_current_stream_capturing():
+        raise NotImplementedError("llamax_b200: attention dropout under CUDA-graph capture is not supported")
+    device = torch.device(device)
+    gen = torch.cuda.default_generators[device.index if device.index is not None else torch.cuda.current_device()]
+    seed, offset = gen.initial_seed(), gen.get_offset()
+    gen.set_offset(offset + ATTN_DROPOUT_OFFSET_STEP)
+    return seed, offset
+
+
+def _check_dropout(dropout_p) -> float:
+    p = float(dropout_p)
+    if not 0.0 <= p < 1.0:
+        raise ValueError(f"attention dropout_p must be in [0, 1), got {dropout_p}")
+    return p
+
+
 def attn_fwd(q: Tensor, k: Tensor, v: Tensor, B: int, S: int, Hq: int, Hkv: int, D: int, prefix_len,
-             scale: float | None = None, doc_start: Tensor | None = None):
+             scale: float | None = None, doc_start: Tensor | None = None, *, dropout_p: float = 0.0, rng=None):
     """q [B*S, Hq*D] / k, v [B*S, Hkv*D] row views (unit inner stride). prefix_len: int, or an int tensor [B] with one
-    prefix length per sequence. Returns (o [B*S, Hq*D], lse [B,Hq,S])."""
+    prefix length per sequence. Returns (o [B*S, Hq*D], lse [B,Hq,S]).
+    dropout_p > 0: o = (P o Z / (1 - p)) V with a Philox keep mask Z (include/llamax_b200.h: the drop rate is
+    round(256 p) / 256); rng = (seed, offset), drawn with attn_dropout_rng when None. Pass the same pair to attn_bwd.
+    lse stays that of the undropped softmax."""
+    dropout_p = _check_dropout(dropout_p)
+    if dropout_p > 0.0 and rng is None:
+        rng = attn_dropout_rng(q.device)
     lib, st = _prep(q)
     for t in (q, k, v):
         assert t.dtype is torch.bfloat16 and t.dim() == 2 and t.stride(1) == 1 and t.shape[0] == B * S
@@ -645,6 +675,12 @@ def attn_fwd(q: Tensor, k: Tensor, v: Tensor, B: int, S: int, Hq: int, Hkv: int,
     lse = torch.empty(B, Hq, S, device=q.device, dtype=torch.float32)
     scale = float(scale) if scale is not None else D ** -0.5
     p_scalar, p_b = _prefix_args(prefix_len, B, q.device)
+    if dropout_p > 0.0:
+        seed, offset = rng
+        _call(lib, "llamax_attn_fwd_dropout",
+              (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0), _p(lse), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), scale, dropout_p, seed, offset, st,),
+              "attn_fwd_drop", 4.0 * B * Hq * D * _pairs(S, prefix_len), 0.0)
+        return o, lse
     _call(lib, "llamax_attn_fwd",
           (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0), _p(lse), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), scale, st,),
           "attn_fwd", 4.0 * B * Hq * D * _pairs(S, prefix_len), 0.0)
@@ -652,13 +688,19 @@ def attn_fwd(q: Tensor, k: Tensor, v: Tensor, B: int, S: int, Hq: int, Hkv: int,
 
 
 def attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, prefix_len, scale=None, doc_start=None,
-             doc_end=None, rope_inverse=None, delta=None, *, deterministic: bool | None = None):
+             doc_end=None, rope_inverse=None, delta=None, *, deterministic: bool | None = None, dropout_p: float = 0.0,
+             rng=None):
     """Writes dq/dk/dv (row views like q/k/v). rope_inverse: fp32 [>= S, D/2, 2] table -> dq, dk come back already
     rotated through the RoPE backward (no separate rope_(..., inverse=True) pass needed). delta: fp32 [B, Hq, S] =
     sum_d dout * o already computed (bf16_gemm_rowdot): o is then not read and may be None.
     deterministic (None: torch.are_deterministic_algorithms_enabled()): dq from a kernel that sums the kv tiles of each
-    query tile in a fixed order (it recomputes the S and dP products) instead of fp32 atomics; dk, dv are unchanged."""
+    query tile in a fixed order (it recomputes the S and dP products) instead of fp32 atomics; dk, dv are unchanged.
+    dropout_p > 0: the backward of attn_fwd(..., dropout_p, rng) with the same (seed, offset) pair `rng`, which
+    regenerates the forward's mask (delta = rowsum(dout * o) stays valid)."""
     det = deterministic_mode(deterministic)
+    dropout_p = _check_dropout(dropout_p)
+    if dropout_p > 0.0 and rng is None:
+        raise ValueError("attn_bwd with dropout_p > 0 needs the (seed, offset) pair its forward used")
     if rope_inverse is not None:
         assert rope_inverse.dtype is torch.float32 and rope_inverse.is_contiguous()
         assert rope_inverse.shape[0] >= S and rope_inverse.shape[1] == D // 2
@@ -672,6 +714,17 @@ def attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, prefix_len, sc
         o = None
     scale = float(scale) if scale is not None else D ** -0.5
     p_scalar, p_b = _prefix_args(prefix_len, B, q.device)
+    if dropout_p > 0.0:
+        seed, offset = rng
+        if det:
+            _call(lib, "llamax_attn_bwd_deterministic_dropout",
+                  (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0) if o is not None else 0, _p(lse), _p(dout), dout.stride(0), _p(dq), dq.stride(0), _p(dk), dk.stride(0), _p(dv), dv.stride(0), _p(delta), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), _p(doc_end), scale, _p(rope_inverse), dropout_p, seed, offset, st,),
+                  "attn_bwd_drop_det", 14.0 * B * Hq * D * _pairs(S, prefix_len), 0.0)
+        else:
+            _call(lib, "llamax_attn_bwd_dropout",
+                  (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0) if o is not None else 0, _p(lse), _p(dout), dout.stride(0), _p(dq), dq.stride(0), _p(dk), dk.stride(0), _p(dv), dv.stride(0), _p(dq_accum), _p(delta), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), _p(doc_end), scale, _p(rope_inverse), dropout_p, seed, offset, st,),
+                  "attn_bwd_drop", 10.0 * B * Hq * D * _pairs(S, prefix_len), 0.0)
+        return dq, dk, dv
     if det:
         _call(lib, "llamax_attn_bwd_deterministic",
               (_p(q), q.stride(0), _p(k), k.stride(0), _p(v), v.stride(0), _p(o), o.stride(0) if o is not None else 0, _p(lse), _p(dout), dout.stride(0), _p(dq), dq.stride(0), _p(dk), dk.stride(0), _p(dv), dv.stride(0), _p(delta), B, S, Hq, Hkv, D, p_scalar, _p(p_b), _p(doc_start), _p(doc_end), scale, _p(rope_inverse), st,),

@@ -1,5 +1,7 @@
 """Attention forward (and backward) throughput at the bench shapes, graph-replayed: TFLOP/s over unmasked pairs.
-usage: [LLAMAX_B200_LIB=other.so] python tools/attn_fwd_perf.py [bwd]"""
+usage: [LLAMAX_B200_LIB=other.so] python tools/attn_fwd_perf.py [bwd] [sdpa] [dropout=P]
+dropout=P: attention dropout at rate P (a fixed seed: the generator draw is not allowed in a graph capture); with sdpa,
+SDPA runs at the same dropout_p."""
 import os
 import sys
 
@@ -16,6 +18,8 @@ import pynvml
 Hq, Hkv, D = 32, 8, 128
 with_bwd = "bwd" in sys.argv[1:]
 with_sdpa = "sdpa" in sys.argv[1:]   # also time cuDNN SDPA (causal configs) the same way
+drop_p = float(next((a.split("=", 1)[1] for a in sys.argv[1:] if a.startswith("dropout=")), 0.0))
+drop = dict(dropout_p=drop_p, rng=(1234, 0)) if drop_p > 0 else {}
 pynvml.nvmlInit()
 _h = pynvml.nvmlDeviceGetHandleByIndex(0)
 
@@ -84,14 +88,14 @@ for B, S, P in ((8, 2048, 0), (2, 8192, 0), (8, 1756, 1500), (4, 4096, 1024)):
     q, k, v = g[:, : Hq * D], g[:, Hq * D : (Hq + Hkv) * D], g[:, (Hq + Hkv) * D :]
     pairs = S * P + (S - P) * (S - P + 1) / 2
     fl = 4.0 * B * Hq * D * pairs
-    ms, sus = timeit(lambda: ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P))
-    line = f"B={B} S={S} P={P}: fwd burst {fl / ms / 1e9:7.1f} sustained {fl / sus / 1e9:7.1f} TFLOP/s [{last_clocks}]"
+    ms, sus = timeit(lambda: ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P, **drop))
+    line = f"B={B} S={S} P={P} dropout={drop_p}: fwd burst {fl / ms / 1e9:7.1f} sustained {fl / sus / 1e9:7.1f} TFLOP/s [{last_clocks}]"
     if with_bwd:
-        o, lse = ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P)
+        o, lse = ops.attn_fwd(q, k, v, B, S, Hq, Hkv, D, P, **drop)
         dout = torch.randn(B * S, Hq * D, device="cuda").bfloat16()
         dqkv = torch.empty_like(g)
         dq, dk, dv = dqkv[:, : Hq * D], dqkv[:, Hq * D : (Hq + Hkv) * D], dqkv[:, (Hq + Hkv) * D :]
-        msb, susb = timeit(lambda: ops.attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, P))
+        msb, susb = timeit(lambda: ops.attn_bwd(q, k, v, o, lse, dout, dq, dk, dv, B, S, Hq, Hkv, D, P, **drop))
         line += f" | bwd burst {2.5 * fl / msb / 1e9:7.1f} sustained {2.5 * fl / susb / 1e9:7.1f} TFLOP/s [{last_clocks}]"
     print(line, flush=True)
     if with_sdpa and P == 0:
@@ -102,16 +106,22 @@ for B, S, P in ((8, 2048, 0), (2, 8192, 0), (8, 1756, 1500), (4, 4096, 1024)):
         k4 = k.view(B, S, Hkv, D).transpose(1, 2).contiguous().requires_grad_(True)
         v4 = v.view(B, S, Hkv, D).transpose(1, 2).contiguous().requires_grad_(True)
         do4 = torch.randn(B, Hq, S, D, device="cuda").bfloat16()
-        with sdpa_kernel(SDPBackend.CUDNN_ATTENTION):
+        backends = [SDPBackend.CUDNN_ATTENTION] + ([SDPBackend.FLASH_ATTENTION, SDPBackend.EFFICIENT_ATTENTION]
+                                                   if drop_p > 0 else [])
+        with sdpa_kernel(backends):
             def f():
-                return F.scaled_dot_product_attention(q4, k4, v4, is_causal=True, enable_gqa=True)
+                return F.scaled_dot_product_attention(q4, k4, v4, is_causal=True, enable_gqa=True, dropout_p=drop_p)
 
             def fb():
                 f().backward(do4)
                 q4.grad = k4.grad = v4.grad = None
 
-            ms, sus = timeit(f)
-            line = f"B={B} S={S} P={P}: cuDNN SDPA fwd burst {fl / ms / 1e9:7.1f} sustained {fl / sus / 1e9:7.1f} TFLOP/s [{last_clocks}]"
+            try:
+                ms, sus = timeit(f)
+            except Exception as e:
+                print(f"B={B} S={S} P={P} dropout={drop_p}: SDPA: {str(e)[:120]}", flush=True)
+                continue
+            line = f"B={B} S={S} P={P} dropout={drop_p}: SDPA fwd burst {fl / ms / 1e9:7.1f} sustained {fl / sus / 1e9:7.1f} TFLOP/s [{last_clocks}]"
             try:
                 mfb, sfb = timeit(fb)
                 line += f" | bwd (fwd+bwd - fwd) burst {2.5 * fl / (mfb - ms) / 1e9:7.1f} sustained {2.5 * fl / (sfb - sus) / 1e9:7.1f} TFLOP/s [{last_clocks}]"
