@@ -6,8 +6,6 @@
 #include "common.cuh"
 #include "host_utils.h"
 #include <algorithm>
-
-#include <cstdlib>
 #include <type_traits>
 
 #include "llamax_b200.h"
@@ -25,7 +23,7 @@ static inline bool row_cfg(int64_t D, RowCfg& c, bool one_vec_per_thread = false
   const int nvec = (int)(D / 8);
   // two 16-byte vectors per thread when the row allows it (measured on B200: 256 threads x 2 vectors beats
   // 512 x 1 for D = 4096 rows by ~25 %), at most 512 threads per row
-  static const int vec_target = getenv("LLAMAX_ROW_VECS") ? std::max(1, atoi(getenv("LLAMAX_ROW_VECS"))) : 2;  // A/B only
+  constexpr int vec_target = 2;
   int threads = std::min(512, (((nvec + vec_target - 1) / vec_target + 31) / 32) * 32);
   if (one_vec_per_thread) threads = std::min(512, ((nvec + 31) / 32) * 32);  // persistent kernels: more warps per CTA
   int v = (nvec + threads - 1) / threads;
@@ -460,13 +458,11 @@ row_wpr_kernel(const __nv_bfloat16* __restrict__ x, int64_t ldx, const __nv_bflo
   cp_async_wait<0>();
 }
 
-// rows of up to 32 * 16 vectors, 16-byte aligned, enough of them to fill the machine. LLAMAX_ROW_WPR=0 falls back to the
-// block-per-row ring kernels (A/B).
+// rows of up to 32 * 16 vectors, 16-byte aligned, enough of them to fill the machine; other rows go to the block-per-row
+// ring kernels
 static bool wpr_cfg(int nvec, int64_t M, bool aligned, int& kvec, int& grid, int& smem, bool norm) {
-  static const bool enabled = getenv("LLAMAX_ROW_WPR") == nullptr || atoi(getenv("LLAMAX_ROW_WPR")) != 0;
-  static const int per_sm_env = getenv("LLAMAX_ROW_WPR_CTAS") ? std::max(1, atoi(getenv("LLAMAX_ROW_WPR_CTAS"))) : 0;
-  const int per_sm = per_sm_env > 0 ? per_sm_env : (norm ? 3 : 4);   // = the kernels' launch bounds (registers)
-  if (!enabled || !aligned || nvec > 512 || M < 1024) return false;
+  const int per_sm = norm ? 3 : 4;   // = the kernels' launch bounds (registers)
+  if (!aligned || nvec > 512 || M < 1024) return false;
   const int v = (nvec + 31) / 32;
   kvec = v <= 1 ? 1 : v <= 2 ? 2 : v <= 4 ? 4 : v <= 8 ? 8 : 16;
   smem = (kWprWarps + (norm ? 1 : 0)) * 32 * kvec * 16;
@@ -1187,15 +1183,12 @@ using namespace lx;
 typedef __nv_bfloat16 bf16;
 
 // Ring (persistent, cp.async-prefetched) row kernels: used when the ring fits next to enough resident CTAs and there
-// are enough rows for the prefetch depth to matter. LLAMAX_ROW_RING=0 keeps the one-CTA-per-row kernels (A/B).
+// are enough rows for the prefetch depth to matter; otherwise the one-CTA-per-row kernels.
 static bool ring_cfg(const RowCfg& c, int64_t M, bool aligned, int& grid, int& smem) {
-  static const bool enabled = getenv("LLAMAX_ROW_RING") == nullptr || atoi(getenv("LLAMAX_ROW_RING")) != 0;
-  static const int per_sm_env = getenv("LLAMAX_ROW_RING_CTAS") ? atoi(getenv("LLAMAX_ROW_RING_CTAS")) : 0;
   smem = kRingStages * c.threads * c.V * 16;
-  if (!enabled || !aligned || smem > 96 * 1024) return false;
+  if (!aligned || smem > 96 * 1024) return false;
   const int by_smem = (200 * 1024) / (smem + 1024), by_threads = 2048 / c.threads;
-  int per_sm = std::max(1, std::min(by_smem, by_threads));
-  if (per_sm_env > 0) per_sm = std::min(per_sm, per_sm_env);
+  const int per_sm = std::max(1, std::min(by_smem, by_threads));
   grid = sm_count() * per_sm;
   if (M < (int64_t)grid * 2) return false;
   return true;
@@ -1283,10 +1276,9 @@ int llamax_swiglu_fwd(const void* a, const void* b, int64_t ld, void* g, void* q
   if ((q8 == nullptr) != (qscale == nullptr)) return set_error(LLAMAX_ERR_ARG, "swiglu_fwd: q8 and qscale go together");
   if (!row_cfg(F, c) || ld % 8) return set_error(LLAMAX_ERR_ARG, "swiglu_fwd: F and ld must be multiples of 8");
   if (M == 0) return 0;
-  static const bool ring_on = getenv("LLAMAX_SWIGLU_RING") == nullptr || atoi(getenv("LLAMAX_SWIGLU_RING")) != 0;
   const bool aligned = ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) % 16) == 0;
   const int smem = kRingStages * 2 * c.threads * c.V * 16;
-  if (ring_on && aligned && c.V <= 4 && smem <= 200 * 1024) {
+  if (aligned && c.V <= 4 && smem <= 200 * 1024) {
     const int per_sm = std::max(1, std::min((216 * 1024) / (smem + 1280), 2048 / c.threads));
     const int grid = sm_count() * per_sm;
     if (M >= (int64_t)grid * 2) {
@@ -1327,11 +1319,10 @@ int llamax_rmsnorm_bwd(const void* dy, const void* x, const void* w, const void*
   if (!row_cfg(D, c, true)) return set_error(LLAMAX_ERR_ARG, "rmsnorm_bwd: D must be a multiple of 8 and <= 65536");
   if (nparts <= 0 || nparts > 4096) return set_error(LLAMAX_ERR_ARG, "rmsnorm_bwd: nparts out of range");
   // ring kernel: rows of up to 256 threads x 2 vectors (the model width), 16-byte aligned streams, a few rows per CTA
-  static const bool ring_on = getenv("LLAMAX_RMSNORM_BWD_RING") == nullptr || atoi(getenv("LLAMAX_RMSNORM_BWD_RING")) != 0;
   RowCfg cr;
   const bool aligned = ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) |
                          reinterpret_cast<uintptr_t>(dres)) % 16) == 0;
-  if (ring_on && aligned && row_cfg(D, cr) && cr.threads <= 256 && cr.V <= 2 && M >= (int64_t)nparts * 2) {
+  if (aligned && row_cfg(D, cr) && cr.threads <= 256 && cr.V <= 2 && M >= (int64_t)nparts * 2) {
     const int smem = kRingStages * 3 * cr.threads * cr.V * 16;
     LX_DISPATCH_V(cr.V, {
       LX_RING_SMEM(rmsnorm_bwd_ring_kernel<kV>, smem, "rmsnorm_bwd");

@@ -865,11 +865,10 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 // ------------------------------------------------------------------------------------------------
 // Wave-alignment counters (see the producer of gemm_wide_kernel): one int per sync point, a slot of kSyncInts per launch
 // out of a per-device ring (concurrent launches from other streams / threads get different slots), zeroed in stream
-// order before the launch. Returns null when the feature is off, the launch has too many sync points, or allocation fails.
+// order before the launch. Returns null when the launch has too many sync points or allocation fails.
 static int* acquire_wave_sync(int points, cudaStream_t stream) {
-  static const bool use_sync = !(getenv("LLAMAX_GEMM_WAVESYNC") != nullptr && atoi(getenv("LLAMAX_GEMM_WAVESYNC")) == 0);
   constexpr int kSyncInts = 128, kSyncSlots = 64, kMaxDev = 16;
-  if (!use_sync || points > kSyncInts) return nullptr;
+  if (points > kSyncInts) return nullptr;
   static std::mutex mu;
   static int* ring[kMaxDev] = {nullptr};
   static std::atomic<unsigned> next_slot{0};
@@ -933,21 +932,18 @@ static int launch_gemm_r(const void* A, int64_t lda, const void* B, int64_t ldb,
 
   GemmParams pp = p;
   {
-    static const int forced = getenv("LLAMAX_GEMM_GROUP") ? atoi(getenv("LLAMAX_GEMM_GROUP")) : 0;   // A/B switch
     const int num_m = (p.M + kBM * CG - 1) / (kBM * CG), num_n = (p.N + kBN - 1) / kBN;
-    pp.group = forced != 0 ? forced : (num_m >= num_n ? -kGroupM : kGroupM);
-    // Wave alignment every `sync_every` visits (see gemm_wide_kernel). Measured per kernel form, sustained, same box
-    // (tools/sync_every_ab.py): the w2 grad_input GEMM with the SwiGLU-backward epilogue — the form that moves the most
+    pp.group = num_m >= num_n ? -kGroupM : kGroupM;
+    // Wave alignment every `sync_every` visits (see gemm_wide_kernel). Measured per kernel form, sustained, same box:
+    // the w2 grad_input GEMM with the SwiGLU-backward epilogue — the form that moves the most
     // DRAM bytes per flop (5.8 GB per launch) — gains 2.5 % at any period 1..8 (1016-1026 -> 1044-1050 TFLOP/s); the
     // INT8 forward GEMM (2429-2437 -> 2291-2414 TOP/s) and the short-K bf16 GEMMs (1292-1295 -> 1270-1291) lose: their
-    // operand panels fit the L2 whatever the drift, and the barrier only adds a wait. Default: that one form, period 2.
-    // LLAMAX_GEMM_SYNC_EVERY overrides the period for every form (0 = off).
-    static const int forced_sync = getenv("LLAMAX_GEMM_SYNC_EVERY") ? atoi(getenv("LLAMAX_GEMM_SYNC_EVERY")) : -1;
-    const int sync_every = forced_sync >= 0 ? forced_sync : (kSwi ? 2 : 0);
+    // operand panels fit the L2 whatever the drift, and the barrier only adds a wait. So: that one form, period 2.
+    constexpr int kSyncEvery = 2;
     const int visits = (num_tiles + clusters - 1) / clusters;
-    if (sync_every > 0 && visits > sync_every) {
-      pp.wave_sync = acquire_wave_sync(visits / sync_every + 1, stream);
-      pp.sync_every = sync_every;
+    if (kSwi && visits > kSyncEvery) {
+      pp.wave_sync = acquire_wave_sync(visits / kSyncEvery + 1, stream);
+      pp.sync_every = kSyncEvery;
     }
   }
   cudaLaunchConfig_t cfg{};
@@ -1012,8 +1008,7 @@ static int launch_gemm_mix(const void* A, int64_t lda, const void* B8, int64_t l
   const int num_m = (p.M + 2 * kBM - 1) / (2 * kBM), num_n = (p.N + kBN - 1) / kBN;
   const int clusters = std::min(sm_count() / 2, num_m * num_n);
   GemmParams pp = p;
-  static const int forced = getenv("LLAMAX_GEMM_GROUP") ? atoi(getenv("LLAMAX_GEMM_GROUP")) : 0;   // A/B switch
-  pp.group = forced != 0 ? forced : (num_m >= num_n ? -kGroupM : kGroupM);
+  pp.group = num_m >= num_n ? -kGroupM : kGroupM;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(clusters * 2);
   cfg.blockDim = dim3(kMixThreads);
@@ -1051,8 +1046,7 @@ static int launch_gemm(const void* A, int64_t lda, const void* B, int64_t ldb, c
   if constexpr (kInt8) {
     // forward projections with the residual connection (wo, w2): pipelined residual reads; needs resid != C and a
     // 16-byte aligned residual (rows start on 16-byte boundaries when ldr % 8 == 0)
-    static const bool no_res = getenv("LLAMAX_NO_RES_PIPE") != nullptr;   // A/B switch for benchmarking
-    if (!no_res && p.resid != nullptr && (p.flags & 1) == 0 && static_cast<const void*>(p.resid) != p.C &&
+    if (p.resid != nullptr && (p.flags & 1) == 0 && static_cast<const void*>(p.resid) != p.C &&
         reinterpret_cast<uintptr_t>(p.resid) % 16 == 0 && p.ldr % 8 == 0) {
       if (p.lora_rank <= 0) return launch_gemm_r<kInt8, CG, 0, false, false, true>(A, lda, B, ldb, p, stream);
       if (p.lora_rank <= 8) return launch_gemm_r<kInt8, CG, 8, false, false, true>(A, lda, B, ldb, p, stream);
@@ -1277,8 +1271,7 @@ static int launch_gemm_wide(const void* A, int64_t lda, const void* B, int64_t l
     return rc;
   const int num_m = (M + 511) / 512, num_n = (N + kBN - 1) / kBN;
   int clusters = std::min(sm_count() / 2, num_m * num_n);
-  static const int forced = getenv("LLAMAX_GEMM_GROUP") ? atoi(getenv("LLAMAX_GEMM_GROUP")) : 0;   // A/B switch
-  const int group = forced != 0 ? forced : (num_m >= num_n ? -kGroupM : kGroupM);
+  const int group = num_m >= num_n ? -kGroupM : kGroupM;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(clusters * 2);
   cfg.blockDim = dim3(kGemmThreads);
@@ -1292,7 +1285,7 @@ static int launch_gemm_wide(const void* A, int64_t lda, const void* B, int64_t l
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   const int visits = (num_m * num_n + clusters - 1) / clusters;
-  int* wave_sync = visits > 1 ? acquire_wave_sync(visits, stream) : nullptr;   // LLAMAX_GEMM_WAVESYNC=0: off (A/B)
+  int* wave_sync = visits > 1 ? acquire_wave_sync(visits, stream) : nullptr;
   cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_wide_kernel, tmA, tmB, (__nv_bfloat16*)C, ldc, M, N, K, group, wave_sync);
   if (e != cudaSuccess) return set_cuda_error(e, "wide gemm: launch");
   return 0;
@@ -1832,19 +1825,16 @@ int llamax_bf16_gemm(const void* A, int64_t lda, const void* B, int64_t ldb, voi
   if (!A || !B || !C) return set_error(LLAMAX_ERR_ARG, "bf16_gemm: null pointer");
   if (M <= 0 || N <= 0 || K <= 0) return set_error(LLAMAX_ERR_ARG, "gemm: empty problem");
   const bool plain = col_scale == nullptr && (epi == nullptr || (epi->lora_h == nullptr && epi->resid == nullptr));
-  static const bool no_skinny = getenv("LLAMAX_NO_SKINNY") != nullptr;  // A/B switch for benchmarking
-  if (plain && N <= 32 && !no_skinny)  // LoRA down / dh projections: HBM-bound skinny kernel
+  if (plain && N <= 32)  // LoRA down / dh projections: HBM-bound skinny kernel
     return launch_skinny(A, lda, B, ldb, C, ldc, (int)M, (int)N, (int)K, (cudaStream_t)stream);
-  // long contractions without an epilogue (w1|w3 grad_input, LM-head grad_input): 512 x 256 outputs per CTA-pair visit
-  static const bool no_wide = getenv("LLAMAX_GEMM_WIDE") != nullptr && getenv("LLAMAX_GEMM_WIDE")[0] == '0';  // A/B switch
-  static const int wide_min_k = getenv("LLAMAX_GEMM_WIDE_MINK") ? atoi(getenv("LLAMAX_GEMM_WIDE_MINK")) : 8192;   // A/B
+  // long contractions without an epilogue (w1|w3 grad_input, LM-head grad_input): 512 x 256 outputs per CTA-pair visit;
+  // LLAMAX_GEMM_WIDE=0 keeps them on the 256 x 256 kernel
+  static const bool no_wide = getenv("LLAMAX_GEMM_WIDE") != nullptr && getenv("LLAMAX_GEMM_WIDE")[0] == '0';
   // Very wide outputs with a short contraction (the LM-head logits GEMM [8192, 128256, 4096]) stay on the 256 x 256 kernel:
-  // back to back at the power cap the wide tile looked better there (1106-1113 -> 1230-1236 TFLOP/s, tools/wide_mink_ab.py),
+  // back to back at the power cap the wide tile looked better there (1106-1113 -> 1230-1236 TFLOP/s),
   // but INSIDE the step, where the LM head runs at the clocks the lighter passes before it leave, it is slower — 7.1 ms
   // (1203-1222 TFLOP/s) against 5.5-5.7 ms (1509-1573) in the bench line's per-shape table, same code otherwise.
-  // LLAMAX_GEMM_WIDE_LMHEAD=1 puts those shapes on the wide tile again (A/B).
-  static const bool wide_lmhead = getenv("LLAMAX_GEMM_WIDE_LMHEAD") != nullptr && getenv("LLAMAX_GEMM_WIDE_LMHEAD")[0] == '1';
-  if (plain && !no_wide && g_gemm_cg == 2 && (K >= wide_min_k || (wide_lmhead && N >= 32768 && K >= 2048)) && M >= 1024 &&
+  if (plain && !no_wide && g_gemm_cg == 2 && K >= 8192 && M >= 1024 &&
       N >= 256 && N % 8 == 0 && ldc % 8 == 0 &&
       lda % 8 == 0 && ldb % 8 == 0 && reinterpret_cast<uintptr_t>(A) % 16 == 0 && reinterpret_cast<uintptr_t>(B) % 16 == 0 &&
       reinterpret_cast<uintptr_t>(C) % 16 == 0)
@@ -1864,14 +1854,13 @@ int llamax_bf16_gemm(const void* A, int64_t lda, const void* B, int64_t ldb, voi
 // Token splits of lora_wgrad: one CTA per SM is resident (147 KB ring), so the kernel lasts waves x (tokens per split + a
 // fixed fill/drain cost of ~5 stages). Pick the split count that minimises that: "just enough CTAs to cover the SMs" left
 // a nearly empty second wave (P = 4096: 32 tiles x 5 splits = 160 CTAs on 148 SMs; 9 splits = 288 CTAs, two full waves
-// of half the length). LLAMAX_WGRAD_SPLITS_OLD=1 keeps the old rule (A/B). At most LLAMAX_LORA_WGRAD_MAX_SPLITS splits.
+// of half the length). At most LLAMAX_LORA_WGRAD_MAX_SPLITS splits.
 static void lora_wgrad_splits(int64_t M, int p_tiles, int& splits, int& k_per_split) {
-  static const bool old_rule = getenv("LLAMAX_WGRAD_SPLITS_OLD") != nullptr;
   splits = std::max(1, std::min(LLAMAX_LORA_WGRAD_MAX_SPLITS, (sm_count() + p_tiles - 1) / p_tiles));
   k_per_split = (int)((M + splits - 1) / splits);
   k_per_split = ((k_per_split + 63) / 64) * 64;
   splits = (int)((M + k_per_split - 1) / k_per_split);
-  if (!old_rule && p_tiles * 2 <= sm_count()) {   // wide outputs (P = 14336) stream at HBM rate either way: 79 vs 81 us
+  if (p_tiles * 2 <= sm_count()) {   // wide outputs (P = 14336) stream at HBM rate either way: 79 vs 81 us
     int64_t best_cost = INT64_MAX;
     for (int s = 1; s <= LLAMAX_LORA_WGRAD_MAX_SPLITS; ++s) {
       int kp = (int)((M + s - 1) / s);
@@ -1951,8 +1940,6 @@ int llamax_lora_bwd_pair(const void* dY, int64_t lddy, const void* Bt, int64_t l
   int splits = m_blocks * 4 >= sm_count() * 3
                    ? 1
                    : std::max(1, std::min(total_chunks / 8, (5 * sm_count() / 2 + m_blocks - 1) / m_blocks));
-  static const int splits_env = getenv("LLAMAX_LORA_PAIR_SPLITS") ? atoi(getenv("LLAMAX_LORA_PAIR_SPLITS")) : 0;   // A/B only
-  if (splits_env > 0) splits = std::min(splits_env, total_chunks);
   int chunks_per_split = (total_chunks + splits - 1) / splits;
   splits = (total_chunks + chunks_per_split - 1) / chunks_per_split;
   cudaError_t e = cudaMemsetAsync(dB, 0, (size_t)N * R * sizeof(float), st);

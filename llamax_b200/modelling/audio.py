@@ -12,7 +12,6 @@ reference's README plans (README.md:16) but runs as plain causal attention (audi
 (`prefix_lm=False`) keeps the reference behaviour.
 """
 
-import os
 from typing import NamedTuple
 
 import torch
@@ -21,8 +20,8 @@ from torch import Tensor, nn
 from .. import ops
 from .llama import Llama, LlamaConfig, PrefixLM
 
-# A/B switch (benchmarking only): "0" runs the stem through nn.Conv1d / nn.GELU (cuDNN)
-_OWN_STEM = os.environ.get("LLAMAX_AUDIO_STEM", "1") != "0"
+# False: the stem runs through nn.Conv1d / nn.GELU (cuDNN), the tests' reference for AudioStemFn
+_OWN_STEM = True
 
 
 

@@ -60,14 +60,8 @@ def _get_scratch(device, numel: int) -> Tensor:
 # (checked at the first backward, i.e. at peak activation memory); "1": always; "0": never (shared scratch).
 _CACHE_MODE = os.environ.get("LLAMAX_WEIGHT_CACHE", "auto")
 _CACHE_HEADROOM = 24 << 30
-# A/B switch (benchmarking only): "0" restores the two-pass LoRA backward (skinny dh GEMM + lora_wgrad per linear)
-_LORA_PAIR = os.environ.get("LLAMAX_LORA_PAIR", "1") != "0"
-# The adapters of linears that share an input (wq | wk | wv, w1 | w3) take ONE lora_bwd_pair launch over the concatenated
-# gradient [M, sum N] with a block-diagonal scale * B^T [sum R, sum N]: dh of every adapter comes out of the same pass
-# (the off-diagonal zeros contribute exact zeros) and each dB is its diagonal block of the [sum N, sum R] result —
-# bit-identical to one launch per adapter, whose fixed cost (two memsets, prologue, pipeline fill and drain: ~25 us at the
-# clocks of a power-capped step, more than the streaming time of the [M, 1024] wk / wv gradients) is paid once. "0": A/B.
-_LORA_GROUP_PAIR = os.environ.get("LLAMAX_LORA_GROUP_PAIR", "1") != "0"
+# False: one lora_bwd_pair launch per adapter even where _group_mergeable allows one per input group (the tests' reference)
+_LORA_GROUP_PAIR = True
 
 
 # OPT-IN, NON-PARITY mode (SURVEY section 8 row f4; the reference author's TODO at subclasses/int8.py:105): grad_input =
@@ -75,9 +69,6 @@ _LORA_GROUP_PAIR = os.environ.get("LLAMAX_LORA_GROUP_PAIR", "1") != "0"
 # The gradient is quantised to 8 bits per row, so results differ from the reference beyond the parity tolerance;
 # default off, never used by bench.py's headline.
 _INT8_GRAD = os.environ.get("LLAMAX_INT8_GRAD_INPUT", "0") == "1"
-# A/B switch (benchmarking only): "0" runs the w2 grad_input GEMM and the SwiGLU backward as two launches (identical
-# results); default: SwiGLU backward as the GEMM's epilogue, the [M, F] gradient dg never exists in HBM
-_FUSE_SWIGLU_BWD = os.environ.get("LLAMAX_FUSE_SWIGLU_BWD", "1") != "0"
 # OPT-IN: mixed-input GEMMs (SURVEY K4 / K5): the int8 weight is expanded to bf16 INSIDE the GEMM (converter warps between
 # the TMA ring and the tensor core), so the weight-only forward needs no de-quantised scratch and grad_input needs no
 # (scale * W)^T operand at all — wo and w2 are consumed as stored, q|k|v and w1|w3 as row-concatenated int8 copies
@@ -98,8 +89,6 @@ _FUSE_DELTA = os.environ.get("LLAMAX_FUSE_DELTA", "0") == "1"
 def set_fuse_delta(on: bool) -> None:
     global _FUSE_DELTA
     _FUSE_DELTA = bool(on)
-# A/B switch (benchmarking only): "0" restores three INT8 GEMM launches for wq, wk, wv
-_QKV_ONE_LAUNCH = os.environ.get("LLAMAX_QKV_ONE_LAUNCH", "1") != "0"
 # SURVEY K7 (opt-in): RoPE applied by the epilogue of the single q | k | v INT8 launch instead of the in-place pass over
 # q | k (bit-identical; removes 2.0 ms/step of HBM pass and adds its arithmetic and a 64 B table read per 16 outputs to an
 # epilogue that is the critical path at K = 4096: measured in DESIGN.md). head_dim 128, dynamic INT8, LoRA rank 0 or 8.
@@ -328,6 +317,12 @@ def _lora_prepare(items, M: int, device, groups=()):
 
 
 def _group_mergeable(specs) -> bool:
+    """The adapters of linears that share an input (wq | wk | wv, w1 | w3) take ONE lora_bwd_pair launch over the
+    concatenated gradient [M, sum N] with a block-diagonal scale * B^T [sum R, sum N]: dh of every adapter comes out of
+    the same pass (the off-diagonal zeros contribute exact zeros) and each dB is its diagonal block of the [sum N, sum R]
+    result — bit-identical to one launch per adapter, whose fixed cost (two memsets, prologue, pipeline fill and drain:
+    ~25 us at the clocks of a power-capped step, more than the streaming time of the [M, 1024] wk / wv gradients) is
+    paid once."""
     r_tot = sum(s.R for s in specs)
     return (_lora_pair() and _LORA_GROUP_PAIR and len(specs) > 1 and all(s.R > 0 for s in specs) and r_tot <= 32
             and all(s.lora_scale == specs[0].lora_scale for s in specs) and all(s.N % 8 == 0 for s in specs))
@@ -336,7 +331,7 @@ def _group_mergeable(specs) -> bool:
 def _lora_pair() -> bool:
     """lora_bwd_pair reduces dB and dh across CTAs with fp32 atomics: under torch.use_deterministic_algorithms the
     two-pass form runs instead (the skinny dh GEMM streams each contraction in one CTA; lora_wgrad's deterministic form)."""
-    return _LORA_PAIR and not ops.deterministic_mode()
+    return not ops.deterministic_mode()
 
 
 def _lora_dh_dB(dy: Tensor, bt: Tensor, ht: Tensor, out_dh: Tensor, scale: float, out_dht: Tensor) -> Tensor:
@@ -383,7 +378,7 @@ def _group_backward(specs, dy_cat: Tensor, n_total: int, x_in: Tensor, wt: Tenso
     lora_grads = []
     dht = ops.transposed_rank_buffer(r_total, dy_cat.shape[0], dy_cat.device) if r_total > 0 else None
     merged = prep.get(("group", group_key)) if group_key is not None else None
-    if merged is not None:   # one pass over [M, n_total] for all adapters of the group (see _LORA_GROUP_PAIR)
+    if merged is not None:   # one pass over [M, n_total] for all adapters of the group (see _group_mergeable)
         bt_cat, ht_cat = merged
         if not a_placed and i8 is None and mixed is None:
             for s in specs:
@@ -495,7 +490,7 @@ class FusedDecoderBlock(torch.autograd.Function):
         nq, nk = Hq * D, Hkv * D
         qkv = torch.empty(M, nq + 2 * nk, device=x.device, dtype=torch.bfloat16)
         rope_done = False
-        if _QKV_ONE_LAUNCH and dyn_qkv and _qkv_mergeable(sq, sk, sv, nq, nk):
+        if dyn_qkv and _qkv_mergeable(sq, sk, sv, nq, nk):
             # ONE INT8 GEMM over the row-concatenated [Wq; Wk; Wv] (a resident 25 MB int8 copy per layer at 8B): N = 6144
             # instead of 4096 + 1024 + 1024 — the two N = 1024 launches fill 3.5 waves of 74 CTA pairs and ran at 1870 TOP/s
             # against 2370-2630 for the wide ones. The epilogue picks each column segment's own LoRA-h columns.
@@ -635,7 +630,8 @@ class FusedDecoderBlock(torch.autograd.Function):
         wt2, _ = operand("w2")
         g2 = None
         a_, b_ = ab[:, :F_], ab[:, F_:]
-        fuse = _FUSE_SWIGLU_BWD and not _INT8_GRAD and F_ % 16 == 0
+        # SwiGLU backward as the epilogue of the w2 grad_input GEMM: the [M, F] gradient dg never exists in HBM
+        fuse = not _INT8_GRAD and F_ % 16 == 0
         dh2 = at2 = None
         if s2.R > 0:
             bt2, at2, ht2 = prep[id(s2)]
