@@ -37,7 +37,7 @@ int llamax_set_gemm_cta_group(int cg);
  *   LoRA up-projection  : modelling/lora.py:43   (lora_h = x @ lora_a^T computed by the caller)
  *   residual connection : modelling/llama.py:172-173 */
 typedef struct {
-  const void* lora_h; /* bf16 [M, lora_rank], row pitch ldh; NULL = no LoRA term */
+  const void* lora_h; /* bf16 [M, lora_rank], any row pitch ldh and any 2-byte aligned base; NULL = no LoRA term */
   int64_t ldh;
   const void* lora_b; /* bf16 [N, lora_rank] contiguous */
   int32_t lora_rank;  /* multiple of 4, <= 16 */

@@ -558,9 +558,11 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     static_assert(kBN == kEpiThreads, "one staged column per epilogue thread");
     constexpr bool kPipeStage = kInt8 || kSwi;
     constexpr int kRV = kRank > 0 ? kRank / 8 : 1;
+    // h_vec: every h row starts on a 16-byte boundary (segment offsets are multiples of kRank, hence of 8 elements),
+    // so h may be read with 16-byte loads. The header allows any h pitch and base: otherwise h is read element-wise.
+    const bool h_vec = R == kRank && reinterpret_cast<uintptr_t>(p.lora_h) % 16 == 0 && p.ldh % 8 == 0;
     const bool fast_stage = kPipeStage && !dump &&
-                            (kRank == 0 || (R == kRank && reinterpret_cast<uintptr_t>(p.lora_b) % 16 == 0 &&
-                                            reinterpret_cast<uintptr_t>(p.lora_h) % 16 == 0 && p.ldh % 8 == 0));
+                            (kRank == 0 || (h_vec && reinterpret_cast<uintptr_t>(p.lora_b) % 16 == 0));
     uint32_t ncs = 0;
     float nrs = 1.f;
     uint4 nlb[kRV], nh[kRV];
@@ -645,7 +647,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         if (row_ok && !fast_stage) {
           const __nv_bfloat16* hp = p.lora_h + (int64_t)row * p.ldh +
                                     (p.seg_n0 > 0 ? (col0 >= p.seg_n1 ? 2 * R : col0 >= p.seg_n0 ? R : 0) : 0);
-          if (R == kRank) {  // 16-byte vector loads (h rows are 16-byte aligned for rank 8 / 16)
+          if (h_vec) {
 #pragma unroll
             for (int r = 0; r < kRank; r += 8) {
               const uint4 u = *reinterpret_cast<const uint4*>(hp + r);

@@ -131,10 +131,12 @@ def test_bad_arguments_raise():
         ops.rowquant_int8(torch.zeros(4, 16, dtype=torch.bfloat16))  # CPU tensor: no fallback
 
 
-@pytest.mark.parametrize("M,N,R", [(300, 264, 8), (1024, 4096, 16), (2048, 14336, 8), (129, 128, 24), (640, 1024, 32)])
+@pytest.mark.parametrize("M,N,R", [(300, 264, 8), (1024, 4096, 16), (2048, 14336, 8), (129, 128, 24), (640, 1024, 32),
+                                   (16384, 4096, 8), (16384, 14336, 32), (16383, 4096, 32)])
 def test_lora_bwd_pair_matches_separate_products(M, N, R):
     """Fused one-pass LoRA backward (dh = dY Bt^T and dB = alpha dY^T h) vs the fp32 products (autograd of
-    modelling/lora.py:43); covers the split-N path (fp32 dh partials) and ragged token / column tails."""
+    modelling/lora.py:43); covers the split-N path (fp32 dh partials), the one-wave path without a split that
+    M >= 111 token blocks take on 148 SMs (dh written by the CTA itself), and ragged token / column tails."""
     torch.manual_seed(M + N + R)
     dy = torch.randn(M, N + 16, device="cuda").bfloat16()[:, :N]            # pitched view
     bt = (torch.randn(R, N, device="cuda") * 0.1).bfloat16()
@@ -178,7 +180,8 @@ def test_bf16_gemm_tn_overlapping_rows():
 
 @pytest.mark.parametrize("cg", [1, 2])
 @pytest.mark.parametrize("M,F,K,R,pad", [(256, 512, 128, 0, 0), (301, 1792, 520, 8, 16), (1000, 464, 264, 8, 8),
-                                         (130, 16, 64, 16, 16), (2048, 14336, 72, 8, 16)])
+                                         (130, 16, 64, 16, 16), (2048, 14336, 72, 8, 16), (301, 1792, 520, 4, 16),
+                                         (1000, 464, 264, 12, 8)])
 def test_gemm_with_swiglu_backward_epilogue_equals_two_launches(cg, M, F, K, R, pad):
     """The w2 grad_input GEMM with the SwiGLU backward as its epilogue (dg never written) must give exactly what
     bf16_gemm -> swiglu_bwd gives: same bf16 rounding of dg, same element formulas. Ragged M, F tails inside a tile,
@@ -261,7 +264,8 @@ def test_bf16_gemm_wide_tile_path(M, N, K):
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("M,N,K,Rk,resid", [(256, 256, 64, 0, False), (512, 768, 1024, 8, True), (300, 264, 208, 0, False),
                                             (1000, 1032, 4096, 16, True), (77, 6144, 512, 8, False),
-                                            (4096, 4096, 448, 0, False)])   # > 74 tiles: several tiles per CTA pair
+                                            (4096, 4096, 448, 0, False),    # > 74 tiles: several tiles per CTA pair
+                                            (512, 768, 1024, 4, True), (300, 264, 208, 12, False)])
 def test_mixed_weight_only_forward_equals_dequant_then_gemm(M, N, K, Rk, resid):
     """int8.py:118: bf16(x @ bf16(W8)^T) * scale. The in-GEMM int8 -> bf16 expansion is exact, so the mixed kernel must
     reproduce dequant_weight + bf16_gemm(round_before_scale) bit for bit, and the reference formula within 1e-2."""
@@ -287,7 +291,8 @@ def test_mixed_weight_only_forward_equals_dequant_then_gemm(M, N, K, Rk, resid):
 
 
 @pytest.mark.parametrize("M,N,K1,Rt,Rk", [(256, 256, 64, 0, 0), (512, 768, 1024, 24, 0), (300, 272, 192, 8, 0),
-                                          (1000, 528, 4096, 0, 8), (2048, 4096, 6144, 24, 0), (130, 512, 8192, 16, 16)])
+                                          (1000, 528, 4096, 0, 8), (2048, 4096, 6144, 24, 0), (130, 512, 8192, 16, 16),
+                                          (300, 272, 192, 8, 4), (1000, 528, 4096, 0, 12)])
 def test_mixed_grad_input_equals_dequant_then_gemm(M, N, K1, Rt, Rk):
     """int8.py:127 with the weight consumed AS STORED ([out, in] int8, rows = contraction index), the per-row scale folded
     in during the expansion, and the LoRA A rows as a bf16 tail: bit-identical to the de-quantised-operand GEMM."""
@@ -315,7 +320,7 @@ def test_mixed_grad_input_equals_dequant_then_gemm(M, N, K1, Rt, Rk):
         assert rel_err(out, y) <= 1e-2
 
 
-@pytest.mark.parametrize("M,F,K,R", [(384, 512, 256, 8), (300, 1792, 512, 0)])
+@pytest.mark.parametrize("M,F,K,R", [(384, 512, 256, 8), (300, 1792, 512, 0), (384, 512, 256, 4), (300, 1792, 512, 12)])
 def test_mixed_grad_input_with_swiglu_backward_epilogue(M, F, K, R):
     g = torch.Generator().manual_seed(5)
     dy = torch.randn(M, K, generator=g).bfloat16().cuda()
@@ -344,10 +349,12 @@ def test_mixed_gemm_bad_arguments_raise():
         ops.bf16_int8_gemm_bwd(x, W8, s)
 
 
-@pytest.mark.parametrize("M,K,n0,n1,N,R", [(300, 512, 256, 512, 768, 8), (2048, 4096, 4096, 5120, 6144, 8), (515, 256, 512, 768, 1280, 16)])
+@pytest.mark.parametrize("M,K,n0,n1,N,R", [(300, 512, 256, 512, 768, 8), (2048, 4096, 4096, 5120, 6144, 8), (515, 256, 512, 768, 1280, 16),
+                                           (300, 512, 256, 512, 768, 4), (515, 256, 512, 768, 1280, 12)])
 def test_int8_gemm_lora_column_segments_equal_three_launches(M, K, n0, n1, N, R):
     """q | k | v in ONE launch: column segments [0, n0), [n0, n1), [n1, N) take their own R columns of the shared LoRA-h
-    matrix [M, 3R] and their own rows of the concatenated B; bit-identical to three launches on the three weights."""
+    matrix [M, 3R] and their own rows of the concatenated B; bit-identical to three launches on the three weights.
+    Ranks 4 and 12 (zero-padded to the kernel's 8 / 16) take the per-segment h offset of the unstaged path."""
     g = torch.Generator().manual_seed(N + R)
     A, W = _rand_i8(M, K, gen=g).cuda(), _rand_i8(N, K, gen=g).cuda()
     sa = (torch.rand(M, generator=g) * 0.1).bfloat16().cuda()
@@ -362,7 +369,8 @@ def test_int8_gemm_lora_column_segments_equal_three_launches(M, K, n0, n1, N, R)
     assert torch.equal(out, ref)
 
 
-@pytest.mark.parametrize("M,S,N,K,R", [(512, 256, 512, 256, 8), (1024, 512, 4096, 4096, 8), (300, 100, 256, 192, 0)])
+@pytest.mark.parametrize("M,S,N,K,R", [(512, 256, 512, 256, 8), (1024, 512, 4096, 4096, 8), (300, 100, 256, 192, 0),
+                                       (512, 256, 512, 256, 4), (300, 100, 256, 192, 12)])
 def test_bf16_gemm_rowdot_epilogue(M, S, N, K, R):
     """The grad_input GEMM of wo also returns delta[b, h, s] = sum_d dO * O (groups of 128 columns = heads): C is
     bit-identical to the plain GEMM and the dot products equal those of the stored (rounded) C in fp32."""
